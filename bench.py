@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the mask-evaluation hot path on B200 (see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--layout crop|span|full] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--layout crop|span|full] [--config NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...        # the reference's CPU algorithm on the host cores
 
@@ -77,6 +77,10 @@ def parse():
     ap.add_argument('--api-images', type=int, default=200, help='images per call of the e2e_api leg')
     ap.add_argument('--cpu-images', type=int, default=0)
     ap.add_argument('--cpu-threads', type=int, default=0, help='reference arm: worker processes (0 = all cores)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last step of the headline run computed to '
+                         'DIR/<name>.npy (float64; a seeded sample of arrays longer than 2^19 elements), so that two '
+                         'builds can be compared output for output on identical inputs')
     return ap.parse_args()
 
 
@@ -549,6 +553,48 @@ def oracle_sample_check(run):
             'matcher rules, TP/FP/FN at every threshold', 'equal': True}
 
 
+DUMP_CAP = 1 << 19      # elements kept per dumped array: 4 MB in float64, ten arrays at most
+
+
+def dump_outputs(run, out_dir):
+    """--dump-outputs: what the last timed step of the headline run computed, as its caller receives it from the
+    device, one float64 DIR/<name>.npy each: `totals` (TP/FP/FN per threshold) or `spp_hist` (satellites per
+    particle), per-image `counts`, per-mask `area`, per-row `best_col` / `best_inter` / `best_score`, and the
+    intersections -- `imat` (the dense G x P matrices) or, with --sparse, `sparse_row` / `sparse_col` /
+    `sparse_inter` sorted by row and column.  The launch groups of a step share the row and matrix buffers, so the
+    per-row arrays and the intersections hold the images of the last group (all images when the step is one launch,
+    as for the default C2 batch).  An array of more than DUMP_CAP elements is cut to the elements at DUMP_CAP
+    positions drawn with a fixed seed (the same positions for every array of that length)."""
+    import torch
+    last, g = run.pipes[-1], run.pipes[-1].batch.groups
+    u32 = lambda t: t.long() & 0xffffffff                     # uint32 payload in an int32 tensor
+    out = {}
+    if run.mode == 0:
+        n_th = len(run.thresholds)
+        out['totals'] = run.totals.view(n_th, 3)
+        out['counts'] = torch.cat([p.counts[:p.batch.groups.n_groups * n_th * 3].view(-1, n_th, 3)
+                                   for p in run.pipes])
+    else:
+        out['spp_hist'] = run.pipes[0].spp_hist
+        out['counts'] = torch.cat([p.counts for p in run.pipes])
+    if run.area_hist is not None:
+        out['area_hist'] = run.area_hist
+    out['area'] = torch.cat([u32(p.table.area[:p.table.n]) for p in run.pipes])
+    out['best_col'] = last.rows.best_col[:g.n_rows]
+    out['best_inter'] = u32(last.rows.best_inter[:g.n_rows])
+    out['best_score'] = last.rows.best_score[:g.n_rows]
+    if last.sparse is not None:
+        out['sparse_row'], out['sparse_col'], out['sparse_inter'] = last.sparse.triplets()
+    elif last.rows.imat is not None and g.imat_off is not None:
+        out['imat'] = last.rows.imat[:g.imat_size]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        if t.numel() > DUMP_CAP:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_CAP, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), t.to(torch.float64).cpu().numpy())
+
+
 def strings_of(batch_dev):
     """Compressed RLE strings of a DeviceBatch (GPU encoder; setup, untimed): (uint8 blob, int32 lengths)."""
     import torch
@@ -804,8 +850,8 @@ def run_c5_strong(args, dev, rank, world, dist, sync):
              for s0 in range(0, mine, by_imat)]
     sub_args = argparse.Namespace(**dict(vars(args), kernel='rows', unfused=False, mma_sort=False))
     run = LayoutRun(sub_args, dev, hosts, engine.LAYOUT_CROP, cfg)
-    passes = 3
-    ms, kt, tot = run.timed(passes, 3, world, dist, sync)
+    passes = args.steps
+    ms, kt, tot = run.timed(passes, args.warmup, world, dist, sync)
     hist = run.area_hist.cpu().numpy()
     return {'workload': 'c5_dataset: %d images of 1024x1024 px, 500 x 500 masks, split over %d GPU(s)' % (total, world),
             'scaling': 'strong', 'images': total, 'images_per_gpu': mine, 'passes_timed': passes,
@@ -901,6 +947,8 @@ def main():
     head = layout_summary(args, run, ms, kt, args.steps, job_images)
     launches = int(args.steps * len(run.subs) * run.kernels_per_sub())
     check = None if (args.no_check or rank != 0) else oracle_sample_check(run)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(run, args.dump_outputs)
 
     # ---- end to end: C ABI from host buffers, and the Python drop-in signature
     e2e = e2e_api = None

@@ -1500,3 +1500,35 @@ def test_many_images_one_call_entry(mods, monkeypatch):
     for got, (a_, b_) in zip(res, [(gt, pr), (cg, cp)]):
         want = mods.R.det_seg_scores(a_, b_, 0.5)
         assert all(np.array_equal(np.asarray(got[k]), np.asarray(want[k])) for k in want)
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: float64 arrays of the last timed step, equal whatever --steps is (the inputs are
+    seeded), under 64 MB; the totals are those of the JSON line and the per-image counts sum to them."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+    def bench(steps, out):
+        cmd = [sys.executable, os.path.join(root, 'bench.py'), '--images', '8', '--steps', str(steps), '--warmup', '1',
+               '--no-cpu', '--no-e2e', '--no-span', '--no-c5', '--no-check', '--dump-outputs', str(out)]
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-800:]
+        return json.loads([l for l in r.stdout.splitlines() if l.startswith('{')][-1])
+
+    a, b = bench(2, tmp_path / 'a'), bench(5, tmp_path / 'b')
+    assert (a['steps'], b['steps']) == (2, 5)
+    names = sorted(os.listdir(tmp_path / 'a'))
+    assert names == sorted(os.listdir(tmp_path / 'b'))
+    assert {'totals.npy', 'counts.npy', 'area.npy', 'best_col.npy', 'best_inter.npy', 'best_score.npy',
+            'imat.npy'} <= set(names)
+    nbytes = 0
+    for n in names:
+        x, y = np.load(tmp_path / 'a' / n), np.load(tmp_path / 'b' / n)
+        assert x.dtype == np.float64 and np.array_equal(x, y), n
+        nbytes += x.nbytes
+    assert nbytes <= 64 << 20
+    totals = np.load(tmp_path / 'a' / 'totals.npy')
+    assert totals[0].tolist() == a['totals_tp_fp_fn_at_0.50']
+    assert np.array_equal(np.load(tmp_path / 'a' / 'counts.npy').sum(axis=0), totals)

@@ -14,13 +14,9 @@ What each test pins, by reference call site:
   test_gpu_path_against_real_pycocotools   the drop-in functions themselves against the reference's loops run on
                                   the real pycocotools (GPU only)
 
-Inputs: the frozen fixtures under tests/golden/ (they travel to the GPU box) and, when /root/reference is present
-(the build container), ALL 6,012 strings of the five prediction pickles and all 2,389 polygons of the four VIA files.
+Inputs: the frozen fixtures under tests/golden/ (3,411 RLE strings cut from the reference's shipped prediction
+pickles, 238 polygons of its VIA validation file).
 """
-import glob
-import json
-import os
-
 import numpy as np
 import pytest
 
@@ -28,15 +24,13 @@ from oracle import ampis_ref as R
 from oracle import cocomask as rle
 from tests import _util as U
 
-REF = '/root/reference/examples'
-
 
 def _real_mask():
     return pytest.importorskip('pycocotools.mask', reason='pycocotools is not installed (parity stays unpinned)')
 
 
 def _fixture_strings():
-    """Every RLE dict available: golden fixtures + (in the build container) all shipped prediction pickles."""
+    """Every RLE dict of the golden fixtures."""
     out = []
     g = U.load('powder_match.npz')
     for k in range(len(g['names'])):
@@ -48,30 +42,16 @@ def _fixture_strings():
     m = U.load('spheroidite_measure.npz')
     for k in range(len(m['names'])):
         out += U.unpack_strings(m['%d_blob' % k], m['%d_off' % k], m['%d_size' % k])
-    if os.path.isdir(REF):
-        from ampis_b200.containers import load_pickle
-        for f in sorted(glob.glob(REF + '/*/data/*.pickle')):
-            for e in load_pickle(f):
-                out += list(e['pred']['instances'].pred_masks)
     return out
 
 
 def _fixture_polygons():
-    """(flat [x0, y0, ...] polygon, (h, w)) pairs: golden fixture + all shipped VIA files."""
+    """(flat [x0, y0, ...] polygon, (h, w)) pairs of the golden fixture."""
     out = []
     p = U.load('powder_polygons.npz')
     for k in range(int(p['n_images'])):
         xy, off, size = p['%d_poly_xy' % k], p['%d_poly_off' % k], tuple(int(v) for v in p['%d_size' % k])
         out += [(xy[off[i]:off[i + 1]].tolist(), size) for i in range(len(off) - 1)]
-    if os.path.isdir(REF):
-        for f in sorted(glob.glob(REF + '/powder/data/via_2.0.8/*.json')):
-            for img in json.load(open(f))['_via_img_metadata'].values():
-                for reg in img['regions']:
-                    sa = reg['shape_attributes']
-                    if sa.get('name') != 'polygon':
-                        continue
-                    poly = np.stack([np.asarray(sa['all_points_x'], float), np.asarray(sa['all_points_y'], float)], 1)
-                    out.append(((poly + 0.5).ravel().tolist(), (1024, 1536)))        # data_utils.py:467
     return out
 
 
