@@ -1228,6 +1228,104 @@ def region_measurements(masks):
             'convex_area': convex[:n].cpu().numpy().astype(np.int64)}
 
 
+#: measurements region_measurements_for can take, each one kernel (or pair of kernels) over one CROP table
+REGION_MEASUREMENTS = ('moments', 'perimeter_hist', 'convex_area', 'moments3', 'filled', 'crofton', 'convex_feret',
+                       'image', 'filled_image')
+#: ampis_rle_moments3 is exact while both sides of the frame stay below this
+MOMENTS3_MAX_SIDE = 65536
+
+
+def _ragged_u8(flat, off, shapes):
+    return [flat[off[i]:off[i + 1]].reshape(shapes[i]).view(np.bool_) for i in range(len(shapes))]
+
+
+def region_measurements_for(masks, need):
+    """Per-mask raw measurements behind compute_rprops for the measurement names in `need` only (see
+    REGION_MEASUREMENTS): one CROP-layout table, then only the launches those names require.  Always present:
+    area[n], bbox[n,4] (x0,y0,x1,y1).  Optional, all exact integers:
+      moments[n,6], perimeter_hist[n,10], convex_area[n]   as region_measurements;
+      moments3: list of n 4x4 nested lists of Python ints, M[p][q] = sum r^p c^q in box-local coordinates;
+      filled: filled_area[n] (binary_fill_holes with an all-ones 3x3 structure);
+      filled_image: list of n bool box images of the filled masks (implies filled);
+      crofton: crofton_trans[n,4], differing pixel pairs along rows, columns, diagonal, anti-diagonal;
+      convex_feret: convex_ranges (list of n int32[box_w, 2] box-local row ranges [lo, hi) of
+        convex_hull_image) and feret_d2[n] = (2 * feret_diameter_max)^2;
+      image: list of n bool box images."""
+    need = set(need)
+    bad = need - set(REGION_MEASUREMENTS)
+    if bad:
+        raise ValueError('unknown region measurements %s' % sorted(bad))
+    if 'filled_image' in need:
+        need.add('filled')
+    t = table_from_rle(masks, layout=LAYOUT_CROP)
+    dev, n = t.device, t.n
+    bb = t.bbox_np()
+    out = {'area': t.areas_np().astype(np.int64), 'bbox': bb}
+    bw = np.maximum(bb[:, 2] - bb[:, 0] + 1, 0).astype(np.int64)
+    bh = np.where(bw > 0, bb[:, 3] - bb[:, 1] + 1, 0).astype(np.int64)
+    if 'moments' in need:
+        mom = torch.empty(max(6 * n, 1), dtype=torch.int64, device=dev)
+        N.call('ampis_rle_moments', _p(t.cum), _p(t.cnt_off), _p(t.cnt_len), _p(t.h), n, _p(mom), _stream())
+        out['moments'] = mom[:6 * n].cpu().numpy().view(np.uint64).reshape(n, 6)
+    if 'moments3' in need:
+        if n and max(int(t.h[:n].max().item()), int(t.w[:n].max().item())) > MOMENTS3_MAX_SIDE:
+            raise ValueError('moments to order 3 are exact for frames up to %d pixels a side' % MOMENTS3_MAX_SIDE)
+        m3 = torch.empty(max(32 * n, 1), dtype=torch.int64, device=dev)
+        N.call('ampis_rle_moments3', _p(t.cum), _p(t.cnt_off), _p(t.cnt_len), _p(t.h), _p(t.bbox), n, _p(m3),
+               _stream())
+        halves = m3[:32 * n].cpu().numpy().view(np.uint64).reshape(n, 16, 2).tolist()
+        out['moments3'] = [[[lo | (hi << 64) for lo, hi in row[4 * p:4 * p + 4]] for p in range(4)] for row in halves]
+    if 'perimeter_hist' in need:
+        border = torch.empty_like(t.bits)
+        hist = torch.empty(max(10 * n, 1), dtype=torch.int32, device=dev)
+        N.call('ampis_crop_perimeter', _p(t.bits), _p(t.bits_off), _p(t.bbox), n, _p(border), _p(hist), _stream())
+        out['perimeter_hist'] = hist[:10 * n].cpu().numpy().reshape(n, 10).astype(np.int64)
+    if 'filled' in need or 'crofton' in need:
+        filled = torch.zeros_like(t.bits) if 'filled' in need else None
+        farea = torch.empty(max(n, 1), dtype=torch.int64, device=dev) if 'filled' in need else None
+        trans = torch.empty(max(4 * n, 1), dtype=torch.int64, device=dev) if 'crofton' in need else None
+        N.call('ampis_crop_fill_holes', _p(t.bits), _p(t.bits_off), _p(t.bbox), n, _p(filled), _p(farea), _p(trans),
+               _stream())
+        if filled is not None:
+            out['filled_area'] = farea[:n].cpu().numpy()
+        if trans is not None:
+            out['crofton_trans'] = trans[:4 * n].cpu().numpy().reshape(n, 4)
+    if 'convex_area' in need or 'convex_feret' in need:
+        off = np.zeros(n + 1, np.int64)
+        np.cumsum(10 * bw + 4, out=off[1:])
+        scratch = torch.empty(max(int(off[n]), 1), dtype=torch.int32, device=dev)
+        d_off = _dev(off[:n], torch.int64, dev)          # named: a temporary would be recycled before the launch
+        if 'convex_area' in need:
+            convex = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
+            N.call('ampis_crop_convex_area', _p(t.bits), _p(t.bits_off), _p(t.bbox), n, _p(d_off), _p(scratch),
+                   _p(convex), _stream())
+            out['convex_area'] = convex[:n].cpu().numpy().astype(np.int64)
+        if 'convex_feret' in need:
+            col_off = np.zeros(n + 1, np.int64)
+            np.cumsum(bw, out=col_off[1:])
+            d_col = _dev(col_off[:n], torch.int64, dev)
+            ranges = torch.empty(max(2 * int(col_off[n]), 1), dtype=torch.int32, device=dev)
+            d2 = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
+            N.call('ampis_crop_convex_feret', _p(t.bits), _p(t.bits_off), _p(t.bbox), n, _p(d_off), _p(scratch),
+                   _p(d_col), _p(ranges), _p(d2), _stream())
+            rg = ranges[:2 * int(col_off[n])].cpu().numpy().reshape(-1, 2)
+            out['convex_ranges'] = [rg[col_off[i]:col_off[i + 1]] for i in range(n)]
+            out['feret_d2'] = d2[:n].cpu().numpy()
+    if 'image' in need or 'filled_image' in need:
+        img_off = np.zeros(n + 1, np.int64)
+        np.cumsum(bh * bw, out=img_off[1:])
+        d_img_off = _dev(img_off[:n], torch.int64, dev)
+        shapes = list(zip(bh.tolist(), bw.tolist()))
+        for key, src in (('image', t.bits), ('filled_image', filled if 'filled_image' in need else None)):
+            if key not in need:
+                continue
+            img = torch.empty(max(int(img_off[n]), 1), dtype=torch.uint8, device=dev)
+            N.call('ampis_crop_unpack_image', _p(src), _p(t.bits_off), _p(t.bbox), n, _p(d_img_off), _p(img),
+                   _stream())
+            out[key] = _ragged_u8(to_host(img[:int(img_off[n])]), img_off, shapes)
+    return out
+
+
 def polygons_to_bool(polys, h, w):
     """list of flat [x0,y0,x1,y1,...] polygons -> bool[n, h, w] host array by skimage's polygon2mask
     rule (structures._poly2mask), rasterised on the GPU."""

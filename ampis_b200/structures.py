@@ -164,19 +164,31 @@ class InstanceSet(object):
         inlier_instances = ~touches
         self.instances = self.instances[inlier_instances]
 
-    #: region properties compute_rprops derives from the GPU measurements (skimage names)
+    #: region properties compute_rprops derives from the GPU measurements (skimage names): every non-intensity
+    #: property of scikit-image 0.18.3 except euler_number
     RPROPS_GPU_KEYS = ('area', 'bbox', 'bbox_area', 'centroid', 'local_centroid', 'convex_area', 'eccentricity',
                        'equivalent_diameter', 'extent', 'label', 'major_axis_length', 'minor_axis_length',
-                       'orientation', 'perimeter', 'solidity')
+                       'orientation', 'perimeter', 'solidity', 'moments', 'moments_central', 'moments_normalized',
+                       'moments_hu', 'inertia_tensor', 'inertia_tensor_eigvals', 'filled_area', 'filled_image',
+                       'perimeter_crofton', 'feret_diameter_max', 'convex_image', 'image', 'coords', 'slice')
+    #: properties regionprops_table keeps whole, one object cell per region
+    RPROPS_OBJECT_KEYS = ('image', 'filled_image', 'convex_image', 'coords', 'slice')
+    #: shape of the array-valued properties, split into key-i(-j) columns; integer-valued properties
+    _RPROPS_SHAPES = {'bbox': (4,), 'centroid': (2,), 'local_centroid': (2,), 'moments': (4, 4),
+                      'moments_central': (4, 4), 'moments_normalized': (4, 4), 'moments_hu': (7,),
+                      'inertia_tensor': (2, 2), 'inertia_tensor_eigvals': (2,)}
+    _RPROPS_INT_KEYS = ('area', 'bbox', 'bbox_area', 'convex_area', 'label', 'filled_area')
 
     def compute_rprops(self, keys=None, return_df=False):
         """Region properties per mask (reference structures.py:474-514, which decodes every mask to a
         full int64 frame and runs skimage.measure.regionprops_table on it).  Here the GPU delivers
         exact integer measurements from the run table and the packed bounding-box windows
-        (csrc/rprops.cu: raw moments, perimeter histogram, convex-hull pixel count) and the
-        properties are formed on the host with skimage 0.18.3's formulas.  Default keys are the
-        reference's; cells are 1-element arrays (empty for an empty mask) as regionprops_table
-        returns them; tuple-valued properties become ``key-0``, ``key-1`` ... columns."""
+        (csrc/rprops.cu: raw moments, perimeter histogram, convex hull, hole fill, Crofton transitions,
+        Feret diameter, box images) and the properties are formed on the host with skimage 0.18.3's
+        formulas.  Default keys are the reference's; cells are 1-element arrays (empty for an empty mask)
+        as regionprops_table returns them; tuple- and array-valued properties become ``key-0``, ``key-1``
+        ... (``key-0-0`` ... for 2-D arrays) columns, and image, filled_image, convex_image, coords and slice
+        one column of 1-element object arrays."""
         if keys is None:
             keys = ['area', 'equivalent_diameter', 'major_axis_length', 'perimeter', 'solidity', 'orientation']
         unsupported = [k for k in keys if k not in self.RPROPS_GPU_KEYS]
@@ -186,24 +198,29 @@ class InstanceSet(object):
         rle = masks_to_rle(self.instances.masks, self.instances.image_size)
         if type(rle) == dict:
             rle = [rle]
-        props = region_properties(rle)
+        props = region_properties(rle, keys)
         rows = []
         for p in props:
             row = {}
             for k in keys:
                 v = p.get(k)
-                if isinstance(v, tuple):
-                    for j, x in enumerate(v):
-                        row['%s-%d' % (k, j)] = np.array([x])
+                if k in self.RPROPS_OBJECT_KEYS:
+                    cell = np.empty(1 if v is not None else 0, dtype=object)
+                    if v is not None:
+                        cell[0] = v
+                    row[k] = cell
                 elif v is None:            # empty mask: regionprops finds no region
-                    width = {'bbox': 4, 'centroid': 2, 'local_centroid': 2}.get(k, 0)
-                    empty = np.array([], np.int64 if k in ('area', 'bbox', 'bbox_area', 'convex_area', 'label')
-                                     else np.float64)
-                    if width:
-                        for j in range(width):
-                            row['%s-%d' % (k, j)] = empty
+                    empty = np.array([], np.int64 if k in self._RPROPS_INT_KEYS else np.float64)
+                    shape = self._RPROPS_SHAPES.get(k)
+                    if shape:
+                        for loc in np.ndindex(shape):
+                            row['-'.join(map(str, (k,) + loc))] = empty
                     else:
                         row[k] = empty
+                elif isinstance(v, (tuple, list, np.ndarray)):
+                    a = np.asarray(v)
+                    for loc in np.ndindex(a.shape):
+                        row['-'.join(map(str, (k,) + loc))] = np.array([a[loc].item()])
                 else:
                     row[k] = np.array([v])
             rows.append(row)
@@ -326,45 +343,160 @@ def masks_to_bitmask_array(masks, size=None):
 
 
 _PERIMETER_CODES = [5, 7, 15, 17, 25, 27, 21, 33, 13, 23]
+_PERIMETER_WEIGHTS = np.zeros(50, dtype=np.double)
+_PERIMETER_WEIGHTS[[5, 7, 15, 17, 25, 27]] = 1
+_PERIMETER_WEIGHTS[[21, 33]] = np.sqrt(2)
+_PERIMETER_WEIGHTS[[13, 23]] = (1 + np.sqrt(2)) / 2
+
+#: the GPU measurements (engine.REGION_MEASUREMENTS) each region property is formed from
+_MEASUREMENTS_OF = {
+    'area': (), 'bbox': (), 'bbox_area': (), 'equivalent_diameter': (), 'extent': (), 'label': (), 'slice': (),
+    'centroid': ('moments',), 'local_centroid': ('moments',), 'eccentricity': ('moments',),
+    'major_axis_length': ('moments',), 'minor_axis_length': ('moments',), 'orientation': ('moments',),
+    'inertia_tensor': ('moments',), 'inertia_tensor_eigvals': ('moments',),
+    'perimeter': ('perimeter_hist',), 'convex_area': ('convex_area',), 'solidity': ('convex_area',),
+    'moments': ('moments3',), 'moments_central': ('moments3',), 'moments_normalized': ('moments3',),
+    'moments_hu': ('moments3',), 'filled_area': ('filled',), 'filled_image': ('filled_image',),
+    'perimeter_crofton': ('crofton',), 'feret_diameter_max': ('convex_feret',), 'convex_image': ('convex_feret',),
+    'image': ('image',), 'coords': ('image',),
+}
+_DEFAULT_KEYS = ('area', 'bbox', 'bbox_area', 'centroid', 'local_centroid', 'convex_area', 'eccentricity',
+                 'equivalent_diameter', 'extent', 'major_axis_length', 'minor_axis_length', 'orientation', 'perimeter',
+                 'solidity', 'label')
 
 
-def region_properties(rle):
+def _box_props(n, bb):
+    x0, y0, x1, y1 = (int(v) for v in bb)
+    bbox_area = (y1 - y0 + 1) * (x1 - x0 + 1)
+    return {'area': n, 'bbox': (y0, x0, y1 + 1, x1 + 1), 'bbox_area': bbox_area,
+            'equivalent_diameter': float(np.sqrt(4 * n / np.pi)), 'extent': n / bbox_area, 'label': 1,
+            'slice': (slice(y0, y1 + 1), slice(x0, x1 + 1))}
+
+
+def _second_order_props(mom, y0, x0):
+    """Centroids, inertia tensor and the ellipse properties from the exact order-2 raw moments."""
+    N, Sx, Sy, Sxx, Syy, Sxy = (int(v) for v in mom)
+    # central second moments times N, exact integers: N*mu20 = N*Syy - Sy^2, ...
+    n_rr, n_cc, n_rc = N * Syy - Sy * Sy, N * Sxx - Sx * Sx, N * Sxy - Sx * Sy
+    a, c, b = n_cc / (N * N), n_rr / (N * N), -(n_rc / (N * N))    # inertia tensor [[a, b], [b, c]]; -0.0 kept
+    half_tr, half_diff = (a + c) / 2, (a - c) / 2
+    l1 = half_tr + np.sqrt(half_diff * half_diff + b * b)
+    det = (n_cc * n_rr - n_rc * n_rc) / (N ** 4)                    # exact numerator: no cancellation
+    l2 = max(det / l1, 0.0) if l1 > 0 else 0.0
+    if n_cc == n_rr:
+        orientation = -np.pi / 4. if b < 0 else np.pi / 4.
+    else:
+        orientation = 0.5 * np.arctan2(-2 * b, c - a)
+    return {'centroid': (Sy / N, Sx / N), 'local_centroid': ((Sy - N * y0) / N, (Sx - N * x0) / N),
+            'eccentricity': 0. if l1 == 0 else float(np.sqrt(1 - l2 / l1)),
+            'major_axis_length': float(4 * np.sqrt(l1)), 'minor_axis_length': float(4 * np.sqrt(l2)),
+            'orientation': float(orientation), 'inertia_tensor': np.array([[a, b], [b, c]]),
+            'inertia_tensor_eigvals': [float(l1), float(l2)]}
+
+
+_BINOM = [[1], [1, 1], [1, 2, 1], [1, 3, 3, 1]]
+
+
+def _moment_props(M):
+    """moments, moments_central, moments_normalized, moments_hu (skimage 0.18.3) from the exact box-local raw
+    moments M[p][q] = sum r^p c^q (Python ints).  The central moments are expanded exactly about the rational
+    centroid -- N^(p+q) mu[p][q] is an integer -- and rounded once."""
+    N, Sr, Sc = M[0][0], M[1][0], M[0][1]
+    mu = np.zeros((4, 4))
+    for p in range(4):
+        for q in range(4):
+            num = 0
+            for i in range(p + 1):
+                for j in range(q + 1):
+                    num += _BINOM[p][i] * _BINOM[q][j] * (-Sr) ** (p - i) * (-Sc) ** (q - j) * N ** (i + j) * M[i][j]
+            mu[p, q] = num / N ** (p + q)
+    nu = np.full((4, 4), np.nan)
+    for p in range(4):
+        for q in range(4):
+            if p + q >= 2:
+                nu[p, q] = mu[p, q] / (mu[0, 0] ** ((p + q) / 2 + 1))
+    return {'moments': np.array(M, dtype=np.float64), 'moments_central': mu, 'moments_normalized': nu,
+            'moments_hu': _hu(nu)}
+
+
+def _hu(nu):
+    """skimage 0.18.3 measure._moments_cy.moments_hu, in its order of operations."""
+    hu = np.zeros((7,), dtype=np.double)
+    t0 = nu[3, 0] + nu[1, 2]
+    t1 = nu[2, 1] + nu[0, 3]
+    q0 = t0 * t0
+    q1 = t1 * t1
+    n4 = 4 * nu[1, 1]
+    s = nu[2, 0] + nu[0, 2]
+    d = nu[2, 0] - nu[0, 2]
+    hu[0] = s
+    hu[1] = d * d + n4 * nu[1, 1]
+    hu[3] = q0 + q1
+    hu[5] = d * (q0 - q1) + n4 * t0 * t1
+    t0 *= q0 - 3 * q1
+    t1 *= 3 * q0 - q1
+    q0 = nu[3, 0] - 3 * nu[1, 2]
+    q1 = 3 * nu[2, 1] - nu[0, 3]
+    hu[2] = q0 * q0 + q1 * q1
+    hu[4] = q0 * t0 + q1 * t1
+    hu[6] = q1 * t0 - q0 * t1
+    return hu
+
+
+_CROFTON_SCALE = np.pi / 8
+
+
+def region_properties(rle, keys=None):
     """skimage 0.18.3 region properties of every mask of an RLE list (one region per mask, as
     ``regionprops_table(mask.astype(int))`` sees it) from the exact GPU measurements.  Returns one
-    dict per mask ({} for an empty mask)."""
-    m = engine.region_measurements(rle)
-    weights = np.zeros(50, dtype=np.double)
-    weights[[5, 7, 15, 17, 25, 27]] = 1
-    weights[[21, 33]] = np.sqrt(2)
-    weights[[13, 23]] = (1 + np.sqrt(2)) / 2
+    dict per mask ({} for an empty mask).  keys=None: the fifteen scalar and tuple properties of
+    _DEFAULT_KEYS; otherwise the listed properties of InstanceSet.RPROPS_GPU_KEYS, and only the GPU
+    measurements those need are taken."""
+    if keys is None:
+        m = engine.region_measurements(rle)
+        keys = _DEFAULT_KEYS
+    else:
+        keys = list(keys)
+        unknown = [k for k in keys if k not in _MEASUREMENTS_OF]
+        if unknown:
+            raise NotImplementedError('region properties %s are not part of the GPU path' % unknown)
+        m = engine.region_measurements_for(rle, {x for k in keys for x in _MEASUREMENTS_OF[k]})
     out = []
     for i in range(len(rle)):
         n = int(m['area'][i])
         if n == 0:
             out.append({})
             continue
-        x0, y0, x1, y1 = (int(v) for v in m['bbox'][i])
-        N, Sx, Sy, Sxx, Syy, Sxy = (int(v) for v in m['moments'][i])
-        # central second moments times N, exact integers: N*mu20 = N*Syy - Sy^2, ...
-        n_rr, n_cc, n_rc = N * Syy - Sy * Sy, N * Sxx - Sx * Sx, N * Sxy - Sx * Sy
-        a, c, b = n_cc / (N * N), n_rr / (N * N), -(n_rc / (N * N))    # inertia tensor [[a, b], [b, c]]; -0.0 kept
-        half_tr, half_diff = (a + c) / 2, (a - c) / 2
-        l1 = half_tr + np.sqrt(half_diff * half_diff + b * b)
-        det = (n_cc * n_rr - n_rc * n_rc) / (N ** 4)                    # exact numerator: no cancellation
-        l2 = max(det / l1, 0.0) if l1 > 0 else 0.0
-        if n_cc == n_rr:
-            orientation = -np.pi / 4. if b < 0 else np.pi / 4.
-        else:
-            orientation = 0.5 * np.arctan2(-2 * b, c - a)
-        hist = np.zeros(50, np.int64)
-        hist[_PERIMETER_CODES] = m['perimeter_hist'][i]
-        convex_area = int(m['convex_area'][i])
-        bbox_area = (y1 - y0 + 1) * (x1 - x0 + 1)
-        out.append({'area': n, 'bbox': (y0, x0, y1 + 1, x1 + 1), 'bbox_area': bbox_area,
-                    'centroid': (Sy / N, Sx / N), 'local_centroid': ((Sy - N * y0) / N, (Sx - N * x0) / N),
-                    'convex_area': convex_area, 'eccentricity': 0. if l1 == 0 else float(np.sqrt(1 - l2 / l1)),
-                    'equivalent_diameter': float(np.sqrt(4 * n / np.pi)), 'extent': n / bbox_area,
-                    'major_axis_length': float(4 * np.sqrt(l1)), 'minor_axis_length': float(4 * np.sqrt(l2)),
-                    'orientation': float(orientation), 'perimeter': float(hist @ weights),
-                    'solidity': n / convex_area, 'label': 1})
+        bb = m['bbox'][i]
+        x0, y0 = int(bb[0]), int(bb[1])
+        p = _box_props(n, bb)
+        if 'moments' in m:
+            p.update(_second_order_props(m['moments'][i], y0, x0))
+        if 'perimeter_hist' in m:
+            hist = np.zeros(50, np.int64)
+            hist[_PERIMETER_CODES] = m['perimeter_hist'][i]
+            p['perimeter'] = float(hist @ _PERIMETER_WEIGHTS)
+        if 'convex_area' in m:
+            p['convex_area'] = int(m['convex_area'][i])
+            p['solidity'] = n / p['convex_area']
+        if 'moments3' in m:
+            p.update(_moment_props(m['moments3'][i]))
+        if 'filled_area' in m:
+            p['filled_area'] = int(m['filled_area'][i])
+        if 'filled_image' in m:
+            p['filled_image'] = m['filled_image'][i]
+        if 'crofton_trans' in m:
+            t = m['crofton_trans'][i]
+            p['perimeter_crofton'] = float(_CROFTON_SCALE * (int(t[0]) + int(t[1]) + (int(t[2]) + int(t[3])) / np.sqrt(2)))
+        if 'feret_d2' in m:
+            p['feret_diameter_max'] = float(np.sqrt(float(m['feret_d2'][i]))) / 2
+            rg = m['convex_ranges'][i]
+            rows = np.arange(int(bb[3]) - y0 + 1)[:, None]
+            p['convex_image'] = (rows >= rg[:, 0]) & (rows < rg[:, 1])
+        if 'image' in m:
+            img = m['image'][i]
+            p['image'] = img
+            r, c = np.nonzero(img)
+            p['coords'] = np.stack([r + y0, c + x0], axis=1).astype(np.int64)
+        out.append({k: p[k] for k in keys})
     return out

@@ -439,6 +439,30 @@ int ampis_crop_convex_area(const void *d_bits, const int64_t *d_bits_off, const 
                            const int64_t *d_scratch_off, int32_t *d_scratch, uint64_t *d_convex_area,
                            void *stream);
 
+/* The remaining non-intensity region properties (all but euler_number), same tables:
+ * ampis_rle_moments3: skimage's `moments` to order 3 in box-local coordinates, exact: d_out[32*i + 2*k],
+ *   [32*i + 2*k + 1] = low / high 64 bits of M[p][q] = sum r^p c^q, k = 4p + q, r = row - y0,
+ *   c = column - x0 (d_bbox of ampis_rle_measure).  Exact while both frame sides are <= 65536.
+ * ampis_crop_fill_holes (AMPIS_LAYOUT_CROP table): d_filled (size of the bits arena, same offsets and layout;
+ *   may be null together with d_filled_area) = scipy.ndimage.binary_fill_holes(box image,
+ *   structure=ones((3,3))), d_filled_area[i] its pixel count; d_trans (may be null) = 4 counts per mask of
+ *   pixel pairs that differ, outside the box = 0: along rows, along columns, along (r+1, c+1), along (r+1, c-1)
+ *   -- perimeter_crofton(directions=4) = pi/8 * (t0 + t1 + (t2 + t3) / sqrt 2).
+ * ampis_crop_convex_feret: convex_hull_image as row ranges [lo, hi) (box-local; lo == hi for an empty
+ *   column) at d_ranges[2 * (d_col_off[i] + c)], and d_feret_d2[i] = (2 * feret_diameter_max)^2 as an exact
+ *   integer; scratch as for ampis_crop_convex_area.
+ * ampis_crop_unpack_image: the box image of every mask as row-major 0/1 bytes at d_img + d_img_off[i]
+ *   (box_h * box_w bytes; pass the filled arena of ampis_crop_fill_holes as d_bits for filled_image). */
+int ampis_rle_moments3(const uint32_t *d_cum, const int64_t *d_cnt_off, const int32_t *d_cnt_len,
+                       const uint32_t *d_h, const int32_t *d_bbox, int32_t n, uint64_t *d_out, void *stream);
+int ampis_crop_fill_holes(const void *d_bits, const int64_t *d_bits_off, const int32_t *d_bbox, int32_t n,
+                          void *d_filled, uint64_t *d_filled_area, uint64_t *d_trans, void *stream);
+int ampis_crop_convex_feret(const void *d_bits, const int64_t *d_bits_off, const int32_t *d_bbox, int32_t n,
+                            const int64_t *d_scratch_off, int32_t *d_scratch, const int64_t *d_col_off,
+                            int32_t *d_ranges, uint64_t *d_feret_d2, void *stream);
+int ampis_crop_unpack_image(const void *d_bits, const int64_t *d_bits_off, const int32_t *d_bbox, int32_t n,
+                            const int64_t *d_img_off, uint8_t *d_img, void *stream);
+
 /* ---- annotation images -> instances (data_utils.get_ddicts 'binary' / 'label', data_utils.py:394-433) ----
  * ampis_ccl_label: skimage.measure.label of a binary image (row-major u8[h][w], non-zero = foreground,
  *   full 8-connectivity, labels 1..n in raster order of each component's first pixel).  d_work i32[h*w],
