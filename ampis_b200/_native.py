@@ -77,6 +77,7 @@ SIGNATURES = {
     'ampis_crop_fill_holes': (C.c_int, [_p, _p, _p, _i32, _p, _p, _p, _p]),
     'ampis_crop_convex_feret': (C.c_int, [_p, _p, _p, _i32, _p, _p, _p, _p, _p, _p]),
     'ampis_crop_unpack_image': (C.c_int, [_p, _p, _p, _i32, _p, _p, _p]),
+    'ampis_rle_intensity': (C.c_int, [_p, _p, _p, _p, _p, _i32, _p, _i32, _p, _i32, _p, _p, _p]),
     'ampis_ccl_label': (C.c_int, [_p, _i32, _i32, _p, _p, _p, _p, C.c_size_t, _p, _p]),
     'ampis_label_values_present': (C.c_int, [_p, _i64, _p, _i32, _p, _p]),
     'ampis_label_dense': (C.c_int, [_p, _p, _i32, _i32, _i32, _p, _p]),

@@ -14,7 +14,14 @@
 // The remaining non-intensity properties (below, after the C entries of the above): moments to order 3 as
 // exact 128-bit sums from the runs; hole fill and Crofton transition counts on the CROP windows; the convex
 // image as per-column row ranges plus the maximum Feret diameter as an exact integer; box images unpacked
-// from the windows for image / coords / filled_image.
+// from the windows for image / coords / filled_image.  The intensity properties (last section): min, max and the
+// weighted moments of an intensity image over every mask, from the run table -- exact for integer pixels.
+#include <cuda_fp16.h>
+#include <math_constants.h>
+
+#include <climits>
+#include <type_traits>
+
 #include "common.cuh"
 
 // ---- moments from runs: warp per mask ---------------------------------------------------------
@@ -650,4 +657,275 @@ extern "C" int ampis_crop_unpack_image(const void *d_bits, const int64_t *d_bits
                                                                          (const int4 *)d_bbox, d_img_off, d_img);
     AMPIS_CHECK_LAUNCH("crop_unpack_image_kernel");
     return AMPIS_OK;
+}
+
+// ==== intensity properties (regionprops with intensity_image) ==========================================
+// Warp per mask over its run table: the lanes walk the 1-runs together, cut at column boundaries into vertical
+// segments, and read the pixels of a segment side by side -- coalesced, because the image is column-major on the
+// device (pixel (row y, column x) at x * h + y, the order of the run positions).  Per column every lane keeps
+// P[p] = sum I r^p of its pixels; when the column changes, P is folded into S[p][q] += P[p] c^q.
+//   integer pixels: exact.  A lane may read any subset of the rows of a column (a column of many short segments
+//     restarts every segment at lane 0), so its P[p] is bounded by the whole column: |P[3]| <= 2^64 sum_{r<2^16} r^3
+//     < 2^126, inside the signed 128-bit P and i192_add_prod's mag < 2^127.  S[p][q] < 2^64 (sum_r r^3) (sum_c c^3)
+//     < 2^188 is kept as a signed 192-bit integer.  8- and 16-bit pixels take their products I r^p in 64 bits.
+//   float pixels: float64 sums, about a given centre (the second, central pass) or about (0, 0).
+typedef __int128 i128;
+
+template <typename T> struct PixFloat {
+    static constexpr bool value = std::is_floating_point<T>::value || std::is_same<T, __half>::value;
+};
+template <typename T> __device__ __forceinline__ double pix_f64(T v) { return (double)v; }
+template <> __device__ __forceinline__ double pix_f64<__half>(__half v) { return (double)__half2float(v); }
+
+// signed 192-bit integer in two's complement: lo = bits 0..127, hi = bits 128..191
+struct I192 {
+    u128 lo;
+    u64 hi;
+};
+
+// s += (neg ? -1 : 1) * mag * m  (mag < 2^127, m < 2^64)
+__device__ __forceinline__ void i192_add_prod(I192 &s, u128 mag, u64 m, bool neg)
+{
+    const u128 a = (u128)(u64)mag * m, b = (u128)(u64)(mag >> 64) * m;      // mag * m = a + b 2^64
+    const u128 lo = a + (b << 64);
+    const u64 hi = (u64)(b >> 64) + (lo < a ? 1u : 0u);
+    if (neg) {
+        const u128 t = s.lo - lo;
+        s.hi -= hi + (t > s.lo ? 1u : 0u);
+        s.lo = t;
+    } else {
+        const u128 t = s.lo + lo;
+        s.hi += hi + (t < s.lo ? 1u : 0u);
+        s.lo = t;
+    }
+}
+
+__device__ __forceinline__ void i192_shfl_add(I192 &s, int d)
+{
+    const u128 olo = shfl_xor_u128(s.lo, d);
+    const u64 ohi = __shfl_xor_sync(0xffffffffu, s.hi, d);
+    const u128 t = s.lo + olo;
+    s.hi += ohi + (t < s.lo ? 1u : 0u);
+    s.lo = t;
+}
+
+// I * rp exactly (rp < 2^48)
+template <typename T> __device__ __forceinline__ i128 pix_mul(T v, u64 rp)
+{
+    if constexpr (sizeof(T) <= 2) {
+        if constexpr (std::is_signed<T>::value) return (i128)((i64)v * (i64)rp);      // |I rp| < 2^63
+        else return (i128)((u64)v * rp);                                              // I rp < 2^64
+    } else if constexpr (std::is_signed<T>::value) {
+        const u64 mag = v < 0 ? (u64)0 - (u64)(i64)v : (u64)(i64)v;
+        const i128 p = (i128)((u128)mag * rp);
+        return v < 0 ? -p : p;
+    } else {
+        return (i128)((u128)(u64)v * rp);
+    }
+}
+
+template <typename T, bool FLT = PixFloat<T>::value, bool SIGNED = std::is_signed<T>::value>
+struct PixStats;                                    // min / max in the widest type of the pixel's kind
+template <typename T, bool SIGNED> struct PixStats<T, true, SIGNED> {
+    typedef double W;
+    static __device__ __forceinline__ W lo() { return -CUDART_INF; }
+    static __device__ __forceinline__ W hi() { return CUDART_INF; }
+};
+template <typename T> struct PixStats<T, false, true> {
+    typedef long long W;
+    static __device__ __forceinline__ W lo() { return LLONG_MIN; }
+    static __device__ __forceinline__ W hi() { return LLONG_MAX; }
+};
+template <typename T> struct PixStats<T, false, false> {
+    typedef unsigned long long W;
+    static __device__ __forceinline__ W lo() { return 0; }
+    static __device__ __forceinline__ W hi() { return ULLONG_MAX; }
+};
+
+// moments: integer pixels 48 u64 per mask (M[p][q] as 3 limbs, low first, k = 4p + q), float pixels 16 f64.
+// stats (raw pass only; 4 x 8 bytes per mask): min, max (long long / unsigned long long / double; NaN when the
+// mask holds a NaN pixel), non-finite pixels of the mask, non-finite pixels of the box (0 unless scan_box).
+template <typename T>
+__global__ void __launch_bounds__(256)
+rle_intensity_kernel(const u32 *__restrict__ cum, const i64 *__restrict__ cnt_off, const int *__restrict__ cnt_len,
+                     const u32 *__restrict__ hh, const int4 *__restrict__ bbox, int n, const T *__restrict__ img,
+                     const double *__restrict__ center, int scan_box, void *__restrict__ moments,
+                     unsigned long long *__restrict__ stats)
+{
+    constexpr bool FLT = PixFloat<T>::value;
+    typedef typename PixStats<T>::W W;
+    typedef typename std::conditional<FLT, double, i128>::type Part;
+    typedef typename std::conditional<FLT, double, I192>::type Sum;
+    const int i = (int)((blockIdx.x * (u32)blockDim.x + threadIdx.x) >> 5);
+    if (i >= n) return;
+    const u32 lane = lane_id();
+    const u32 *C = cum + cnt_off[i];
+    const int m = cnt_len[i];
+    const u64 H = hh[i];
+    const int4 bb = bbox[i];
+    const double cr = center ? center[2 * (i64)i] : 0.0, cc = center ? center[2 * (i64)i + 1] : 0.0;
+    Part P[4];
+    Sum S[16];
+#pragma unroll
+    for (int k = 0; k < 4; k++) P[k] = Part();
+#pragma unroll
+    for (int k = 0; k < 16; k++) S[k] = Sum();
+    W mn = PixStats<T>::hi(), mx = PixStats<T>::lo();
+    bool nan = false;
+    unsigned long long nf_mask = 0, nf_box = 0;
+
+    auto fold = [&](int x) {                       // S[p][q] += P[p] c^q, P = 0
+        if constexpr (FLT) {
+            const double c = (double)(x - bb.x) - cc, c2 = c * c;
+            const double cq[4] = {1.0, c, c2, c2 * c};
+#pragma unroll
+            for (int p = 0; p < 4; p++) {
+#pragma unroll
+                for (int q = 0; q < 4; q++) S[4 * p + q] += q ? P[p] * cq[q] : P[p];
+                P[p] = 0.0;
+            }
+        } else {
+            const u64 c = (u64)(x - bb.x);
+            const u64 cq[4] = {1, c, c * c, c * c * c};
+#pragma unroll
+            for (int p = 0; p < 4; p++) {
+                const bool neg = P[p] < 0;
+                const u128 mag = neg ? (u128)0 - (u128)P[p] : (u128)P[p];
+#pragma unroll
+                for (int q = 0; q < 4; q++) i192_add_prod(S[4 * p + q], mag, cq[q], neg);
+                P[p] = 0;
+            }
+        }
+    };
+
+    int col = -1;
+    for (int r = 1; r < m; r += 2) {                               // odd runs are the 1-runs; warp-uniform
+        u64 p = C[r - 1];
+        const u64 e = C[r];
+        while (p < e) {
+            const u64 x = p / H, cs = x * H;
+            const u64 b = min(e, cs + H) - cs;                     // rows [p - cs, b) of column x
+            if ((int)x != col) {
+                if (col >= 0) fold(col);
+                col = (int)x;
+            }
+            for (u64 y = p - cs + lane; y < b; y += 32) {
+                const T v = img[cs + y];
+                const u32 rl = (u32)y - (u32)bb.y;
+                if constexpr (FLT) {
+                    const double w = pix_f64(v);
+                    if (!center) {
+                        if (isnan(w)) nan = true;
+                        if (!isfinite(w)) nf_mask++;
+                        mn = fmin(mn, w);
+                        mx = fmax(mx, w);
+                    }
+                    const double d = (double)rl - cr, d2 = d * d;
+                    P[0] += w;
+                    P[1] += w * d;
+                    P[2] += w * d2;
+                    P[3] += w * (d2 * d);
+                } else {
+                    const W w = (W)v;
+                    mn = min(mn, w);
+                    mx = max(mx, w);
+                    const u64 r2 = (u64)rl * rl;
+                    P[0] += pix_mul(v, 1);
+                    P[1] += pix_mul(v, rl);
+                    P[2] += pix_mul(v, r2);
+                    P[3] += pix_mul(v, r2 * rl);
+                }
+            }
+            p = cs + H;
+        }
+    }
+    if (col >= 0) fold(col);
+    if constexpr (FLT) {
+        if (!center && scan_box) {                                 // skimage multiplies the whole box by the mask:
+            for (int x = bb.x; x <= bb.z; x++) {                   // a NaN or inf outside the mask turns into NaN
+                for (u32 y = (u32)bb.y + lane; y <= (u32)bb.w; y += 32)
+                    if (!isfinite(pix_f64(img[(u64)x * H + y]))) nf_box++;
+            }
+        }
+    }
+
+#pragma unroll
+    for (int k = 0; k < 16; k++) {
+#pragma unroll
+        for (int d = 16; d; d >>= 1) {
+            if constexpr (FLT) S[k] += __shfl_xor_sync(0xffffffffu, S[k], d);
+            else i192_shfl_add(S[k], d);
+        }
+    }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) {
+        const W omn = __shfl_xor_sync(0xffffffffu, mn, d), omx = __shfl_xor_sync(0xffffffffu, mx, d);
+        if constexpr (FLT) { mn = fmin(mn, omn); mx = fmax(mx, omx); }
+        else { mn = min(mn, omn); mx = max(mx, omx); }
+        nf_mask += __shfl_xor_sync(0xffffffffu, nf_mask, d);
+        nf_box += __shfl_xor_sync(0xffffffffu, nf_box, d);
+    }
+    nan = __any_sync(0xffffffffu, nan);
+    if (lane != 0) return;
+    if constexpr (FLT) {
+        double *M = (double *)moments + 16 * (i64)i;
+#pragma unroll
+        for (int k = 0; k < 16; k++) M[k] = S[k];
+        if (nan) mn = mx = CUDART_NAN;
+    } else {
+        unsigned long long *M = (unsigned long long *)moments + 48 * (i64)i;
+#pragma unroll
+        for (int k = 0; k < 16; k++) {
+            M[3 * k] = (unsigned long long)S[k].lo;
+            M[3 * k + 1] = (unsigned long long)(S[k].lo >> 64);
+            M[3 * k + 2] = S[k].hi;
+        }
+    }
+    if (stats) {
+        unsigned long long *st = stats + 4 * (i64)i;
+        memcpy(&st[0], &mn, 8);
+        memcpy(&st[1], &mx, 8);
+        st[2] = nf_mask;
+        st[3] = nf_box;
+    }
+}
+
+template <typename T>
+static int launch_intensity(const uint32_t *d_cum, const int64_t *d_cnt_off, const int32_t *d_cnt_len,
+                            const uint32_t *d_h, const int32_t *d_bbox, int32_t n, const void *d_img,
+                            const double *d_center, int32_t scan_box, void *d_moments, uint64_t *d_stats,
+                            void *stream)
+{
+    rle_intensity_kernel<T><<<(unsigned)(((i64)n * 32 + 255) / 256), 256, 0, as_stream(stream)>>>(
+        d_cum, d_cnt_off, d_cnt_len, d_h, (const int4 *)d_bbox, n, (const T *)d_img, d_center, scan_box, d_moments,
+        (unsigned long long *)d_stats);
+    AMPIS_CHECK_LAUNCH("rle_intensity_kernel");
+    return AMPIS_OK;
+}
+
+extern "C" int ampis_rle_intensity(const uint32_t *d_cum, const int64_t *d_cnt_off, const int32_t *d_cnt_len,
+                                   const uint32_t *d_h, const int32_t *d_bbox, int32_t n, const void *d_img,
+                                   int32_t pix, const double *d_center, int32_t scan_box, void *d_moments,
+                                   uint64_t *d_stats,
+                                   void *stream)
+{
+    AMPIS_REQUIRE(n >= 0, "n < 0");
+    AMPIS_REQUIRE(pix >= AMPIS_PIX_U8 && pix <= AMPIS_PIX_F64, "unknown pixel type");
+    AMPIS_REQUIRE(!d_center || pix >= AMPIS_PIX_F16, "central sums are for float pixels only");
+    AMPIS_REQUIRE(d_center || d_stats, "the raw pass writes the statistics");
+    if (n == 0) return AMPIS_OK;
+    AMPIS_REQUIRE(d_cum && d_cnt_off && d_cnt_len && d_h && d_bbox && d_img && d_moments, "null pointer");
+    switch (pix) {
+    case AMPIS_PIX_U8: return launch_intensity<uint8_t>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_I8: return launch_intensity<int8_t>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_U16: return launch_intensity<uint16_t>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_I16: return launch_intensity<int16_t>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_U32: return launch_intensity<uint32_t>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_I32: return launch_intensity<int32_t>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_U64: return launch_intensity<uint64_t>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_I64: return launch_intensity<int64_t>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_F16: return launch_intensity<__half>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    case AMPIS_PIX_F32: return launch_intensity<float>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    default: return launch_intensity<double>(d_cum, d_cnt_off, d_cnt_len, d_h, d_bbox, n, d_img, d_center, scan_box, d_moments, d_stats, stream);
+    }
 }

@@ -1230,19 +1230,79 @@ def region_measurements(masks):
 
 #: measurements region_measurements_for can take, each one kernel (or pair of kernels) over one CROP table
 REGION_MEASUREMENTS = ('moments', 'perimeter_hist', 'convex_area', 'moments3', 'filled', 'crofton', 'convex_feret',
-                       'image', 'filled_image')
-#: ampis_rle_moments3 is exact while both sides of the frame stay below this
+                       'image', 'filled_image', 'intensity', 'weighted_intensity')
+#: ampis_rle_moments3 and ampis_rle_intensity are exact while both sides of the frame stay below this
 MOMENTS3_MAX_SIDE = 65536
+#: pixel type codes of ampis_rle_intensity (AMPIS_PIX_* of include/ampis_b200.h) by numpy dtype
+INTENSITY_PIX = {np.dtype(t): code for t, code in
+                 ((np.bool_, 0), (np.uint8, 0), (np.int8, 1), (np.uint16, 2), (np.int16, 3), (np.uint32, 4),
+                  (np.int32, 5), (np.uint64, 6), (np.int64, 7), (np.float16, 8), (np.float32, 9), (np.float64, 10))}
+_SAME_WIDTH_TORCH = {1: torch.uint8, 2: torch.int16, 4: torch.int32, 8: torch.int64}
+
+
+def _i192(limbs):
+    """Three 64-bit limbs (low first, as Python ints) -> the signed 192-bit integer they hold."""
+    v = limbs[0] | (limbs[1] << 64) | (limbs[2] << 128)
+    return v - (1 << 192) if v >> 191 else v
+
+
+def _intensity_measurements(t, intensity_image, weighted):
+    """ampis_rle_intensity over the masks of table t (see region_measurements_for, 'intensity' and
+    'weighted_intensity').  The image is uploaded once, as raw pixels of its own width, and transposed to
+    column-major order on the device.  Without `weighted`, a float image takes one pass and no box scan."""
+    dev, n = t.device, t.n
+    a = np.asarray(intensity_image)
+    dt = a.dtype.newbyteorder('=')
+    if dt not in INTENSITY_PIX:
+        raise TypeError('intensity images of dtype %s are not supported (%s)'
+                        % (a.dtype, ', '.join(sorted({str(d) for d in INTENSITY_PIX}))))
+    if n and max(int(t.h[:n].max().item()), int(t.w[:n].max().item())) > MOMENTS3_MAX_SIDE:
+        raise ValueError('moments to order 3 are exact for frames up to %d pixels a side' % MOMENTS3_MAX_SIDE)
+    raw = np.ascontiguousarray(a, dtype=dt)
+    img = _dev(raw.view(np.dtype('u1') if dt.itemsize == 1 else np.dtype('i%d' % dt.itemsize)),
+               _SAME_WIDTH_TORCH[dt.itemsize], dev).reshape(raw.shape).t().contiguous()
+    pix, flt = INTENSITY_PIX[dt], dt.kind == 'f'
+    stats = torch.empty(max(4 * n, 1), dtype=torch.int64, device=dev)
+    mom = torch.empty(max((16 if flt else 48) * n, 1), dtype=torch.float64 if flt else torch.int64, device=dev)
+    N.call('ampis_rle_intensity', _p(t.cum), _p(t.cnt_off), _p(t.cnt_len), _p(t.h), _p(t.bbox), n, _p(img), pix,
+           None, int(flt and weighted), _p(mom), _p(stats), _stream())
+    st = stats[:4 * n].cpu().numpy().reshape(n, 4)
+    wide = np.float64 if flt else np.int64 if dt.kind == 'i' else np.uint64
+    out = {'intensity_min': np.ascontiguousarray(st[:, 0]).view(wide).astype(dt),
+           'intensity_max': np.ascontiguousarray(st[:, 1]).view(wide).astype(dt)}
+    if not flt:
+        limbs = mom[:48 * n].cpu().numpy().view(np.uint64).reshape(n, 16, 3).tolist()
+        out['intensity_sum'] = [_i192(row[0]) for row in limbs]
+        if weighted:
+            out['intensity_moments'] = [[[_i192(row[4 * p + q]) for q in range(4)] for p in range(4)] for row in limbs]
+        return out
+    if not weighted:
+        out['intensity_sum'] = mom[:16 * n].view(n, 16)[:, 0].cpu().numpy()
+        return out
+    # float pixels: the central sums in a second pass about the weighted centroid, formed on the device
+    m = mom[:16 * n].view(n, 16)
+    center = torch.stack([m[:, 4] / m[:, 0], m[:, 1] / m[:, 0]], dim=1).contiguous()
+    central = torch.empty(max(16 * n, 1), dtype=torch.float64, device=dev)
+    N.call('ampis_rle_intensity', _p(t.cum), _p(t.cnt_off), _p(t.cnt_len), _p(t.h), _p(t.bbox), n, _p(img), pix,
+           _p(center), 0, _p(central), None, _stream())
+    raw_m, cen_m = m.cpu().numpy().reshape(n, 4, 4), central[:16 * n].cpu().numpy().reshape(n, 4, 4)
+    # skimage weighs the whole box, img[slice] * image: a NaN or inf of the box outside the mask gives NaN * 0
+    out['intensity_sum'] = raw_m[:, 0, 0].copy()             # of the mask's pixels, for the mean
+    outside = st[:, 3] > st[:, 2]
+    raw_m[outside] = np.nan
+    cen_m[outside] = np.nan
+    out['intensity_moments'], out['intensity_central'] = raw_m, cen_m
+    return out
 
 
 def _ragged_u8(flat, off, shapes):
     return [flat[off[i]:off[i + 1]].reshape(shapes[i]).view(np.bool_) for i in range(len(shapes))]
 
 
-def region_measurements_for(masks, need):
+def region_measurements_for(masks, need, intensity_image=None):
     """Per-mask raw measurements behind compute_rprops for the measurement names in `need` only (see
     REGION_MEASUREMENTS): one CROP-layout table, then only the launches those names require.  Always present:
-    area[n], bbox[n,4] (x0,y0,x1,y1).  Optional, all exact integers:
+    area[n], bbox[n,4] (x0,y0,x1,y1).  Optional, all exact integers but the sums of float intensity images:
       moments[n,6], perimeter_hist[n,10], convex_area[n]   as region_measurements;
       moments3: list of n 4x4 nested lists of Python ints, M[p][q] = sum r^p c^q in box-local coordinates;
       filled: filled_area[n] (binary_fill_holes with an all-ones 3x3 structure);
@@ -1250,11 +1310,22 @@ def region_measurements_for(masks, need):
       crofton: crofton_trans[n,4], differing pixel pairs along rows, columns, diagonal, anti-diagonal;
       convex_feret: convex_ranges (list of n int32[box_w, 2] box-local row ranges [lo, hi) of
         convex_hull_image) and feret_d2[n] = (2 * feret_diameter_max)^2;
-      image: list of n bool box images."""
+      image: list of n bool box images;
+      intensity (needs `intensity_image`, a 2-D array of the masks' frame size, bool / integer / float16-64):
+        intensity_min[n], intensity_max[n] in the image's dtype (NaN when a float mask holds a NaN pixel) and
+        intensity_sum[n], the sum of the mask's pixels (exact Python ints for integer and bool images);
+      weighted_intensity (implies intensity, needs the image as well): intensity_moments, M[p][q] = sum I r^p c^q in box-local coordinates -- for integer and bool images a list
+        of n 4x4 nested lists of exact Python ints; for float images float64[n,4,4] summed in float64, with
+        intensity_central[n,4,4], the sums about the weighted centroid (M[1][0] / M[0][0], M[0][1] / M[0][0]).
+        A NaN or inf in a mask's box but outside the mask makes both NaN, as skimage's img[slice] * image does."""
     need = set(need)
     bad = need - set(REGION_MEASUREMENTS)
     if bad:
         raise ValueError('unknown region measurements %s' % sorted(bad))
+    if 'weighted_intensity' in need:
+        need.add('intensity')
+    if 'intensity' in need and intensity_image is None:
+        raise ValueError('the intensity measurements need an intensity image')
     if 'filled_image' in need:
         need.add('filled')
     t = table_from_rle(masks, layout=LAYOUT_CROP)
@@ -1323,6 +1394,8 @@ def region_measurements_for(masks, need):
             N.call('ampis_crop_unpack_image', _p(src), _p(t.bits_off), _p(t.bbox), n, _p(d_img_off), _p(img),
                    _stream())
             out[key] = _ragged_u8(to_host(img[:int(img_off[n])]), img_off, shapes)
+    if 'intensity' in need:
+        out.update(_intensity_measurements(t, intensity_image, 'weighted_intensity' in need))
     return out
 
 

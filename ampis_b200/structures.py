@@ -171,15 +171,21 @@ class InstanceSet(object):
                        'orientation', 'perimeter', 'solidity', 'moments', 'moments_central', 'moments_normalized',
                        'moments_hu', 'inertia_tensor', 'inertia_tensor_eigvals', 'filled_area', 'filled_image',
                        'perimeter_crofton', 'feret_diameter_max', 'convex_image', 'image', 'coords', 'slice')
+    #: the intensity properties of scikit-image 0.18.3; compute_rprops takes them when given an intensity_image
+    RPROPS_INTENSITY_KEYS = ('intensity_image', 'max_intensity', 'mean_intensity', 'min_intensity',
+                             'weighted_centroid', 'weighted_local_centroid', 'weighted_moments',
+                             'weighted_moments_central', 'weighted_moments_normalized', 'weighted_moments_hu')
     #: properties regionprops_table keeps whole, one object cell per region
-    RPROPS_OBJECT_KEYS = ('image', 'filled_image', 'convex_image', 'coords', 'slice')
+    RPROPS_OBJECT_KEYS = ('image', 'filled_image', 'convex_image', 'coords', 'slice', 'intensity_image')
     #: shape of the array-valued properties, split into key-i(-j) columns; integer-valued properties
     _RPROPS_SHAPES = {'bbox': (4,), 'centroid': (2,), 'local_centroid': (2,), 'moments': (4, 4),
                       'moments_central': (4, 4), 'moments_normalized': (4, 4), 'moments_hu': (7,),
-                      'inertia_tensor': (2, 2), 'inertia_tensor_eigvals': (2,)}
+                      'inertia_tensor': (2, 2), 'inertia_tensor_eigvals': (2,), 'weighted_centroid': (2,),
+                      'weighted_local_centroid': (2,), 'weighted_moments': (4, 4), 'weighted_moments_central': (4, 4),
+                      'weighted_moments_normalized': (4, 4), 'weighted_moments_hu': (7,)}
     _RPROPS_INT_KEYS = ('area', 'bbox', 'bbox_area', 'convex_area', 'label', 'filled_area')
 
-    def compute_rprops(self, keys=None, return_df=False):
+    def compute_rprops(self, keys=None, return_df=False, intensity_image=None):
         """Region properties per mask (reference structures.py:474-514, which decodes every mask to a
         full int64 frame and runs skimage.measure.regionprops_table on it).  Here the GPU delivers
         exact integer measurements from the run table and the packed bounding-box windows
@@ -187,18 +193,29 @@ class InstanceSet(object):
         Feret diameter, box images) and the properties are formed on the host with skimage 0.18.3's
         formulas.  Default keys are the reference's; cells are 1-element arrays (empty for an empty mask)
         as regionprops_table returns them; tuple- and array-valued properties become ``key-0``, ``key-1``
-        ... (``key-0-0`` ... for 2-D arrays) columns, and image, filled_image, convex_image, coords and slice
-        one column of 1-element object arrays."""
+        ... (``key-0-0`` ... for 2-D arrays) columns, and image, filled_image, convex_image, coords, slice and
+        intensity_image one column of 1-element object arrays.
+
+        intensity_image: the grayscale image the masks were found on (2-D, the shape of ``instances.image_size``,
+        otherwise ValueError as skimage raises), needed for RPROPS_INTENSITY_KEYS; bool, integer and
+        float16/32/64 pixels.  Its min, max and weighted moments are measured on the GPU -- exact integer sums for
+        integer and bool images, float64 sums for float images -- and formed here as skimage 0.18.3 does.
+        max_intensity, min_intensity and mean_intensity cells are float64, as regionprops_table's are.  One
+        deviation: the mean of a float16 / float32 image is taken in float64, where numpy sums in the input
+        precision."""
         if keys is None:
             keys = ['area', 'equivalent_diameter', 'major_axis_length', 'perimeter', 'solidity', 'orientation']
-        unsupported = [k for k in keys if k not in self.RPROPS_GPU_KEYS]
+        supported = self.RPROPS_GPU_KEYS + self.RPROPS_INTENSITY_KEYS
+        unsupported = [k for k in keys if k not in supported]
         if unsupported:
             raise NotImplementedError('region properties %s are not part of the GPU path (supported: %s)'
-                                      % (unsupported, list(self.RPROPS_GPU_KEYS)))
+                                      % (unsupported, list(supported)))
+        if intensity_image is not None:
+            _check_intensity_shape(intensity_image, [tuple(self.instances.image_size)])
         rle = masks_to_rle(self.instances.masks, self.instances.image_size)
         if type(rle) == dict:
             rle = [rle]
-        props = region_properties(rle, keys)
+        props = region_properties(rle, keys, intensity_image)
         rows = []
         for p in props:
             row = {}
@@ -221,6 +238,8 @@ class InstanceSet(object):
                     a = np.asarray(v)
                     for loc in np.ndindex(a.shape):
                         row['-'.join(map(str, (k,) + loc))] = np.array([a[loc].item()])
+                elif k in self.RPROPS_INTENSITY_KEYS:     # max / min / mean: float columns in regionprops_table
+                    row[k] = np.array([v], np.float64)
                 else:
                     row[k] = np.array([v])
             rows.append(row)
@@ -358,7 +377,11 @@ _MEASUREMENTS_OF = {
     'moments': ('moments3',), 'moments_central': ('moments3',), 'moments_normalized': ('moments3',),
     'moments_hu': ('moments3',), 'filled_area': ('filled',), 'filled_image': ('filled_image',),
     'perimeter_crofton': ('crofton',), 'feret_diameter_max': ('convex_feret',), 'convex_image': ('convex_feret',),
-    'image': ('image',), 'coords': ('image',),
+    'image': ('image',), 'coords': ('image',), 'intensity_image': ('image',),
+    'max_intensity': ('intensity',), 'mean_intensity': ('intensity',), 'min_intensity': ('intensity',),
+    'weighted_centroid': ('weighted_intensity',), 'weighted_local_centroid': ('weighted_intensity',),
+    'weighted_moments': ('weighted_intensity',), 'weighted_moments_central': ('weighted_intensity',),
+    'weighted_moments_normalized': ('weighted_intensity',), 'weighted_moments_hu': ('weighted_intensity',),
 }
 _DEFAULT_KEYS = ('area', 'bbox', 'bbox_area', 'centroid', 'local_centroid', 'convex_area', 'eccentricity',
                  'equivalent_diameter', 'extent', 'major_axis_length', 'minor_axis_length', 'orientation', 'perimeter',
@@ -397,11 +420,16 @@ def _second_order_props(mom, y0, x0):
 _BINOM = [[1], [1, 1], [1, 2, 1], [1, 3, 3, 1]]
 
 
-def _moment_props(M):
-    """moments, moments_central, moments_normalized, moments_hu (skimage 0.18.3) from the exact box-local raw
-    moments M[p][q] = sum r^p c^q (Python ints).  The central moments are expanded exactly about the rational
-    centroid -- N^(p+q) mu[p][q] is an integer -- and rounded once."""
+def _exact_central(M):
+    """Central moments float64[4, 4] from exact box-local raw moments M[p][q] = sum w r^p c^q (Python ints; w = 1
+    for a mask, the pixel values for weighted moments, so N = M[0][0] may be zero or negative).  They are expanded
+    exactly about the rational centroid -- N^(p+q) mu[p][q] is an integer -- and rounded once.  N = 0 follows
+    skimage's float arithmetic: the centroid is nan or +-inf, mu[0][0] = sum w = 0.0 and every other entry nan."""
     N, Sr, Sc = M[0][0], M[1][0], M[0][1]
+    if N == 0:
+        mu = np.full((4, 4), np.nan)
+        mu[0, 0] = 0.0
+        return mu
     mu = np.zeros((4, 4))
     for p in range(4):
         for q in range(4):
@@ -410,13 +438,61 @@ def _moment_props(M):
                 for j in range(q + 1):
                     num += _BINOM[p][i] * _BINOM[q][j] * (-Sr) ** (p - i) * (-Sc) ** (q - j) * N ** (i + j) * M[i][j]
             mu[p, q] = num / N ** (p + q)
+    return mu
+
+
+def _moment_props(M, mu):
+    """moments, moments_central, moments_normalized, moments_hu (skimage 0.18.3) from the box-local raw moments M
+    (4x4 Python ints or float64) and the central moments mu (float64[4, 4]).  mu[0][0] is a numpy float, so a
+    weighted mu[0][0] <= 0 gives nan or inf in the normalized moments as in skimage, never a complex number."""
     nu = np.full((4, 4), np.nan)
-    for p in range(4):
-        for q in range(4):
-            if p + q >= 2:
-                nu[p, q] = mu[p, q] / (mu[0, 0] ** ((p + q) / 2 + 1))
+    with np.errstate(divide='ignore', invalid='ignore'):
+        for p in range(4):
+            for q in range(4):
+                if p + q >= 2:
+                    nu[p, q] = mu[p, q] / (mu[0, 0] ** ((p + q) / 2 + 1))
+        hu = _hu(nu)
     return {'moments': np.array(M, dtype=np.float64), 'moments_central': mu, 'moments_normalized': nu,
-            'moments_hu': _hu(nu)}
+            'moments_hu': hu}
+
+
+def _check_intensity_shape(img, sizes):
+    """skimage's condition on an intensity image: 2-D (one channel, as 0.18.3 has) and of the label image's shape;
+    `sizes` are the frame sizes of the masks."""
+    shape = np.shape(img)
+    if len(shape) != 2 or any(tuple(int(v) for v in sz) != shape for sz in sizes):
+        raise ValueError('Label and intensity image must have the same shape.')
+
+
+def _div(a, b):
+    """a / b as skimage's float64 division gives it: correctly rounded, nan or +-inf for b = 0."""
+    with np.errstate(divide='ignore', invalid='ignore'):
+        return a / b if b else float(np.float64(a) / np.float64(b))
+
+
+def _intensity_props(m, i, area, y0, x0, box_img, intensity_image):
+    """The intensity properties of mask i from the 'intensity' / 'weighted_intensity' measurements taken (and, for
+    intensity_image, the 'image' one)."""
+    p = {}
+    if box_img is not None:
+        p['intensity_image'] = np.asarray(intensity_image)[y0:y0 + box_img.shape[0], x0:x0 + box_img.shape[1]] * box_img
+    if 'intensity_min' in m:
+        p.update({'max_intensity': m['intensity_max'][i], 'min_intensity': m['intensity_min'][i],
+                  'mean_intensity': m['intensity_sum'][i] / area})
+    if 'intensity_moments' not in m:
+        return p
+    M = m['intensity_moments'][i]
+    if 'intensity_central' in m:                    # float image: float64 sums, central ones from the second pass
+        mu = m['intensity_central'][i]
+        lr, lc = _div(M[1, 0], M[0, 0]), _div(M[0, 1], M[0, 0])
+    else:
+        mu = _exact_central(M)
+        lr, lc = _div(M[1][0], M[0][0]), _div(M[0][1], M[0][0])
+    mom = _moment_props(M, mu)
+    p.update({'weighted_local_centroid': (lr, lc), 'weighted_centroid': (lr + y0, lc + x0),
+              'weighted_moments': mom['moments'], 'weighted_moments_central': mu,
+              'weighted_moments_normalized': mom['moments_normalized'], 'weighted_moments_hu': mom['moments_hu']})
+    return p
 
 
 def _hu(nu):
@@ -446,12 +522,19 @@ def _hu(nu):
 _CROFTON_SCALE = np.pi / 8
 
 
-def region_properties(rle, keys=None):
+def region_properties(rle, keys=None, intensity_image=None):
     """skimage 0.18.3 region properties of every mask of an RLE list (one region per mask, as
-    ``regionprops_table(mask.astype(int))`` sees it) from the exact GPU measurements.  Returns one
+    ``regionprops_table(mask.astype(int), intensity_image)`` sees it) from the exact GPU measurements.  Returns one
     dict per mask ({} for an empty mask).  keys=None: the fifteen scalar and tuple properties of
-    _DEFAULT_KEYS; otherwise the listed properties of InstanceSet.RPROPS_GPU_KEYS, and only the GPU
-    measurements those need are taken."""
+    _DEFAULT_KEYS; otherwise the listed properties of InstanceSet.RPROPS_GPU_KEYS and RPROPS_INTENSITY_KEYS, and
+    only the GPU measurements those need are taken.
+
+    intensity_image: 2-D array of the masks' frame size (ValueError otherwise), bool, integer or float16/32/64;
+    required by the intensity keys.  max_intensity and min_intensity come in its dtype; weighted moments are exact
+    for bool and integer images (frames up to 65,536 pixels a side) and summed in float64 for float images.
+    mean_intensity is a float64 -- for float16 / float32 images numpy would sum in the input precision."""
+    if intensity_image is not None:
+        _check_intensity_shape(intensity_image, {tuple(mk['size']) for mk in rle})
     if keys is None:
         m = engine.region_measurements(rle)
         keys = _DEFAULT_KEYS
@@ -460,7 +543,12 @@ def region_properties(rle, keys=None):
         unknown = [k for k in keys if k not in _MEASUREMENTS_OF]
         if unknown:
             raise NotImplementedError('region properties %s are not part of the GPU path' % unknown)
-        m = engine.region_measurements_for(rle, {x for k in keys for x in _MEASUREMENTS_OF[k]})
+        wanted = [k for k in keys if k in InstanceSet.RPROPS_INTENSITY_KEYS]
+        if wanted and intensity_image is None:
+            raise NotImplementedError('region properties %s need an intensity image: pass intensity_image, a 2-D '
+                                      'array of the masks\' frame size' % wanted)
+        m = engine.region_measurements_for(rle, {x for k in keys for x in _MEASUREMENTS_OF[k]},
+                                           intensity_image if wanted else None)
     out = []
     for i in range(len(rle)):
         n = int(m['area'][i])
@@ -480,7 +568,7 @@ def region_properties(rle, keys=None):
             p['convex_area'] = int(m['convex_area'][i])
             p['solidity'] = n / p['convex_area']
         if 'moments3' in m:
-            p.update(_moment_props(m['moments3'][i]))
+            p.update(_moment_props(m['moments3'][i], _exact_central(m['moments3'][i])))
         if 'filled_area' in m:
             p['filled_area'] = int(m['filled_area'][i])
         if 'filled_image' in m:
@@ -498,5 +586,8 @@ def region_properties(rle, keys=None):
             p['image'] = img
             r, c = np.nonzero(img)
             p['coords'] = np.stack([r + y0, c + x0], axis=1).astype(np.int64)
+        if 'intensity_min' in m or 'intensity_image' in keys:
+            p.update(_intensity_props(m, i, n, y0, x0, p.get('image') if 'intensity_image' in keys else None,
+                                      intensity_image))
         out.append({k: p[k] for k in keys})
     return out

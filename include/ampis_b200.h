@@ -463,6 +463,34 @@ int ampis_crop_convex_feret(const void *d_bits, const int64_t *d_bits_off, const
 int ampis_crop_unpack_image(const void *d_bits, const int64_t *d_bits_off, const int32_t *d_bbox, int32_t n,
                             const int64_t *d_img_off, uint8_t *d_img, void *stream);
 
+/* The intensity properties (regionprops with an intensity image), same run tables as ampis_rle_moments3:
+ * ampis_rle_intensity: d_img = the intensity image, COLUMN-major (pixel (row y, column x) at x * h + y, the order
+ *   of the run positions), of the pixel type `pix` (AMPIS_PIX_*; bool as AMPIS_PIX_U8).  Per mask:
+ *   - integer pixels: d_moments[48*i + 3*k + {0,1,2}] = the 64-bit limbs, low first, of the signed 192-bit
+ *     M[p][q] = sum I r^p c^q, k = 4p + q, box-local r, c as in ampis_rle_moments3; exact while both frame
+ *     sides are <= 65536.  d_center must be null.
+ *   - float pixels: d_center null: d_moments[16*i + k] = M[p][q] summed in float64.  d_center[2*i], [2*i+1] =
+ *     (r0, c0) box-local: d_moments[16*i + k] = sum I (r - r0)^p (c - c0)^q, the central sums.
+ *   d_stats (written when d_center is null, which requires it): 4 x 8 bytes per mask = min and max pixel of the
+ *   mask (int64 for signed, uint64 for unsigned, float64 for float pixels; NaN when the mask holds a NaN), then
+ *   the number of non-finite pixels of the mask and, when scan_box is non-zero, of its bounding box (both 0 for
+ *   integer pixels; the box scan reads every pixel of the box, so ask for it only where the weighted moments are
+ *   needed). */
+#define AMPIS_PIX_U8    0
+#define AMPIS_PIX_I8    1
+#define AMPIS_PIX_U16   2
+#define AMPIS_PIX_I16   3
+#define AMPIS_PIX_U32   4
+#define AMPIS_PIX_I32   5
+#define AMPIS_PIX_U64   6
+#define AMPIS_PIX_I64   7
+#define AMPIS_PIX_F16   8
+#define AMPIS_PIX_F32   9
+#define AMPIS_PIX_F64  10
+int ampis_rle_intensity(const uint32_t *d_cum, const int64_t *d_cnt_off, const int32_t *d_cnt_len,
+                        const uint32_t *d_h, const int32_t *d_bbox, int32_t n, const void *d_img, int32_t pix,
+                        const double *d_center, int32_t scan_box, void *d_moments, uint64_t *d_stats, void *stream);
+
 /* ---- annotation images -> instances (data_utils.get_ddicts 'binary' / 'label', data_utils.py:394-433) ----
  * ampis_ccl_label: skimage.measure.label of a binary image (row-major u8[h][w], non-zero = foreground,
  *   full 8-connectivity, labels 1..n in raster order of each component's first pixel).  d_work i32[h*w],

@@ -5,6 +5,11 @@ numpy/scipy restatement of skimage 0.18.3 (oracle/ampis_ref.py for the fifteen, 
 the rest) on the same masks.
 
     python profiles/bench_rprops.py [out.md]
+    python profiles/bench_rprops.py --intensity [out.md]
+
+--intensity times the ten intensity keys instead, with a seeded uint16 intensity image of the frame's size, next
+to the numpy restatement of tests/_rprops_intensity_ref.py.  The kernel column times the native entry points only;
+the image upload and its transpose on the device (torch) are part of the measurement step, not of that column.
 
 Inputs are synthetic (csrc/synth.cpp): the 100 first predictions of a C1-like image (1024x768, as
 profiles/bench_functions.py uses) and one C4-like image of 5,000 masks (2048x2048).  Per input it reports
@@ -43,11 +48,14 @@ def main():
     from ampis_b200.containers import Instances
     from oracle import ampis_ref as R
     from oracle import cocomask as rle
+    from tests import _rprops_intensity_ref as MI
     from tests import _rprops_ref as M
     rle.build()
     torch.cuda.set_device(0)
     name, limit = card()
-    keys = list(S.InstanceSet.RPROPS_GPU_KEYS)
+    intensity = '--intensity' in sys.argv
+    args = [a for a in sys.argv[1:] if a != '--intensity']
+    keys = list(S.InstanceSet.RPROPS_INTENSITY_KEYS if intensity else S.InstanceSet.RPROPS_GPU_KEYS)
     new_keys = keys[15:]
     rows = []
 
@@ -57,7 +65,7 @@ def main():
         size = [host.h, host.w]
         return [{'size': size, 'counts': rle.string_from_counts(x)} for x in c], (host.h, host.w)
 
-    def kernel_times(masks):
+    def kernel_times(masks, img):
         """CUDA-event time of every launch of one region_properties call, summed per entry point (ms)."""
         real = E.N.call
         ev = []
@@ -70,7 +78,7 @@ def main():
             ev.append((nm, a, b))
         E.N.call = timed
         try:
-            S.region_properties(masks, keys)
+            S.region_properties(masks, keys, img)
         finally:
             E.N.call = real
         torch.cuda.synchronize()
@@ -94,25 +102,31 @@ def main():
     for label, masks, size, sample in (('C1-like, 100 masks', c1[:100], size1, 100),
                                        ('C4-like, %d masks' % len(c4), c4, size4, 500)):
         n = len(masks)
+        img = np.random.default_rng(5).integers(0, 65536, size, dtype=np.uint16) if intensity else None
         iset = S.InstanceSet(instances=Instances(size, masks=S.RLEMasks(masks), boxes=np.zeros((n, 4)),
                                                  class_idx=np.arange(n)))
-        iset.compute_rprops(keys=keys)                       # warm-up: library load, CUDA context
-        t_call = best(lambda: iset.compute_rprops(keys=keys))
+        iset.compute_rprops(keys=keys, intensity_image=img)  # warm-up: library load, CUDA context
+        t_call = best(lambda: iset.compute_rprops(keys=keys, intensity_image=img))
         need = {x for k in keys for x in S._MEASUREMENTS_OF[k]}
-        t_meas = best(lambda: E.region_measurements_for(masks, need))
-        t_props = best(lambda: S.region_properties(masks, keys))
-        kt = kernel_times(masks)
+        t_meas = best(lambda: E.region_measurements_for(masks, need, img))
+        t_props = best(lambda: S.region_properties(masks, keys, img))
+        kt = kernel_times(masks, img)
         # oracle on box crops of a sample (decode + crop outside the timed region)
         crops = []
         for mk in masks[:sample]:
             d = rle.decode(mk).astype(bool)
             if d.any():
                 r, c = np.nonzero(d)
-                crops.append(np.pad(d[r.min():r.max() + 1, c.min():c.max() + 1], 1))
+                sl = (slice(max(r.min() - 1, 0), r.max() + 2), slice(max(c.min() - 1, 0), c.max() + 2))
+                crops.append((d[sl], img[sl]) if intensity else
+                             np.pad(d[r.min():r.max() + 1, c.min():c.max() + 1], 1))
         t0 = time.perf_counter()
         for d in crops:
-            R.regionprops_one(d)
-            M.regionprops_more(d, new_keys)
+            if intensity:
+                MI.regionprops_intensity(d[0], d[1], keys)
+            else:
+                R.regionprops_one(d)
+                M.regionprops_more(d, new_keys)
         t_oracle = (time.perf_counter() - t0) * n / sample
         row = {'input': label, 'gpu': name, 'power_limit': limit, 'compute_rprops_ms': 1e3 * t_call,
                'region_properties_ms': 1e3 * t_props, 'measurements_ms': 1e3 * t_meas,
@@ -121,9 +135,10 @@ def main():
                'oracle_note': 'measured on %d masks, scaled to %d' % (sample, n) if sample != n else 'all masks'}
         rows.append(row)
         print(json.dumps(row), flush=True)
-    if len(sys.argv) > 1:
-        with open(sys.argv[1], 'w') as f:
-            f.write('# compute_rprops with all %d supported keys\n\n' % len(keys))
+    if args:
+        with open(args[0], 'w') as f:
+            f.write('# compute_rprops with the ten intensity keys, uint16 image\n\n' if intensity else
+                    '# compute_rprops with all %d supported keys\n\n' % len(keys))
             f.write('Measured on %s, power limit %s, by `profiles/bench_rprops.py`. Times in ms. Whole call: warm, '
                     'best of 3. Kernels: CUDA events around every launch of one call, summed per entry point. '
                     'Host formation: `region_properties` minus the measurement step. Oracle: numpy/scipy '
