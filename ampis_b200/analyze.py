@@ -66,12 +66,6 @@ def _rows_vs_cols(rows_rle, cols_rle, mode, dense=False, crowded=None):
 FUSED_CALL = os.environ.get('AMPIS_FUSED_CALL', '1') != '0'
 
 
-def _grid_capacity_error(e):
-    """True for the one library error the table API is the answer to: boxes registered in far more grid cells than
-    the one-call entries provide for.  Everything else (CUDA failures, exhausted retries) must surface."""
-    return 'grid entry list too small' in str(e)
-
-
 def _image_rows(rows_rle, cols_rle, mode):
     """Per-row arg-max results of one image as host arrays: (best_col int64, best_score float64, best_inter int64,
     areas uint32 of rows then columns).  Normally ONE call into the library (ampis_eval_images_host: bounding-box
@@ -83,18 +77,12 @@ def _image_rows(rows_rle, cols_rle, mode):
     G = len(rows_rle)
     if FUSED_CALL:
         crowd = engine.CROWD_PAIR_FRACTION if min(G, len(cols_rle)) >= engine.MMA_MIN_SIDE else -1.0
-        try:
-            r = engine.eval_images([rows_rle], [cols_rle], mode, crowd_frac=crowd, cache=True)
-        except engine.N.AmpisNativeError as e:
-            if not _grid_capacity_error(e):
-                raise
-            r = None                      # the table API sizes the grid exactly
-        if r is not None and not r.crowded:             # copies: the cached arrays stay untouched
+        r = engine.eval_images([rows_rle], [cols_rle], mode, crowd_frac=crowd, cache=True)
+        if not r.crowded:                 # copies: the cached arrays stay untouched
             return r.best_col.astype(np.int64), r.best_score.copy(), r.best_inter.astype(np.int64), r.area.copy()
-        if r is not None:
-            table, groups, res = _rows_vs_cols(rows_rle, cols_rle, mode, crowded=True)
-            return (res.best_col[:G].cpu().numpy().astype(np.int64), res.best_score[:G].cpu().numpy(),
-                    res.best_inter[:G].cpu().numpy().view(np.uint32).astype(np.int64), table.areas_np())
+        table, groups, res = _rows_vs_cols(rows_rle, cols_rle, mode, crowded=True)
+        return (res.best_col[:G].cpu().numpy().astype(np.int64), res.best_score[:G].cpu().numpy(),
+                res.best_inter[:G].cpu().numpy().view(np.uint32).astype(np.int64), table.areas_np())
     table, groups, res = _rows_vs_cols(rows_rle, cols_rle, mode)
     return (res.best_col[:G].cpu().numpy().astype(np.int64), res.best_score[:G].cpu().numpy(),
             res.best_inter[:G].cpu().numpy().view(np.uint32).astype(np.int64), table.areas_np())
@@ -106,13 +94,8 @@ def _piecewise_iou(a, b, interval=80):
     if imax == 0 or jmax == 0:
         return np.zeros((imax, jmax))
     if FUSED_CALL:
-        try:
-            r = engine.eval_image(a, b, engine.MODE_IOU, dense_iou=True)
-        except engine.N.AmpisNativeError as e:
-            if not _grid_capacity_error(e):
-                raise
-            r = None
-        if r is not None and not (min(imax, jmax) >= engine.MMA_MIN_SIDE and r.fill() >= engine.MMA_FILL_THRESHOLD):
+        r = engine.eval_image(a, b, engine.MODE_IOU, dense_iou=True)
+        if not (min(imax, jmax) >= engine.MMA_MIN_SIDE and r.fill() >= engine.MMA_FILL_THRESHOLD):
             return r.iou                  # crowded images go on to the tensor-core contraction, as in _image_rows
     table, groups, res = _rows_vs_cols(a, b, engine.MODE_IOU, dense=True)
     return engine.iou_matrix(table, res, groups, 0).cpu().numpy()
@@ -250,13 +233,8 @@ def det_seg_scores_batch(gt_list, pred_list, iou_thresh=0.5, size=None):
         raise ZeroDivisionError('division by zero')
     # the crowd gate only matters when some image is large enough for the contraction to pay off
     big = max(min(len(g), len(p)) for g, p in zip(gts, prs)) >= engine.MMA_MIN_SIDE
-    try:
-        r = engine.eval_images(gts, prs, engine.MODE_IOU, crowd_frac=engine.CROWD_PAIR_FRACTION if big else -1.0)
-    except engine.N.AmpisNativeError as e:
-        if not _grid_capacity_error(e):
-            raise
-        r = None
-    if r is None or r.crowded:             # crowded batch: image by image (each picks its kernel)
+    r = engine.eval_images(gts, prs, engine.MODE_IOU, crowd_frac=engine.CROWD_PAIR_FRACTION if big else -1.0)
+    if r.crowded:                          # crowded batch: image by image (each picks its kernel)
         return [det_seg_scores(g, p, iou_thresh) for g, p in zip(gts, prs)]
     return _scores_from_rows_batch(r, iou_thresh)
 

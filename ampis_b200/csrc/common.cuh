@@ -34,6 +34,30 @@ void ampis_set_error(const char *fmt, ...);
 
 static inline cudaStream_t as_stream(void *s) { return (cudaStream_t)s; }
 
+// Column-grid entry list of the one-call entries (ampis_eval_image_host / ampis_eval_images_host), 20 bytes per entry
+// (column index + box).  It holds `base` entries (16 per column + 4,096 per image: enough unless some boxes are much
+// larger than the image's mean box) or a 32nd of the device workspace, whichever is more.  A grid that needs more --
+// a thin diagonal across a 1024 x 1024 frame of small blobs registers in all 32 x 32 cells -- is reported as
+// AMPIS_ENOSPC with a workspace whose 32nd holds it.
+#define AMPIS_GRID_ENTRY_BYTES 20
+static inline int64_t ampis_grid_capacity(int64_t base, int64_t d_ws_bytes)
+{
+    const int64_t share = d_ws_bytes / (32 * AMPIS_GRID_ENTRY_BYTES);
+    return share > base ? share : base;
+}
+// Device workspace that leaves `rest` bytes beside the entry list and gives the list room for `entries` entries.  When
+// the workspace's 32nd exceeds base, the list takes that 32nd, so `rest` must fit in the other 31 parts; 512 bytes
+// cover the two 256-byte alignments of the list.
+static inline int64_t ampis_ws_need_with_grid(int64_t rest, int64_t base, int64_t entries)
+{
+    int64_t need = rest + AMPIS_GRID_ENTRY_BYTES * base + 512;
+    const int64_t shared = (rest + 512) * 32 / 31 + 32 * AMPIS_GRID_ENTRY_BYTES;
+    if (shared > need) need = shared;
+    const int64_t by_entries = 32 * AMPIS_GRID_ENTRY_BYTES * (entries + 1);
+    if (entries > base && by_entries > need) need = by_entries;
+    return need;
+}
+
 __device__ __forceinline__ u32 lane_id() { return threadIdx.x & 31u; }
 
 __device__ __forceinline__ u32 warp_sum(u32 v)

@@ -40,7 +40,8 @@ extern "C" int ampis_eval_image_host(const uint8_t *chars, const int64_t *chr_of
     const int32_t nb = (n_rows + ampis_rows_per_block() - 1) / ampis_rows_per_block();
     const bool use_grid = n_cols >= grid_min_cols && n_rows > 0;
     const int cells = ampis_grid_cells();
-    const int64_t grid_cap = use_grid ? 16 * (int64_t)n_cols + 4096 : 0;
+    const int64_t grid_base = use_grid ? 16 * (int64_t)n_cols + 4096 : 0;
+    const int64_t grid_cap = use_grid ? ampis_grid_capacity(grid_base, d_ws_bytes) : 0;
 
     // ---- layout: [upload block][download block][device-only][arena] ---------------------------------------
     Carve c;
@@ -67,11 +68,17 @@ extern "C" int ampis_eval_image_host(const uint8_t *chars, const int64_t *chr_of
     const int64_t gp = (int64_t)n_rows * n_cols;
     const int64_t x_imat = dense ? c.take(4 * gp) : 0, x_iou = dense ? c.take(8 * gp) : 0, x_imoff = dense ? c.take(8) : 0;
     const int64_t fixed0 = c.off;
+    // the grid entry list is the part of fixed0 that grows with d_ws (common.cuh)
+    const int64_t grid_bytes = AMPIS_GRID_ENTRY_BYTES * grid_cap;
+    auto need_for = [&](int64_t rest, int64_t entries) {
+        return use_grid ? ampis_ws_need_with_grid(rest, grid_base, entries) : rest;
+    };
     // what is left: a quarter for the candidate-pair list of the join (44 bytes per pair), the rest for the arena
     // (at least a window of 64 bytes per mask to start with)
     if (h_ws_bytes < host_bytes || d_ws_bytes < fixed0 + 128 * n + 8192) {
-        *need_bytes = fixed0 + 4096 * n + 131072;
+        *need_bytes = need_for(fixed0 - grid_bytes + 4096 * n + 131072, 0);
         if (h_ws_bytes < host_bytes) *need_bytes = -(host_bytes);      // negative: the HOST workspace is the short one
+        ampis_set_error("%s workspace too small", h_ws_bytes < host_bytes ? "host" : "device");
         return AMPIS_ENOSPC;
     }
     const int64_t pair_cap = use_grid ? ((d_ws_bytes - fixed0) / 4 - 1024) / 44 : 0;
@@ -152,15 +159,20 @@ extern "C" int ampis_eval_image_host(const uint8_t *chars, const int64_t *chr_of
     // ---- did everything fit? ------------------------------------------------------------------------------------
     const uint64_t used = *(const uint64_t *)(H + o_cursor);
     const int64_t pairs_found = use_grid && n_rows > 0 && n_cols > 0 ? *(const int64_t *)(H + o_pairtot) : 0;
-    if ((int64_t)used > arena_chunks || pairs_found > pair_cap) {
-        // the free part is split 1 : 3 between the pair list and the arena
-        const int64_t by_arena = (16 * (int64_t)used + 65536) * 4 / 3, by_pairs = (44 * pairs_found + 4096) * 4;
-        *need_bytes = fixed0 + (by_arena > by_pairs ? by_arena : by_pairs) + 65536;
+    const int64_t entries = use_grid && n_cols > 0 ? *(const int64_t *)(H + o_gridtot) : 0;
+    const bool short_ws = (int64_t)used > arena_chunks || pairs_found > pair_cap;
+    if (short_ws || entries > grid_cap) {
+        // the free part is split 1 : 3 between the pair list and the arena (when the grid list overflowed, the join
+        // missed candidates: a later call may still ask for more pair room)
+        int64_t rest = d_ws_bytes - grid_bytes;
+        if (short_ws) {
+            const int64_t by_arena = (16 * (int64_t)used + 65536) * 4 / 3, by_pairs = (44 * pairs_found + 4096) * 4;
+            rest = fixed0 - grid_bytes + (by_arena > by_pairs ? by_arena : by_pairs) + 65536;
+        }
+        *need_bytes = need_for(rest, entries);
+        ampis_set_error("device workspace too small (%lld bytes; grid entries: %lld)", (long long)d_ws_bytes,
+                        (long long)entries);
         return AMPIS_ENOSPC;
-    }
-    if (use_grid && n_cols > 0 && *(const int64_t *)(H + o_gridtot) > grid_cap) {
-        ampis_set_error("grid entry list too small (%lld entries)", (long long)*(const int64_t *)(H + o_gridtot));
-        return AMPIS_EINVAL;          // boxes spread over far more cells than 16 per mask: use the table API
     }
     if (n_rows > 0 && n_cols > 0) {
         memcpy(best_col, H + o_col, (size_t)(4 * (int64_t)n_rows));

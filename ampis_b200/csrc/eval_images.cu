@@ -165,7 +165,8 @@ extern "C" int ampis_eval_images_host(const uint8_t *const *str_ptr, const int32
         for (int64_t i = 0; i < n; i++) AMPIS_REQUIRE(str_ptr[i] || str_len[i] == 0, "bad string descriptor");
     AMPIS_REQUIRE(str_ptr[0] || n_chars == 0, "bad string descriptor");
     const int cells = ampis_grid_cells();
-    const int64_t grid_cap = 16 * (n - R) + 4096 * (int64_t)n_images;
+    const int64_t grid_base = 16 * (n - R) + 4096 * (int64_t)n_images;
+    const int64_t grid_cap = ampis_grid_capacity(grid_base, d_ws_bytes);
     const int64_t scan_tmp = on_device ? (int64_t)ampis_scan_tmp_bytes(n) : 0;
     const int64_t NI = n_images;
 
@@ -217,9 +218,11 @@ extern "C" int ampis_eval_images_host(const uint8_t *const *str_ptr, const int32
                   g_ent = c.take(4 * grid_cap), g_entbb = c.take(16 * grid_cap);
     const int64_t p_off = c.take(8 * R), p_cnt = c.take(4 * R);
     const int64_t fixed0 = c.off;
+    const int64_t grid_bytes = AMPIS_GRID_ENTRY_BYTES * grid_cap;        // the part of fixed0 that grows with d_ws
     if (h_ws_bytes < host_bytes || d_ws_bytes < fixed0 + 128 * n + 8192) {
-        *need_bytes = fixed0 + 4096 * n + 131072;
+        *need_bytes = ampis_ws_need_with_grid(fixed0 - grid_bytes + 4096 * n + 131072, grid_base, 0);
         if (h_ws_bytes < host_bytes) *need_bytes = -(host_bytes);      // negative: the HOST workspace is the short one
+        ampis_set_error("%s workspace too small", h_ws_bytes < host_bytes ? "host" : "device");
         return AMPIS_ENOSPC;
     }
     // what is left: a quarter for the candidate pairs of the join (44 bytes each), the rest for the window arena
@@ -362,16 +365,21 @@ extern "C" int ampis_eval_images_host(const uint8_t *const *str_ptr, const int32
     // ---- did everything fit? -------------------------------------------------------------------------------------
     const uint64_t used = *(const uint64_t *)(H + o_cursor);
     const int64_t found = *(const int64_t *)(H + o_pairfound);
+    const int64_t entries = *(const int64_t *)(H + o_gridtot);
     *pairs_found = found;
     *crowded = *(const int32_t *)(H + o_crowd);
-    if ((int64_t)used > arena_chunks || (!*crowded && found > pair_cap)) {
-        const int64_t by_arena = (16 * (int64_t)used + 65536) * 4 / 3, by_pairs = (44 * found + 4096) * 4;
-        *need_bytes = fixed0 + (by_arena > by_pairs ? by_arena : by_pairs) + 65536;
+    const bool short_ws = (int64_t)used > arena_chunks || (!*crowded && found > pair_cap);
+    if (short_ws || entries > grid_cap) {
+        // (when the grid list overflowed, the join missed candidates: a later call may still ask for more pair room)
+        int64_t rest = d_ws_bytes - grid_bytes;
+        if (short_ws) {
+            const int64_t by_arena = (16 * (int64_t)used + 65536) * 4 / 3, by_pairs = (44 * found + 4096) * 4;
+            rest = fixed0 - grid_bytes + (by_arena > by_pairs ? by_arena : by_pairs) + 65536;
+        }
+        *need_bytes = ampis_ws_need_with_grid(rest, grid_base, entries);
+        ampis_set_error("device workspace too small (%lld bytes; grid entries: %lld)", (long long)d_ws_bytes,
+                        (long long)entries);
         return AMPIS_ENOSPC;
-    }
-    if (*(const int64_t *)(H + o_gridtot) > grid_cap) {
-        ampis_set_error("grid entry list too small (%lld entries)", (long long)*(const int64_t *)(H + o_gridtot));
-        return AMPIS_EINVAL;          // boxes spread over far more cells than 16 per mask: use the table API
     }
     if (have_rows) {
         if (!out_direct) {

@@ -267,7 +267,10 @@ int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_bits_off, co
  * (AMPIS_ST_BAD_TOTAL marks malformed RLE); iou_out, when not NULL, receives the full float64 n_rows x n_cols IoU
  * matrix of analyze._piecewise_iou (analyze.py:54-112).  Nothing is allocated: d_ws (256-byte aligned device memory) and
  * h_ws are the caller's; when one is too small the call returns AMPIS_ENOSPC with *need_bytes = device bytes
- * wanted (> 0) or minus the host bytes wanted (< 0). */
+ * wanted (> 0) or minus the host bytes wanted (< 0).  The column grid's entry list takes the larger of 16 entries per
+ * column + 4,096 and a 32nd of d_ws (20 bytes per entry); boxes far larger than the image's mean box (a thin diagonal
+ * across a frame of small blobs registers in all 32 x 32 cells) can need more, which is reported the same way:
+ * AMPIS_ENOSPC and a device size whose 32nd holds the measured entries. */
 int ampis_eval_image_host(const uint8_t *chars, const int64_t *chr_off, int32_t n_rows, int32_t n_cols,
                           uint32_t h, uint32_t w, int32_t mode, int32_t grid_min_cols,
                           void *d_ws, int64_t d_ws_bytes, void *h_ws, int64_t h_ws_bytes,
@@ -296,7 +299,9 @@ int ampis_eval_image_host(const uint8_t *chars, const int64_t *chr_off, int32_t 
  * on the device (expand_images_kernel + offset scan), so the host work per call is O(n_images) plus the gather.
  * For such batches, str_len and the output arrays are used as DMA endpoints directly when they are page-locked
  * (cudaHostAlloc / cudaHostRegister): no staging copy on either side.
- * Workspaces and AMPIS_ENOSPC protocol as ampis_eval_image_host. */
+ * Workspaces and AMPIS_ENOSPC protocol as ampis_eval_image_host (grid entry list: the larger of 16 entries per column
+ * + 4,096 per image and a 32nd of d_ws).  Nothing carries over from one call to the next: a workspace grown for one
+ * batch may be reused for any other. */
 #define AMPIS_STRINGS_CONTIGUOUS 1   /* flags: the strings lie back to back from str_ptr[0] (only that pointer is read) */
 #define AMPIS_WAIT_BLOCKING      2   /* flags: wait for the results on a blocking event instead of spinning */
 int ampis_eval_images_host(const uint8_t *const *str_ptr, const int32_t *str_len, int32_t n_images,
