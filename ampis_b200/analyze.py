@@ -300,6 +300,128 @@ def _scores_from_rows_batch(r, iou_thresh):
     return out
 
 
+_SCORE_DTYPES = (np.float16, np.float32, np.float64)
+
+
+def _sorted_thresholds(thresholds, what):
+    """(thresholds ascending as float64, position of each caller's threshold in that order).  NaN is refused."""
+    th = np.asarray(thresholds, np.float64).reshape(-1)
+    if len(th) == 0:
+        raise ValueError('%s: at least one threshold is needed' % what)
+    if np.isnan(th).any():
+        raise ValueError('%s: NaN is not a threshold' % what)
+    order = np.argsort(th, kind='stable')
+    pos = np.empty(len(th), np.int64)
+    pos[order] = np.arange(len(th))
+    return th[order], pos
+
+
+def _score_array(s):
+    """A float16/32/64 numpy or torch array of scores as a 1-D numpy array of the same dtype (TypeError otherwise)."""
+    if isinstance(s, torch.Tensor):
+        if s.dtype not in (torch.float16, torch.float32, torch.float64):
+            raise TypeError('scores must be float16, float32 or float64, not %s' % s.dtype)
+        s = s.detach().cpu().numpy()
+    elif not isinstance(s, np.ndarray) or s.dtype.type not in _SCORE_DTYPES:
+        raise TypeError('scores must be float16, float32 or float64 numpy or torch arrays, not %r'
+                        % (getattr(s, 'dtype', type(s)),))
+    return s.reshape(-1)
+
+
+def _score_levels(scores, sorted_th):
+    """Per prediction, the number of sorted thresholds strictly below its score, as numpy decides ``scores > t`` for a
+    Python float t: the threshold is rounded to the scores' dtype (NumPy 2), NaN scores are never above it.  So a
+    prediction is kept at sorted threshold k iff its level > k.  scores: one array of one float dtype."""
+    with np.errstate(over='ignore'):
+        th = sorted_th.astype(scores.dtype)                  # rounding is monotone: still sorted
+    lv = np.searchsorted(th, scores, side='left')
+    lv[np.isnan(scores)] = 0
+    return lv.astype(np.uint16)
+
+
+def _image_scores(p):
+    inst = p if type(p) == Instances else p.instances if type(p) == InstanceSet else None
+    if inst is None or getattr(inst, 'scores', None) is None:
+        raise ValueError('scores are needed for predictions given as %s' % type(p).__name__)
+    return inst.scores
+
+
+def _reorder(a, pos, axis):
+    """a with axis `axis` in the order pos (no copy when pos is the identity: thresholds that came sorted)."""
+    return a if np.array_equal(pos, np.arange(len(pos))) else np.take(a, pos, axis=axis)
+
+
+def det_seg_scores_sweep(gt_list, pred_list, score_thresholds, iou_thresholds=None, scores=None, size=None):
+    """Detection and segmentation counts of a list of images over a grid of prediction-score cut-offs x IoU
+    thresholds, from one evaluation.  Cell (k, j) of image i is ``det_seg_scores(gt_i, kept, iou_thresh=t_j)`` with
+    ``kept = pred_i[scores_i > s_k]`` (numpy's comparison on the caller's scores: NaN is never kept), reduced to counts.
+    AMPIS's matcher is kept (per-GT first arg-max, several GTs may share a prediction, strict ``>``); this is not
+    COCO AP.  An image with no ground truth or nothing kept gets its counts instead of a ZeroDivisionError.
+
+    gt_list / pred_list: per image, any mask container of det_seg_scores_batch (a single image is a list of one).
+    scores: per image, a float16/32/64 numpy or torch array with one score per prediction; None takes
+    ``instances.scores`` of InstanceSet / Instances predictions (RLE lists need scores).  iou_thresholds: None = the
+    ten COCO thresholds 0.50:0.05:0.95; each must be >= 0.
+
+    Returns a dict: ``score_thresholds`` and ``iou_thresholds`` as given (float64), ``n_pred`` int64 [n, K] (kept
+    predictions), ``det_tp`` / ``det_fp`` / ``det_fn`` int64 [n, K, T] (``len`` of det_seg_scores' arrays),
+    ``seg_tp`` / ``seg_fp`` / ``seg_fn`` int64 [n, K, T] (sums of det_seg_scores' arrays), ``totals`` int64 [K, T, 3]
+    (TP / FP / FN over the dataset), ``seg_totals`` int64 [K, T, 3] and ``det_precision`` / ``det_recall`` float64
+    [K, T] from the totals (NaN where the denominator is 0).  One library call (engine.eval_images_sweep)."""
+    from . import batch
+    if len(gt_list) != len(pred_list):
+        raise ValueError('%d ground-truth images against %d prediction images' % (len(gt_list), len(pred_list)))
+    s_th = np.asarray(score_thresholds, np.float64).reshape(-1)
+    i_th = np.asarray(batch.COCO_THRESHOLDS if iou_thresholds is None else iou_thresholds, np.float64).reshape(-1)
+    s_sorted, s_pos = _sorted_thresholds(s_th, 'score_thresholds')
+    i_sorted, i_pos = _sorted_thresholds(i_th, 'iou_thresholds')
+    if i_sorted[0] < 0:
+        raise ValueError('iou_thresholds must not be negative')
+    if len(s_th) > 65535 or len(i_th) > 256:
+        raise ValueError('at most 65,535 score thresholds and 256 IoU thresholds')
+    if scores is None:
+        scores = [_image_scores(p) for p in pred_list]
+    if len(scores) != len(pred_list):
+        raise ValueError('%d score arrays for %d images' % (len(scores), len(pred_list)))
+    rle = lambda m: [] if type(m) == list and not m else masks_to_rle(m, size)
+    gts, prs = [rle(g) for g in gt_list], [rle(p) for p in pred_list]
+    sc = [_score_array(s) for s in scores]
+    for i, (p, s) in enumerate(zip(prs, sc)):
+        if len(s) != len(p):
+            raise ValueError('image %d: %d scores for %d predictions' % (i, len(s), len(p)))
+    n, K, T = len(gts), len(s_th), len(i_th)
+    # levels, one numpy pass per score dtype
+    lens = np.fromiter(map(len, sc), np.int64, n)
+    dtypes = [s.dtype for s in sc]
+    kinds = sorted(set(dtypes), key=str)
+    if len(kinds) <= 1:
+        levels = _score_levels(np.concatenate(sc) if n else np.zeros(0), s_sorted)
+    else:
+        levels = np.zeros(int(lens.sum()), np.uint16)
+        code = np.asarray([kinds.index(d) for d in dtypes])
+        for c, dt in enumerate(kinds):
+            levels[np.repeat(code == c, lens)] = _score_levels(np.concatenate([s for s in sc if s.dtype == dt]), s_sorted)
+    r = engine.eval_images_sweep(gts, prs, levels, K, i_sorted)
+    # kept predictions per image and sorted level: predictions whose level exceeds k
+    img = np.repeat(np.arange(n), lens)
+    hist = np.bincount(img * (K + 1) + levels, minlength=n * (K + 1)).reshape(n, K + 1)
+    kept = np.cumsum(hist[:, ::-1], axis=1)[:, ::-1][:, 1:]                 # [n, K]: sum over levels > k
+    # back to the caller's order of thresholds
+    order = lambda a, ks: _reorder(_reorder(a, s_pos, ks), i_pos, ks + 1)
+    totals, seg_totals = order(r.totals, 0), order(r.seg_totals, 0)
+    tp, fp, fn = (totals[..., c].astype(np.float64) for c in range(3))
+    with np.errstate(invalid='ignore', divide='ignore'):
+        out = {'score_thresholds': s_th, 'iou_thresholds': i_th, 'n_pred': _reorder(kept, s_pos, 1), 'totals': totals,
+               'seg_totals': seg_totals, 'det_precision': tp / (tp + fp), 'det_recall': tp / (tp + fn)}
+    counts = order(r.counts, 1).astype(np.int64)
+    seg = order(r.seg, 1)
+    for c, k in enumerate(('det_tp', 'det_fp', 'det_fn')):
+        out[k] = counts[..., c]
+    for c, k in enumerate(('seg_tp', 'seg_fp', 'seg_fn')):
+        out[k] = seg[..., c]
+    return out
+
+
 def merge_boxes(box1, box2):
     """Smallest [r1, r2, c1, c2] box enclosing both (analyze.py:342-376)."""
     r11, r12, c11, c12 = box1

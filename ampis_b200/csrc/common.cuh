@@ -58,6 +58,19 @@ static inline int64_t ampis_ws_need_with_grid(int64_t rest, int64_t base, int64_
     return need;
 }
 
+// IoU of a (row, column) pair from its intersection and the two areas, as rleIou forms it: the union in uint32 with
+// wrap-around, the quotient in float64.  Every kernel that ranks a row's pairs by IoU uses this one expression, so
+// their arg-maxes agree bit for bit.
+__device__ __forceinline__ double pair_iou(u32 inter, u32 row_area, u32 col_area)
+{
+    return (double)inter / (double)(row_area + col_area - inter);
+}
+// AMPIS's per-row arg-max order: a higher score wins, equal scores go to the lower column index (best_c = -1: none yet)
+__device__ __forceinline__ bool score_beats(double s, int k, double best_s, int best_c)
+{
+    return s > best_s || (s == best_s && (unsigned)k < (unsigned)best_c);
+}
+
 __device__ __forceinline__ u32 lane_id() { return threadIdx.x & 31u; }
 
 __device__ __forceinline__ u32 warp_sum(u32 v)

@@ -493,8 +493,8 @@ rows_from_pairs_kernel(const PairRowArgs p)
                 if ((i64)pos < p.coo_capacity) { p.coo_row[pos] = r; p.coo_col[pos] = k; p.coo_inter[pos] = inter; }
             }
             if (MODE == AMPIS_MODE_IOU) {
-                const double s = (double)inter / (double)(ra + ca4[u] - inter);
-                if (s > best_s || (s == best_s && (unsigned)k < (unsigned)best_c)) { best_s = s; best_i = inter; best_c = k; }
+                const double s = pair_iou(inter, ra, ca4[u]);
+                if (score_beats(s, k, best_s, best_c)) { best_s = s; best_i = inter; best_c = k; }
             } else {
                 if (inter > best_i || (inter == best_i && (unsigned)k < (unsigned)best_c)) { best_i = inter; best_c = k; }
             }

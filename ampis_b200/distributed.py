@@ -140,6 +140,59 @@ def evaluate_sharded(gt_lists, pred_lists, thresholds=batch.COCO_THRESHOLDS, gro
     return out
 
 
+_SWEEP_KEYS = ('n_pred', 'det_tp', 'det_fp', 'det_fn', 'seg_tp', 'seg_fp', 'seg_fn')
+
+
+def _gpu_sweep(gt_lists, pred_lists, scores, score_thresholds, iou_thresholds):
+    from . import analyze
+    return analyze.det_seg_scores_sweep(gt_lists, pred_lists, score_thresholds, iou_thresholds, scores=scores)
+
+
+def sweep_sharded(gt_lists, pred_lists, score_thresholds, iou_thresholds=None, scores=None, group=None, gather=True,
+                  compute_fn=None):
+    """``analyze.det_seg_scores_sweep`` of a dataset whose images are sharded over the ranks: rank r evaluates images
+    r, r+W, ... in one library call on its GPU, the int64 totals are summed with ONE all-reduce and the precision /
+    recall grids are formed from them on every rank.  Every rank passes the full dataset (and, for RLE lists, the
+    full list of per-image score arrays); only its shard is touched.  Returns the keys of det_seg_scores_sweep, the
+    per-image arrays [n_images, ...] in image order when gather (else those of the local shard), plus ``index``
+    (the images this rank evaluated).  compute_fn(gt_shard, pred_shard, score_shard, score_thresholds,
+    iou_thresholds) -> a det_seg_scores_sweep dict overrides the GPU path (CPU tests)."""
+    rank, world = world_info(group)
+    n = len(gt_lists)
+    idx = shard_indices(n, rank, world)
+    if iou_thresholds is None:
+        iou_thresholds = batch.COCO_THRESHOLDS
+    s_th = np.asarray(score_thresholds, np.float64).reshape(-1)
+    i_th = np.asarray(iou_thresholds, np.float64).reshape(-1)
+    K, T = len(s_th), len(i_th)
+    shard = [scores[i] for i in idx] if scores is not None else None
+    local = (compute_fn or _gpu_sweep)([gt_lists[i] for i in idx], [pred_lists[i] for i in idx], shard, s_th, i_th)
+    sums = torch.from_numpy(np.concatenate([np.asarray(local['totals'], np.int64).ravel(),
+                                            np.asarray(local['seg_totals'], np.int64).ravel()]))
+    if world > 1 and dist.get_backend(group) == 'nccl':
+        sums = sums.cuda()
+    all_reduce_sum_(sums, group)
+    sums = sums.cpu().numpy()
+    totals, seg_totals = sums[:3 * K * T].reshape(K, T, 3), sums[3 * K * T:].reshape(K, T, 3)
+    tp, fp, fn = (totals[..., c].astype(np.float64) for c in range(3))
+    with np.errstate(invalid='ignore', divide='ignore'):
+        out = {'score_thresholds': s_th, 'iou_thresholds': i_th, 'totals': totals, 'seg_totals': seg_totals,
+               'det_precision': tp / (tp + fp), 'det_recall': tp / (tp + fn), 'index': idx}
+    shapes = {k: (K,) if k == 'n_pred' else (K, T) for k in _SWEEP_KEYS}
+    if gather:
+        rows = np.concatenate([np.asarray(local[k], np.int64).reshape(len(idx), int(np.prod(shapes[k])))
+                               for k in _SWEEP_KEYS], axis=1)
+        full = gather_rows(rows, idx, n, group)
+        at = 0
+        for k in _SWEEP_KEYS:
+            w = int(np.prod(shapes[k]))
+            out[k] = full[:, at:at + w].reshape((n,) + shapes[k])
+            at += w
+    else:
+        out.update({k: np.asarray(local[k], np.int64) for k in _SWEEP_KEYS})
+    return out
+
+
 def _satellite_rows(part_lists, sat_lists, thresh):
     """Per image of the local shard: (matched, unmatched satellites, satellited particles, particles) and the
     number of satellites of every satellited particle (ascending particle index, powder.py:101-103), from ONE

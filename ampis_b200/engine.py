@@ -381,16 +381,11 @@ def _addr(a):
 _images_cache = {}      # mode -> (key, references that keep the strings alive, result)
 
 
-def eval_images(rows_lists, cols_lists, mode, crowd_frac=-1.0, cache=False):
-    """Many images, rows x columns each, through ampis_eval_images_host -- the per-image work of the reference's
-    analyze.py:149-164 (+ 315-321) or powder.py:80-86 for a whole list of images in ONE library call: the C
-    marshaller hands over the address of every compressed string (no join, no per-mask Python work), the library
-    gathers them into pinned memory and runs string decode -> flat measure + crop decode -> column grids ->
-    candidate-pair join -> AND+popc -> per-row arg-max with one upload, one download and one synchronisation.
-    rows_lists[g] / cols_lists[g]: lists of RLE dicts of image g.  Raises ValueError when the masks of an image do
-    not share one size and on malformed RLE.  cache=True keeps the last result per mode and returns it when the very
-    same string objects come again (a loop over IoU thresholds costs one evaluation)."""
-    device = require_cuda()
+def _marshal_images(rows_lists, cols_lists, refs):
+    """The per-image sizes of a list of images (an ImagesRows with n_rows, n_cols, row_off, mask_off and hw set) and
+    the address, length and size of every compressed string, from the C marshaller: (r, ptr, ln, hw, n, R).  refs:
+    a list that receives the string objects, or None.  Raises ValueError when the masks of an image do not share one
+    size."""
     n_img = len(rows_lists)
     assert len(cols_lists) == n_img
     r = ImagesRows()
@@ -414,7 +409,6 @@ def eval_images(rows_lists, cols_lists, mode, crowd_frac=-1.0, cache=False):
     lists = [None] * (2 * n_img)
     lists[0::2] = rows_lists
     lists[1::2] = cols_lists
-    refs = [] if cache else None            # the string objects themselves: their addresses are the cache key
     got, mixed = marshal().gather(lists, ptr, ln, hw, refs)
     assert got == n
     # one size per image: the first mask of each image speaks for it.  The marshaller has checked every list on its
@@ -434,6 +428,47 @@ def eval_images(rows_lists, cols_lists, mode, crowd_frac=-1.0, cache=False):
                 k = m0 + int(np.nonzero((hw[m0:m1] != hw[m0]).any(axis=1))[0][0])
                 raise ValueError('masks of different image sizes cannot be compared (%s vs %s)'
                                  % (tuple(int(v) for v in hw[m0]), tuple(int(v) for v in hw[k])))
+    return r, ptr, ln, hw, n, R
+
+
+def _call_growing(device, name, call):
+    """rc = call(d_ws, h_ws, need) of a one-call entry with the shared workspaces of `device`, grown and retried as
+    AMPIS_ENOSPC asks; raises on any other error."""
+    need = C.c_int64(0)
+    with _image_ws_lock:
+        ws_pair = _workspaces(device)
+        for _ in range(8):
+            d_ws, h_ws = ws_pair
+            rc = call(d_ws, h_ws, need)
+            if rc != N.ENOSPC:
+                break
+            if need.value < 0:          # pinned host workspace too small
+                ws_pair[1] = torch.empty(int(-need.value * 3 // 2), dtype=torch.uint8, pin_memory=True)
+            else:
+                torch.cuda.current_stream().synchronize()
+                ws_pair[0] = None
+                ws_pair[0] = torch.empty(int(need.value * 3 // 2), dtype=torch.uint8, device=device)
+        N.check(rc, name)
+
+
+def _check_status(status):
+    if status.any():
+        raise ValueError('malformed RLE: run counts do not sum to h*w for masks %s' % np.nonzero(status)[0][:8].tolist())
+
+
+def eval_images(rows_lists, cols_lists, mode, crowd_frac=-1.0, cache=False):
+    """Many images, rows x columns each, through ampis_eval_images_host -- the per-image work of the reference's
+    analyze.py:149-164 (+ 315-321) or powder.py:80-86 for a whole list of images in ONE library call: the C
+    marshaller hands over the address of every compressed string (no join, no per-mask Python work), the library
+    gathers them into pinned memory and runs string decode -> flat measure + crop decode -> column grids ->
+    candidate-pair join -> AND+popc -> per-row arg-max with one upload, one download and one synchronisation.
+    rows_lists[g] / cols_lists[g]: lists of RLE dicts of image g.  Raises ValueError when the masks of an image do
+    not share one size and on malformed RLE.  cache=True keeps the last result per mode and returns it when the very
+    same string objects come again (a loop over IoU thresholds costs one evaluation)."""
+    device = require_cuda()
+    n_img = len(rows_lists)
+    refs = [] if cache else None            # the string objects themselves: their addresses are the cache key
+    r, ptr, ln, hw, n, R = _marshal_images(rows_lists, cols_lists, refs)
     key = None
     if cache:
         key = (mode, float(crowd_frac), ptr[:n].tobytes(), ln[:n].tobytes(), hw[:n].tobytes(), r.n_rows.tobytes())
@@ -449,37 +484,63 @@ def eval_images(rows_lists, cols_lists, mode, crowd_frac=-1.0, cache=False):
     r.status = np.empty(n, np.int32)
     r.pairs_found, r.crowded = 0, False
     if n:
-        need, found, crowded = C.c_int64(0), C.c_int64(0), C.c_int32(0)
+        found, crowded = C.c_int64(0), C.c_int32(0)
         pa = _addr                                               # plain address (argtypes say c_void_p)
         h32, w32 = np.ascontiguousarray(r.hw[:, 0].astype(np.uint32)), np.ascontiguousarray(r.hw[:, 1].astype(np.uint32))
         lib = N.lib()
-        with _image_ws_lock:
-            ws_pair = _workspaces(device)
-            for _ in range(8):
-                d_ws, h_ws = ws_pair
-                rc = lib.ampis_eval_images_host(pa(ptr), pa(ln), n_img, pa(r.n_rows), pa(r.n_cols), pa(h32), pa(w32),
-                                                mode, 0, float(crowd_frac), _p(d_ws), d_ws.numel(), _p(h_ws),
-                                                h_ws.numel(), pa(r.best_col), pa(r.best_inter), pa(r.best_score),
-                                                pa(r.area), pa(r.bbox), pa(r.span), pa(r.status), None, 0, None, None,
-                                                C.byref(found),
-                                                C.byref(crowded), C.byref(need), _stream())
-                if rc != N.ENOSPC:
-                    break
-                if need.value < 0:          # pinned host workspace too small
-                    ws_pair[1] = torch.empty(int(-need.value * 3 // 2), dtype=torch.uint8, pin_memory=True)
-                else:
-                    torch.cuda.current_stream().synchronize()
-                    ws_pair[0] = None
-                    ws_pair[0] = torch.empty(int(need.value * 3 // 2), dtype=torch.uint8, device=device)
-            N.check(rc, 'ampis_eval_images_host')
+        _call_growing(device, 'ampis_eval_images_host', lambda d_ws, h_ws, need: lib.ampis_eval_images_host(
+            pa(ptr), pa(ln), n_img, pa(r.n_rows), pa(r.n_cols), pa(h32), pa(w32), mode, 0, float(crowd_frac), _p(d_ws),
+            d_ws.numel(), _p(h_ws), h_ws.numel(), pa(r.best_col), pa(r.best_inter), pa(r.best_score), pa(r.area),
+            pa(r.bbox), pa(r.span), pa(r.status), None, 0, None, None, C.byref(found), C.byref(crowded),
+            C.byref(need), _stream()))
         r.pairs_found, r.crowded = int(found.value), bool(crowded.value)
-        if r.status.any():
-            raise ValueError('malformed RLE: run counts do not sum to h*w for masks %s'
-                             % np.nonzero(r.status)[0][:8].tolist())
+        _check_status(r.status)
     if cache:
         # the references keep every string object alive, so an address in the key cannot be recycled while the entry lives
         _images_cache[mode] = (key, refs, r)
     return r
+
+
+class ImagesSweep(object):
+    """Result of eval_images_sweep() (numpy), thresholds in the sorted order they were passed in: totals and
+    seg_totals int64 [K, T, 3] (TP / FP / FN and seg TP / FP / FN), counts int32 and seg int64 [n_images, K, T, 3]
+    (None unless per_image), n_rows / n_cols per image, pairs_found."""
+    __slots__ = ('totals', 'seg_totals', 'counts', 'seg', 'n_rows', 'n_cols', 'pairs_found')
+
+
+def eval_images_sweep(rows_lists, cols_lists, levels, n_levels, iou_sorted, per_image=True):
+    """Detection and segmentation counts of many images over a grid of score x IoU thresholds in ONE library call
+    (ampis_eval_images_sweep_host): the decode, join and intersections of eval_images once, then the staircase and
+    count passes of csrc/score.cu.  rows_lists / cols_lists: ground truth / predictions of every image (RLE dicts).
+    levels: uint16 per prediction in image order, the number of the n_levels sorted score thresholds strictly below its
+    score (kept at sorted threshold k iff level > k).  iou_sorted: IoU thresholds, ascending, each >= 0.  No identity
+    cache: the result depends on the levels as well as on the strings."""
+    device = require_cuda()
+    n_img = len(rows_lists)
+    r, ptr, ln, hw, n, R = _marshal_images(rows_lists, cols_lists, None)
+    iou = np.ascontiguousarray(iou_sorted, np.float64)
+    K, T = int(n_levels), len(iou)
+    lv = np.ascontiguousarray(levels, np.uint16)
+    assert len(lv) == int(r.n_cols.astype(np.int64).sum())
+    out = ImagesSweep()
+    out.n_rows, out.n_cols, out.pairs_found = r.n_rows, r.n_cols, 0
+    out.totals = np.zeros((K, T, 3), np.int64)
+    out.seg_totals = np.zeros((K, T, 3), np.int64)
+    out.counts = np.zeros((n_img, K, T, 3), np.int32) if per_image else None
+    out.seg = np.zeros((n_img, K, T, 3), np.int64) if per_image else None
+    status = np.empty(max(n, 1), np.int32)
+    found = C.c_int64(0)
+    pa = _addr
+    h32, w32 = np.ascontiguousarray(r.hw[:, 0].astype(np.uint32)), np.ascontiguousarray(r.hw[:, 1].astype(np.uint32))
+    lib = N.lib()
+    _call_growing(device, 'ampis_eval_images_sweep_host', lambda d_ws, h_ws, need: lib.ampis_eval_images_sweep_host(
+        pa(ptr), pa(ln), n_img, pa(r.n_rows), pa(r.n_cols), pa(h32), pa(w32), 0, pa(lv) if len(lv) else None, K,
+        pa(iou), T, _p(d_ws), d_ws.numel(), _p(h_ws), h_ws.numel(), pa(status), pa(out.totals), pa(out.seg_totals),
+        pa(out.counts) if per_image and out.counts.size else None, pa(out.seg) if per_image and out.seg.size else None,
+        C.byref(found), C.byref(need), _stream()))
+    out.pairs_found = int(found.value)
+    _check_status(status[:n])
+    return out
 
 
 def measure_rle(masks):

@@ -312,6 +312,30 @@ int ampis_eval_images_host(const uint8_t *const *str_ptr, const int32_t *str_len
                            const double *thresholds, int32_t n_thresh, int32_t *grp_counts, int64_t *totals,
                            int64_t *pairs_found, int32_t *crowded, int64_t *need_bytes, void *stream);
 
+/* ---- many images, detection and segmentation counts over score x IoU thresholds, one call ------------------------
+ * What ampis_eval_images_host followed by analyze.py:166-174 + 300-339 gives for every cut-off of the predictions'
+ * confidence scores, from one decode, one join and one intersection per candidate pair.  Strings, sizes, flags and
+ * workspaces as ampis_eval_images_host (rows = ground truth, columns = predictions; IoU matching; no crowd gate: a
+ * crowded image only makes more candidate pairs).  levels[p], one per prediction in image order: the number of
+ * (sorted) score thresholds strictly below its score, 0 for a NaN score; prediction p is kept at sorted score
+ * threshold k iff levels[p] > k (levels[p] <= n_levels).  iou_thresh[0 .. n_iou): sorted ascending, each in
+ * [0, inf).  For score level k and IoU threshold j, each cell equals det_seg_scores on the kept predictions: TP /
+ * FP / FN = matched rows, kept predictions no matched row claims, unmatched rows; seg TP / FP / FN = sums over the
+ * matched rows of intersection, prediction area - intersection, GT area - intersection.  Outputs: totals and
+ * seg_totals int64[n_levels][n_iou][3] (required); counts int32[n_images][n_levels][n_iou][3] and seg_sums
+ * int64[n_images][n_levels][n_iou][3] (NULL: not formed, their device space is not needed); status int32 per mask as
+ * ampis_eval_images_host.  The per-image arrays are copied after the one wait for the results (blocking copies when
+ * they are pageable).  An image may hold at most AMPIS_SWEEP_MAX_PREDS predictions (AMPIS_EINVAL otherwise);
+ * 1 <= n_levels <= 65535, 1 <= n_iou <= AMPIS_SWEEP_MAX_IOU. */
+#define AMPIS_SWEEP_MAX_PREDS 32768
+#define AMPIS_SWEEP_MAX_IOU   256
+int ampis_eval_images_sweep_host(const uint8_t *const *str_ptr, const int32_t *str_len, int32_t n_images,
+                                 const int32_t *n_rows, const int32_t *n_cols, const uint32_t *h, const uint32_t *w,
+                                 int32_t flags, const uint16_t *levels, int32_t n_levels, const double *iou_thresh,
+                                 int32_t n_iou, void *d_ws, int64_t d_ws_bytes, void *h_ws, int64_t h_ws_bytes,
+                                 int32_t *status, int64_t *totals, int64_t *seg_totals, int32_t *counts,
+                                 int64_t *seg_sums, int64_t *pairs_found, int64_t *need_bytes, void *stream);
+
 /* ---- dense intersection matrices on the tensor cores (tcgen05, int8 contraction) -----------
  * Same quantity as the dense output of ampis_intersect_rows -- I[r][c] = popcount(row AND col),
  * what rleIou's run walk accumulates per pair (analyze.py:108,158; powder.py:82) -- computed for
