@@ -36,16 +36,17 @@ SIGNATURES = {
     'ampis_rle_measure_paint': (C.c_int, [_p, _p, _p, _p, _p, _i32, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p,
                                           _i32, _p]),
     'ampis_rle_measure_paint_flat': (C.c_int, [_p, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p,
-                                               _p, _i32, _p]),
+                                               _p, _i32, _i32, _p]),
     'ampis_rle_measure_paint_flat_zero': (C.c_int, [_p, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64,
-                                                    _p, _p, _i32, _p, _i64, _p]),
+                                                    _p, _p, _i32, _p, _i64, _i32, _p]),
     'ampis_intersect_rows_crop': (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _i32, _p, _p, _p,
                                             _p, _p]),
     'ampis_grid_cells': (C.c_int, []),
     'ampis_grid_build': (C.c_int, [_p, _p, _p, _i32, _p, _p, _p, _p, _i64, _p, _p]),
     'ampis_intersect_rows_grid': (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _p, _p, _i64,
                                             _p, _i32, _p, _i64, _p, _p, _p, _p, _p, _p, _i64, _p, _p]),
-    'ampis_intersect_rows_pairs': (C.c_int, [_p, _p, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p, _p,
+    'ampis_pairs_read_intervals': (C.c_int, []),
+    'ampis_intersect_rows_pairs': (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p, _p,
                                              _i64, _p, _p, _p, _p, _i32, _p, _i64, _p, _p, _p, _p, _p, _p, _i64, _p,
                                              _p, _p]),
     'ampis_rle_decode_crop': (C.c_int, [_p, _p, _p, _p, _p, _p, _i32, _p, _i64, _p]),

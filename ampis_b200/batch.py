@@ -188,7 +188,9 @@ class Pipeline(object):
 
     def __init__(self, batch, layout, arena, rows_out=None, thresholds=COCO_THRESHOLDS, totals=None,
                  sat_thresh=0.5, fused=True, kernel='rows', area_hist=None, area_bin_width=64, mma_sort=True,
-                 sparse_capacity=None):
+                 sparse_capacity=None, intervals=True):
+        """intervals: when the table goes to the pairs join (and nowhere else), store column-convex masks as one
+        interval word per column (engine.MaskTable.measure_paint); False keeps bitmap windows everywhere."""
         dev = batch.device
         self.area_hist, self.area_bin_width = area_hist, area_bin_width     # optional int64 histogram (+=)
         self.batch, self.layout, self.arena, self.fused = batch, layout, arena, fused
@@ -213,6 +215,8 @@ class Pipeline(object):
                 del dry
         elif layout == engine.LAYOUT_CROP and kernel == 'scan':
             self.grid = 'scan'
+        # the decoded table is read by the join alone (the area histogram and satellite counts read the areas only)
+        self.intervals = bool(intervals) and self.pairs is not None and kernel not in ('mma', 'mma2')
         self.mma_sort = mma_sort    # tiles from spatially sorted masks (contracts fewer slabs on large frames)
         if kernel in ('mma', 'mma2'):
             batch.groups.mma_tiles(kernel == 'mma2')
@@ -267,7 +271,8 @@ class Pipeline(object):
             if mark: mark(1)
             with_decode = ZERO_WITH_DECODE and not zero_ahead and self.pairs is not None and g.imat_off is not None \
                 and self.rows.imat is not None and engine.ROWS_KERNEL == 'pairs' and self.kernel not in ('mma', 'mma2')
-            t.measure_paint(self.arena, zero=self.rows.imat[:g.imat_size] if with_decode else None)
+            t.measure_paint(self.arena, zero=self.rows.imat[:g.imat_size] if with_decode else None,
+                            intervals=self.intervals)
             if with_decode and t.zeroed:
                 zeroed = True
         else:

@@ -16,6 +16,26 @@ typedef int64_t i64;
 
 #define AMPIS_CHUNK_BITS 128u   // one uint4 = 128 pixels of the column-major bit vector
 
+// reg.x of an AMPIS_LAYOUT_CROP mask whose window is in INTERVAL form (rle_flat.cu, decoded with intervals on): one
+// word per box column, (first row ^ 0xffff) | last row << 16, first row > last row for a column without pixels.  Only
+// the pairs join (intersect_pairs.cu) reads such windows; a crop bitmap window has reg.x = 0.
+#define AMPIS_WIN_INTERVALS 1u
+
+// rows y0 .. y0 + 31 of an interval word v as one 32-bit band (bit k = row y0 + k)
+__device__ __forceinline__ u32 interval_band(u32 v, u32 y0)
+{
+    const int ys = (int)((v & 0xffffu) ^ 0xffffu) - (int)y0, yl = (int)(v >> 16) - (int)y0;
+    if (ys > yl || yl < 0 || ys > 31) return 0u;
+    return (0xffffffffu << max(ys, 0)) & (0xffffffffu >> (31 - min(yl, 31)));
+}
+
+// pixels two interval words have in common
+__device__ __forceinline__ u32 interval_overlap(u32 a, u32 b)
+{
+    const int ys = (int)max((a & 0xffffu) ^ 0xffffu, (b & 0xffffu) ^ 0xffffu), yl = (int)min(a >> 16, b >> 16);
+    return (u32)max(yl - ys + 1, 0);
+}
+
 void ampis_set_error(const char *fmt, ...);
 
 #define AMPIS_CHECK_LAUNCH(name)                                              \

@@ -104,6 +104,8 @@ extern "C" int ampis_eval_image_host(const uint8_t *chars, const int64_t *chr_of
     // ---- kernels --------------------------------------------------------------------------------------------
     int rc;
 #define STEP(call) do { rc = (call); if (rc != AMPIS_OK) return rc; } while (0)
+    // interval windows for the pairs join; the column scan of narrow images (ampis_intersect_rows_crop) reads bitmaps
+    const int32_t iv = use_grid && ampis_pairs_read_intervals() ? 1 : 0;
     STEP(ampis_rle_string_decode(D + u_chars, (const int64_t *)(D + u_off), (int32_t)n, (uint32_t *)(D + d_cnt),
                                  (const int64_t *)(D + u_off), (int32_t *)(D + d_cntlen), stream));
     STEP(ampis_rle_measure_paint_flat((const uint32_t *)(D + d_cnt), (const int64_t *)(D + u_off), (const int32_t *)(D + d_cntlen),
@@ -111,7 +113,7 @@ extern "C" int ampis_eval_image_host(const uint8_t *chars, const int64_t *chr_of
                                       (uint32_t *)(D + d_cum), (uint32_t *)(D + o_area), (int32_t *)(D + o_bbox),
                                       (uint32_t *)(D + o_span), (uint32_t *)(D + d_reg), (int64_t *)(D + d_bitsoff),
                                       (int32_t *)(D + o_status), D + arena0, arena_chunks, (uint64_t *)(D + o_cursor),
-                                      (int32_t *)(D + d_list), (int32_t)(n_chars / n), stream));
+                                      (int32_t *)(D + d_list), (int32_t)(n_chars / n), iv, stream));
     if (dense) {
         e = cudaMemsetAsync(D + x_imoff, 0, 8, st);                 // the image's matrix starts at offset 0
         if (e != cudaSuccess) { ampis_set_error("imat offset: %s", cudaGetErrorString(e)); return AMPIS_ECUDA; }
@@ -123,7 +125,8 @@ extern "C" int ampis_eval_image_host(const uint8_t *chars, const int64_t *chr_of
                                   (int32_t *)(D + g_entbb), grid_cap, (uint64_t *)(D + o_gridtot), stream));
             e = cudaMemsetAsync(D + p_grp, 0, (size_t)(4 * (int64_t)n_rows), st);          // every row belongs to group 0
             if (e != cudaSuccess) { ampis_set_error("row groups: %s", cudaGetErrorString(e)); return AMPIS_ECUDA; }
-            STEP(ampis_intersect_rows_pairs(D + arena0, (const int64_t *)(D + d_bitsoff), (const int32_t *)(D + o_bbox),
+            STEP(ampis_intersect_rows_pairs(D + arena0, (const int64_t *)(D + d_bitsoff),
+                                            iv ? (const uint32_t *)(D + d_reg) : nullptr, (const int32_t *)(D + o_bbox),
                                             (const uint32_t *)(D + o_area), (const int32_t *)(D + u_rowmask),
                                             (const int32_t *)(D + p_grp), n_rows, (const int32_t *)(D + u_grb),
                                             (const int32_t *)(D + u_gcb), (const int32_t *)(D + u_gcc),

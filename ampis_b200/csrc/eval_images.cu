@@ -37,7 +37,8 @@ __global__ void crowd_gate_kernel(unsigned long long *pair_count, unsigned long 
     if (limit >= 0 && (long long)n > limit) { *flag = 1; } else { *flag = 0; }
 }
 
-extern "C" int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_bits_off, const int32_t *d_bbox,
+extern "C" int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_bits_off, const uint32_t *d_reg,
+                                          const int32_t *d_bbox,
                                           const uint32_t *d_area, const int32_t *d_row_mask, const int32_t *d_row_grp,
                                           int32_t n_rows, const int32_t *d_grp_row_begin,
                                           const int32_t *d_grp_col_begin, const int32_t *d_grp_col_count,
@@ -340,6 +341,8 @@ static int images_front(const ImagesIn &in, ImagesExtra &x, double crowd_frac, I
     // ---- kernels --------------------------------------------------------------------------------------------------
     int rc;
 #define STEP(call) do { rc = (call); if (rc != AMPIS_OK) return rc; } while (0)
+    // the windows go to the pairs join and nowhere else: interval form for the column-convex masks
+    const int32_t iv = ampis_pairs_read_intervals();
     if (on_device) {
         expand_images_kernel<<<n_images, 256, 0, st>>>(
             (const int *)(D + i_nr), (const int *)(D + i_nc), (const u32 *)(D + i_h), (const u32 *)(D + i_w),
@@ -358,7 +361,7 @@ static int images_front(const ImagesIn &in, ImagesExtra &x, double crowd_frac, I
                                       (uint32_t *)(D + o_area), (int32_t *)(D + o_bbox), (uint32_t *)(D + o_span),
                                       (uint32_t *)(D + d_reg), (int64_t *)(D + d_bitsoff), (int32_t *)(D + o_status),
                                       D + arena0, arena_chunks, (uint64_t *)(D + o_cursor), (int32_t *)(D + d_list),
-                                      (int32_t)(n_chars / n), in.stream));
+                                      (int32_t)(n_chars / n), iv, in.stream));
     e = cudaMemsetAsync(D + o_gridtot, 0, (size_t)(o_crowd + 8 - o_gridtot), st);      // grid total, pair total, pairs found, crowd flag
     if (e != cudaSuccess) { ampis_set_error("memset: %s", cudaGetErrorString(e)); return AMPIS_ECUDA; }
     if (r.have_rows) {
@@ -368,7 +371,8 @@ static int images_front(const ImagesIn &in, ImagesExtra &x, double crowd_frac, I
         // crowd gate: more candidate pairs than crowd_frac of all pairs -> the intersections are not computed
         const long long limit = crowd_frac >= 0.0 && crowd_frac < 1.0 ? (long long)(crowd_frac * (double)all_pairs) : -1;
         const int64_t cap = limit >= 0 && limit < pair_cap ? limit : pair_cap;
-        STEP(ampis_intersect_rows_pairs(D + arena0, (const int64_t *)(D + d_bitsoff), (const int32_t *)(D + o_bbox),
+        STEP(ampis_intersect_rows_pairs(D + arena0, (const int64_t *)(D + d_bitsoff),
+                                        iv ? (const uint32_t *)(D + d_reg) : nullptr, (const int32_t *)(D + o_bbox),
                                         (const uint32_t *)(D + o_area), (const int32_t *)(D + x_rowmask),
                                         (const int32_t *)(D + x_rowgrp), (int32_t)R, (const int32_t *)(D + x_grb),
                                         (const int32_t *)(D + x_gcb), (const int32_t *)(D + x_gcc),

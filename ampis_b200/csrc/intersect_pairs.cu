@@ -17,6 +17,11 @@
 //       pair and the whole warp for large overlaps, is the first form of the pass: AMPIS_PI_FLAT=0.)
 //   rows_from_pairs_kernel   one thread per row: IoU / overlap score of its pairs, first arg-max (ties broken on the
 //       column index, so the order of a row's pairs does not matter), dense matrix cells and sparse triplets.
+//
+// Either side of a pair may be an INTERVAL window (one word per column, AMPIS_WIN_INTERVALS; rle_flat.cu).  Its
+// descriptor side then reads PD_IV | first band of the overlap instead of the words per column, and its word offset
+// points at the first overlap column.  An interval x interval column is two loads and a closed form; an interval x
+// bitmap column turns the interval into bands on the fly.  Only pair_intersect_flat_kernel reads interval windows.
 #include <algorithm>
 #include <cstdlib>
 #include "common.cuh"
@@ -36,9 +41,28 @@ struct __align__(16) PairDesc {
     i64 a_word, b_word;
     u32 rn, cn, nw, ncols;
 };
+#define PD_IV 0x80000000u                // rn / cn flag: that side is an interval window; the low bits = first band
+
+// the descriptor of the pair (row mask rm with box rb at word a_base, column mask cm with box cbx): overlap of the two
+// windows (crop_common.cuh: overlap_of) as word offsets.  ia / ib: the side is an interval window
+__device__ __forceinline__ PairDesc pair_desc_of(i64 a_base, int4 rb, bool ia, i64 b_base, int4 cbx, bool ib)
+{
+    const u32 xa = (u32)max(rb.x, cbx.x), xb = (u32)min(rb.z, cbx.z);
+    const u32 rw0 = (u32)rb.y >> 5, rw1 = (u32)rb.w >> 5, cw0 = (u32)cbx.y >> 5, cw1 = (u32)cbx.w >> 5;
+    const u32 wa = max(rw0, cw0), wb = min(rw1, cw1);
+    PairDesc d;
+    d.rn = ia ? PD_IV | wa : rw1 - rw0 + 1u;
+    d.cn = ib ? PD_IV | wa : cw1 - cw0 + 1u;
+    d.nw = wb - wa + 1u;
+    d.ncols = xb - xa + 1u;
+    d.a_word = a_base + (ia ? (i64)(xa - (u32)rb.x) : (i64)(xa - (u32)rb.x) * d.rn + (wa - rw0));
+    d.b_word = b_base + (ib ? (i64)(xa - (u32)cbx.x) : (i64)(xa - (u32)cbx.x) * d.cn + (wa - cw0));
+    return d;
+}
 
 struct PairJoinArgs {
     const i64 *bits_off;
+    const uint2 *reg;                    // NULL: every window is a bitmap
     PairDesc *pair_desc;
     const int4 *bbox;
     const u32 *area;
@@ -126,21 +150,12 @@ pairs_from_grid_kernel(const PairJoinArgs p)
     p.row_pair_cnt[r] = room ? cnt : 0;
     if (!room || cnt == 0) return;
     const i64 a_base = p.bits_off[rm] * 4;
+    const bool ia = p.reg && (p.reg[rm].x & AMPIS_WIN_INTERVALS);
     auto put = [&](i64 q, int k, const int4 cbx) {
         const int cm = cb + k;
         p.pair_ab[q] = make_int2(rm, cm);
-        // overlap of the two windows (crop_common.cuh: overlap_of), as word offsets
-        const u32 xa = (u32)max(rb.x, cbx.x), xb = (u32)min(rb.z, cbx.z);
-        const u32 rw0 = (u32)rb.y >> 5, rw1 = (u32)rb.w >> 5, cw0 = (u32)cbx.y >> 5, cw1 = (u32)cbx.w >> 5;
-        const u32 wa = max(rw0, cw0), wb = min(rw1, cw1);
-        PairDesc d;
-        d.rn = rw1 - rw0 + 1u;
-        d.cn = cw1 - cw0 + 1u;
-        d.nw = wb - wa + 1u;
-        d.ncols = xb - xa + 1u;
-        d.a_word = a_base + (i64)(xa - (u32)rb.x) * d.rn + (wa - rw0);
-        d.b_word = __ldg(p.bits_off + cm) * 4 + (i64)(xa - (u32)cbx.x) * d.cn + (wa - cw0);
-        p.pair_desc[q] = d;
+        p.pair_desc[q] = pair_desc_of(a_base, rb, ia, __ldg(p.bits_off + cm) * 4, cbx,
+                                      p.reg && (__ldg(&p.reg[cm].x) & AMPIS_WIN_INTERVALS));
     };
     if (cnt <= PJ_KEEP) {
 #pragma unroll
@@ -226,20 +241,12 @@ pairs_from_grid8_kernel(const PairJoinArgs p)
     if (!room || cnt == 0) return;
     const i64 mine = first + (incl - (u32)cnt);
     const i64 a_base = p.bits_off[rm] * 4;
+    const bool ia = p.reg && (p.reg[rm].x & AMPIS_WIN_INTERVALS);
     auto put = [&](i64 q, int k, const int4 cbx) {
         const int cm = cb + k;
         p.pair_ab[q] = make_int2(rm, cm);
-        const u32 xa = (u32)max(rb.x, cbx.x), xb = (u32)min(rb.z, cbx.z);
-        const u32 rw0 = (u32)rb.y >> 5, rw1 = (u32)rb.w >> 5, cw0 = (u32)cbx.y >> 5, cw1 = (u32)cbx.w >> 5;
-        const u32 wa = max(rw0, cw0), wb = min(rw1, cw1);
-        PairDesc d;
-        d.rn = rw1 - rw0 + 1u;
-        d.cn = cw1 - cw0 + 1u;
-        d.nw = wb - wa + 1u;
-        d.ncols = xb - xa + 1u;
-        d.a_word = a_base + (i64)(xa - (u32)rb.x) * d.rn + (wa - rw0);
-        d.b_word = __ldg(p.bits_off + cm) * 4 + (i64)(xa - (u32)cbx.x) * d.cn + (wa - cw0);
-        p.pair_desc[q] = d;
+        p.pair_desc[q] = pair_desc_of(a_base, rb, ia, __ldg(p.bits_off + cm) * 4, cbx,
+                                      p.reg && (__ldg(&p.reg[cm].x) & AMPIS_WIN_INTERVALS));
     };
     if (cnt <= PJ8_KEEP) {
         put(mine, k0, __ldg(p.bbox + cb + k0));
@@ -330,15 +337,18 @@ pair_intersect_kernel(const u32 *__restrict__ words, const PairDesc *__restrict_
 // pairs of a warp ran in lockstep to the trip count of the largest, 2/3 of the lanes busy on average.
 #define PF_PAIRS 8
 #define PF_WORDS 4u
+// interval x interval: columns per item (four loads of a lane in flight; four columns spill at 40 registers)
+#define PF_IV_COLS 2u
 
 struct __align__(16) PfWarp {
     uint4 lo[PF_PAIRS], hi[PF_PAIRS];       // the descriptors of the batch
     u32 start[PF_PAIRS + 1];                // first item of every pair
-    u32 nsub[PF_PAIRS];                     // items per overlap column
+    u32 nsub[PF_PAIRS];                     // items per overlap column (0: PF_IV_COLS columns per item)
     u32 acc[PF_PAIRS];
 };
 
-// U = passes of 32 items a warp has in flight (their loads are issued before the first popcount)
+// U = passes of 32 items a warp has in flight (their loads are issued before the first popcount).  Only U = 1 (the
+// default) reads interval windows: with them the two-pass form spills (72 bytes) at the 40 registers of 6 CTAs per SM
 template <int U>
 __global__ void __launch_bounds__(256, 6)
 pair_intersect_flat_kernel(const u32 *__restrict__ words, const PairDesc *__restrict__ pair_desc,
@@ -364,8 +374,10 @@ pair_intersect_flat_kernel(const u32 *__restrict__ words, const PairDesc *__rest
                 const uint4 *src = reinterpret_cast<const uint4 *>(pair_desc + q0 + lane);
                 lo = __ldg(src);
                 hi = __ldg(src + 1);
-                ns = max((hi.z + PF_WORDS - 1u) / PF_WORDS, 1u);
-                items = hi.z ? hi.w * ns : 0u;
+                // interval x interval: PF_IV_COLS columns per item whatever the height
+                const bool ii = U == 1 && (hi.x & hi.y & PD_IV);
+                ns = ii ? 0u : max((hi.z + PF_WORDS - 1u) / PF_WORDS, 1u);
+                items = hi.z ? (ii ? (hi.w + PF_IV_COLS - 1u) / PF_IV_COLS : hi.w * ns) : 0u;
             }
             S.lo[lane] = lo; S.hi[lane] = hi; S.nsub[lane] = ns; S.acc[lane] = 0u;
         }
@@ -382,14 +394,14 @@ pair_intersect_flat_kernel(const u32 *__restrict__ words, const PairDesc *__rest
         const u32 s1 = S.start[1], s2 = S.start[2], s3 = S.start[3], s4 = S.start[4], s5 = S.start[5], s6 = S.start[6],
                   s7 = S.start[7];
         for (u32 c0 = 0; c0 < T; c0 += 32 * U) {
-            u32 v[U], j[U], it[U], x0[U], x1[U], wa[U], wb[U];
+            u32 v[U], j[U], it[U], x0[U], x1[U], wa[U], wb[U], iv[U];
             const u32 *pa[U], *pb[U];
             bool ok[U];
 #pragma unroll
             for (int u = 0; u < U; u++) {
                 const u32 c = c0 + 32u * u + lane;
                 ok[u] = c < T;
-                v[u] = 0u; j[u] = 0u; it[u] = 0u; x0[u] = 0u; x1[u] = 0u; wa[u] = 0u; wb[u] = 0u;
+                v[u] = 0u; j[u] = 0u; it[u] = 0u; x0[u] = 0u; x1[u] = 0u; wa[u] = 0u; wb[u] = 0u; iv[u] = 0u;
                 pa[u] = pb[u] = words;
                 if (ok[u]) {
                     j[u] = (u32)(c >= s1) + (u32)(c >= s2) + (u32)(c >= s3) + (u32)(c >= s4) + (u32)(c >= s5) +
@@ -402,18 +414,42 @@ pair_intersect_flat_kernel(const u32 *__restrict__ words, const PairDesc *__rest
                         dx = it[u] / ns;
                         w0 = (it[u] - dx * ns) * PF_WORDS;
                         w1 = min(hi.z, w0 + PF_WORDS);
+                    } else if (ns == 0u) {
+                        dx = it[u] * PF_IV_COLS;
                     }
-                    pa[u] = words + (i64)(((u64)lo.y << 32) | lo.x) + (i64)dx * hi.x + w0;
-                    pb[u] = words + (i64)(((u64)lo.w << 32) | lo.z) + (i64)dx * hi.y + w0;
+                    const bool ia = U == 1 && (hi.x & PD_IV), ib = U == 1 && (hi.y & PD_IV);
+                    pa[u] = words + (i64)(((u64)lo.y << 32) | lo.x) + (ia ? (i64)dx : (i64)dx * hi.x + w0);
+                    pb[u] = words + (i64)(((u64)lo.w << 32) | lo.z) + (ib ? (i64)dx : (i64)dx * hi.y + w0);
                     wa[u] = w0; wb[u] = w1;
-                    // the first two bands of the column (most overlaps have one or two): all loads of all passes in flight
-                    x0[u] = __ldg(pa[u]) & __ldg(pb[u]);
-                    if (w0 + 1u < w1) x1[u] = __ldg(pa[u] + 1) & __ldg(pb[u] + 1);
+                    if (!(ia | ib)) {
+                        // the first two bands of the column (most overlaps have one or two): all loads of all passes
+                        // in flight
+                        x0[u] = __ldg(pa[u]) & __ldg(pb[u]);
+                        if (w0 + 1u < w1) x1[u] = __ldg(pa[u] + 1) & __ldg(pb[u] + 1);
+                    } else if (ia & ib) {
+                        const u32 left = hi.w - dx;
+                        u32 qa[PF_IV_COLS], qb[PF_IV_COLS];
+#pragma unroll
+                        for (u32 k = 0; k < PF_IV_COLS; k++) {
+                            qa[k] = k < left ? __ldg(pa[u] + k) : 0u;         // a zero word is an empty column
+                            qb[k] = k < left ? __ldg(pb[u] + k) : 0u;
+                        }
+#pragma unroll
+                        for (u32 k = 0; k < PF_IV_COLS; k++) iv[u] += interval_overlap(qa[k], qb[k]);
+                        wb[u] = w0;
+                    } else {
+                        // interval x bitmap: the interval word as bands (wa..) of the overlap, ANDed with the bitmap's
+                        const u32 v = __ldg(ia ? pa[u] : pb[u]), y0 = ((ia ? hi.x : hi.y) & ~PD_IV) * 32u;
+                        const u32 *bm = ia ? pb[u] : pa[u];
+                        for (u32 w = w0; w < w1; w++)
+                            iv[u] += __popc(interval_band(v, y0 + 32u * w) & __ldg(bm + (w - w0)));
+                        wb[u] = w0;
+                    }
                 }
             }
 #pragma unroll
             for (int u = 0; u < U; u++) {
-                v[u] = __popc(x0[u]) + __popc(x1[u]);
+                v[u] = __popc(x0[u]) + __popc(x1[u]) + iv[u];
                 for (u32 w = wa[u] + 2u; w < wb[u]; w++) v[u] += __popc(__ldg(pa[u] + (w - wa[u])) & __ldg(pb[u] + (w - wa[u])));
                 // sums per pair: the lanes of a pair are contiguous
                 const u32 reach = ok[u] ? min(lane, it[u]) : 0u;
@@ -506,7 +542,18 @@ rows_from_pairs_kernel(const PairRowArgs p)
     p.best_score[r] = best_s;
 }
 
-extern "C" int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_bits_off, const int32_t *d_bbox,
+// AMPIS_PI_FLAT: 1 (default) = lanes over the concatenated columns of eight pairs, 2 = the same with two passes in
+// flight, 0 = eight lanes per pair (profiles/experiments_r02.md: 0.395 / 0.387 / 0.383 ms of rows per C2 step)
+static int pi_flat()
+{
+    static const int flat = [] { const char *v = getenv("AMPIS_PI_FLAT"); return v ? atoi(v) : 1; }();
+    return flat;
+}
+
+extern "C" int ampis_pairs_read_intervals(void) { return pi_flat() == 1; }
+
+extern "C" int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_bits_off, const uint32_t *d_reg,
+                                          const int32_t *d_bbox,
                                           const uint32_t *d_area, const int32_t *d_row_mask, const int32_t *d_row_grp,
                                           int32_t n_rows, const int32_t *d_grp_row_begin,
                                           const int32_t *d_grp_col_begin, const int32_t *d_grp_col_count,
@@ -523,6 +570,7 @@ extern "C" int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_b
 {
     AMPIS_REQUIRE(n_rows >= 0 && pair_capacity >= 0 && grid_capacity >= 0 && imat_ints >= 0, "negative size");
     AMPIS_REQUIRE(mode == AMPIS_MODE_IOU || mode == AMPIS_MODE_SAT, "bad mode");
+    AMPIS_REQUIRE(!d_reg || ampis_pairs_read_intervals(), "interval windows need the default pair pass (AMPIS_PI_FLAT=1)");
     if (n_rows == 0) return AMPIS_OK;
     AMPIS_REQUIRE(d_bits_off && d_bbox && d_area && d_row_mask && d_row_grp && d_grp_row_begin && d_grp_col_begin &&
                       d_grp_col_count && d_grp_shift && d_cell_off && d_row_pair_off && d_row_pair_cnt &&
@@ -554,7 +602,7 @@ extern "C" int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_b
     }
     if (e != cudaSuccess) { ampis_set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return AMPIS_ECUDA; }
     PairJoinArgs j;
-    j.bits_off = d_bits_off; j.pair_desc = (PairDesc *)d_pair_desc;
+    j.bits_off = d_bits_off; j.reg = (const uint2 *)d_reg; j.pair_desc = (PairDesc *)d_pair_desc;
     j.bbox = (const int4 *)d_bbox; j.area = d_area; j.row_mask = d_row_mask; j.row_grp = d_row_grp; j.n_rows = n_rows;
     j.grp_col_begin = d_grp_col_begin; j.grp_col_count = d_grp_col_count; j.grp_shift = d_grp_shift;
     j.cell_off = d_cell_off; j.entries = d_entries; j.entry_bbox = (const int4 *)d_entry_bbox;
@@ -577,9 +625,7 @@ extern "C" int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_b
         i64 want = (pair_capacity + 31) / 32;                      // 8 warps x 4 pairs per CTA and trip
         const i64 cap = 148 * 8 * 8;
         if (want > cap) want = cap;
-        // AMPIS_PI_FLAT: 1 (default) = lanes over the concatenated columns of eight pairs, 2 = the same with two passes in
-        // flight, 0 = eight lanes per pair (profiles/experiments_r02.md: 0.395 / 0.387 / 0.383 ms of rows per C2 step)
-        static const int flat = [] { const char *v = getenv("AMPIS_PI_FLAT"); return v ? atoi(v) : 1; }();
+        const int flat = pi_flat();
         if (flat == 1)
             pair_intersect_flat_kernel<1><<<(unsigned)std::min<i64>((pair_capacity + 63) / 64, cap), 256, 0, st>>>(
                 (const u32 *)d_bits, (const PairDesc *)d_pair_desc, d_pair_inter, (const unsigned long long *)d_pair_count,

@@ -27,6 +27,14 @@
 // Masks that do not fit the per-warp budgets (more than FL_PAIR_CAP pairs, window larger than the tile, frame of
 // 2^31 pixels or more or taller than 65,536 rows) are appended to a list that rle_measure_paint_list_kernel (a warp
 // per mask, any size; rle_paint.cu) works off in a second launch.
+//
+// Interval windows (IV = true; asked for by callers whose table only goes to the pairs join, intersect_pairs.cu):
+// a COLUMN-CONVEX mask -- every 1-run inside one column, no column with two 1-runs, as every particle blob of the
+// synthetic data and most real particles are -- is stored as ONE word per box column, (first row ^ 0xffff) | last
+// row << 16, so that a zero word is an empty column (AMPIS_WIN_INTERVALS in reg.x; common.cuh).  The measure pass
+// tests the property per pair, without a scan: a pair after the first of its mask whose 0-run is shorter than the
+// first row of its 1-run has the previous 1-run in the same column.  The painter then stores one word per 1-run
+// instead of OR-ing bands.
 #include <algorithm>
 #include "common.cuh"
 #include "rle_measure.cuh"
@@ -54,6 +62,7 @@ struct __align__(16) FlatWarp {
     const u32 *src[FL_KMAX];        // per mask of the warp: its first run count
     u32 pb[FL_KMAX + 1];            // first pair of every mask of the round
     u32 area[FL_KMAX], first[FL_KMAX], last[FL_KMAX], ymin[FL_KMAX], ymaxi[FL_KMAX], total[FL_KMAX];
+    u32 convex[FL_KMAX];            // per mask of the round: column-convex so far (IV only)
     uint8_t mid[FL_PAIR_CAP];       // mask (index inside the round) of every pair
 };
 
@@ -94,7 +103,7 @@ __device__ __forceinline__ void paint_rows(u32 *tile, u32 idx, u32 ys, u32 yl)
 
 // Persistent: the grid is one wave (FL_CTAS_PER_SM CTAs per SM) and every warp strides over the groups of K masks,
 // so no SM waits for the slowest warp of a CTA before it is given new work.
-template <bool ZERO>
+template <bool ZERO, bool IV>
 __global__ void __launch_bounds__(FL_WARPS * 32, FL_CTAS_PER_SM)
 rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_off, const int *__restrict__ cnt_len,
                      const u32 *__restrict__ hh, const u32 *__restrict__ ww, int n, int K,
@@ -106,9 +115,10 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
     __shared__ FlatWarp s_warp[FL_WARPS];
     FlatWarp &S = s_warp[threadIdx.x >> 5];
     const u32 lane = lane_id();
-    const i64 nwarps = (i64)gridDim.x * FL_WARPS;
-    for (i64 gw = (i64)blockIdx.x * FL_WARPS + (threadIdx.x >> 5); gw * K < n; gw += nwarps) {
-        const i64 i0 = gw * K;
+    // 32-bit group counter (gw < n < 2^31, one wave of warps added): a 64-bit one spills in the interval variant
+    const u32 nwarps = gridDim.x * FL_WARPS;
+    for (u32 gw = blockIdx.x * FL_WARPS + (threadIdx.x >> 5); (i64)gw * K < n; gw += nwarps) {
+        const i64 i0 = (i64)gw * K;
         const int nm = (int)min((i64)K, (i64)n - i0);
 
         // ---- side job: this group's share of a buffer the caller wants zeroed (the dense matrices of the rows that
@@ -150,6 +160,7 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
                 if (j_me == nb - 1) S.pb[nb] = T;
                 S.area[j_me] = 0u; S.first[j_me] = 0xffffffffu; S.last[j_me] = 0u;
                 S.ymin[j_me] = 0xffffffffu; S.ymaxi[j_me] = 0xffffffffu; S.total[j_me] = 0u;
+                if (IV) S.convex[j_me] = 1u;
                 if (my_big) big[1 + atomicAdd(&big[0], 1)] = (int)(i0 + lane);
             }
             __syncwarp();
@@ -192,6 +203,10 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
                 if (good) {
                     const u32 x = div_by(start, H, rcp);
                     const u32 ys = start - x * H, yl = ys + o - 1u;
+                    // column-convex test (IV): a 1-run over several columns, or one whose 0-run starts in its own
+                    // column behind an earlier pair of the mask -- the 1-run before it ends in this column, or (a
+                    // zero-length 1-run in between; conservative) the gap only looks so -- makes the mask a bitmap
+                    if (IV && (yl >= H || (p > 0u && z < ys))) S.convex[j] = 0u;
                     if (yl >= H) { pr = make_uint2(start | FL_SPAN, o); ypk = (0xffffu - (H - 1u)) << 16; }
                     else { pr = make_uint2(x, ys | (yl << 16)); ypk = ys | ((0xffffu - yl) << 16); }
                 }
@@ -236,11 +251,15 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
                     bb = make_int4((int)div_by(fi, H, geo.y), (int)S.ymin[j_me], (int)div_by(la - 1u, H, geo.y),
                                    (int)(0xffffu - S.ymaxi[j_me]));
                 }
-                chunks = (crop_words(bb) + 3u) / 4u;
+                // an interval window is never larger than the bitmap window: the arena sizes of measure() still hold
+                // (S.convex[j_me] says from here on whether the mask is stored as intervals: no register for it)
+                if (IV && ar == 0u) S.convex[j_me] = 0u;
+                chunks = IV && S.convex[j_me] ? ((u32)(bb.z - bb.x) + 4u) / 4u : (crop_words(bb) + 3u) / 4u;
                 const i64 i = i0 + lane;
                 area[i] = ar;
                 reinterpret_cast<int4 *>(bbox)[i] = bb;
                 reinterpret_cast<uint2 *>(span)[i] = sp;
+                // a bitmap until painted below: a window larger than the tile goes to the fallback kernel as a bitmap
                 reinterpret_cast<uint2 *>(reg)[i] = make_uint2(0u, chunks);
                 status[i] = S.total[j_me] == HW ? 0 : AMPIS_ST_BAD_TOTAL;
             }
@@ -271,8 +290,14 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
                     const i64 i = i0 + lane;
                     if (room) {
                         bits_off[i] = (i64)base + (rel - chunks);
-                        const u32 wy0 = (u32)bb.y >> 5, nwy = ((u32)bb.w >> 5) - wy0 + 1u;
-                        S.win[j_me] = make_uint4(geo.x, geo.y, (rel - chunks) * 4u - (u32)bb.x * nwy - wy0, nwy);
+                        if (IV && S.convex[j_me]) {
+                            // one word per column; 0 bands per column tells the painter
+                            reinterpret_cast<uint2 *>(reg)[i] = make_uint2(AMPIS_WIN_INTERVALS, chunks);
+                            S.win[j_me] = make_uint4(geo.x, geo.y, (rel - chunks) * 4u - (u32)bb.x, 0u);
+                        } else {
+                            const u32 wy0 = (u32)bb.y >> 5, nwy = ((u32)bb.w >> 5) - wy0 + 1u;
+                            S.win[j_me] = make_uint4(geo.x, geo.y, (rel - chunks) * 4u - (u32)bb.x * nwy - wy0, nwy);
+                        }
                     } else {
                         // arena exhausted: the caller sees *cursor > capacity and retries; until then the mask is empty
                         // for every later kernel (the crop rows kernels size their reads from the box)
@@ -294,7 +319,9 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
                             const u32 ys = pr.y & 0xffffu, yl = pr.y >> 16;
                             if (ys > yl) continue;
                             const uint4 d = S.win[S.mid[f]];
-                            paint_rows(S.tile, d.z + pr.x * d.w, ys, yl);
+                            // interval window: the column's only 1-run; a word left zero is an empty column
+                            if (IV && d.w == 0u) S.tile[d.z + pr.x] = pr.y ^ 0xffffu;
+                            else paint_rows(S.tile, d.z + pr.x * d.w, ys, yl);
                         } else {
                             const uint4 d = S.win[S.mid[f]];
                             const u32 s = pr.x & ~FL_SPAN;
@@ -342,7 +369,8 @@ extern "C" int ampis_rle_measure_paint_flat_zero(const uint32_t *d_cnt, const in
                                                  uint32_t *d_area, int32_t *d_bbox, uint32_t *d_span, uint32_t *d_reg,
                                                  int64_t *d_bits_off, int32_t *d_status, void *d_bits,
                                                  int64_t bits_capacity, uint64_t *d_cursor, int32_t *d_list,
-                                                 int32_t runs_hint, void *d_zero, int64_t zero_bytes, void *stream)
+                                                 int32_t runs_hint, void *d_zero, int64_t zero_bytes,
+                                                 int32_t intervals, void *stream)
 {
     AMPIS_REQUIRE(n >= 0 && zero_bytes >= 0, "n < 0 or zero_bytes < 0");
     cudaStream_t st = as_stream(stream);
@@ -377,18 +405,14 @@ extern "C" int ampis_rle_measure_paint_flat_zero(const uint32_t *d_cnt, const in
             wave = 148 * FL_CTAS_PER_SM;
     }
     const unsigned grid = (unsigned)std::min<int64_t>((warps + FL_WARPS - 1) / FL_WARPS, wave);
-    if (zero_chunks > 0) {
-        // (groups - 1) x share < chunks + groups <= 2^32
-        const uint32_t per = (uint32_t)((zero_chunks + warps - 1) / warps);
-        rle_flat_crop_kernel<true><<<grid, FL_WARPS * 32, 0, st>>>(
-            d_cnt, d_cnt_off, d_cnt_len, d_h, d_w, n, K, d_area, d_bbox, d_span, d_reg, d_bits_off, d_status,
-            (uint4 *)d_bits, bits_capacity, (unsigned long long *)d_cursor, d_list, (uint4 *)d_zero,
-            (uint32_t)zero_chunks, per);
-    } else {
-        rle_flat_crop_kernel<false><<<grid, FL_WARPS * 32, 0, st>>>(
-            d_cnt, d_cnt_off, d_cnt_len, d_h, d_w, n, K, d_area, d_bbox, d_span, d_reg, d_bits_off, d_status,
-            (uint4 *)d_bits, bits_capacity, (unsigned long long *)d_cursor, d_list, nullptr, 0u, 0u);
-    }
+    // (groups - 1) x share < chunks + groups <= 2^32
+    const uint32_t per = zero_chunks > 0 ? (uint32_t)((zero_chunks + warps - 1) / warps) : 0u;
+    auto kernel = zero_chunks > 0 ? (intervals ? rle_flat_crop_kernel<true, true> : rle_flat_crop_kernel<true, false>)
+                                  : (intervals ? rle_flat_crop_kernel<false, true> : rle_flat_crop_kernel<false, false>);
+    kernel<<<grid, FL_WARPS * 32, 0, st>>>(d_cnt, d_cnt_off, d_cnt_len, d_h, d_w, n, K, d_area, d_bbox, d_span, d_reg,
+                                           d_bits_off, d_status, (uint4 *)d_bits, bits_capacity,
+                                           (unsigned long long *)d_cursor, d_list,
+                                           zero_chunks > 0 ? (uint4 *)d_zero : nullptr, (uint32_t)zero_chunks, per);
     AMPIS_CHECK_LAUNCH("rle_flat_crop_kernel");
     return ampis_launch_measure_paint_list(d_cnt, d_cnt_off, d_cnt_len, d_h, d_w, d_list, n, d_cum, d_area, d_bbox,
                                            d_span, d_reg, d_bits_off, d_status, d_bits, bits_capacity, d_cursor, st);
@@ -399,9 +423,9 @@ extern "C" int ampis_rle_measure_paint_flat(const uint32_t *d_cnt, const int64_t
                                             uint32_t *d_area, int32_t *d_bbox, uint32_t *d_span, uint32_t *d_reg,
                                             int64_t *d_bits_off, int32_t *d_status, void *d_bits,
                                             int64_t bits_capacity, uint64_t *d_cursor, int32_t *d_list,
-                                            int32_t runs_hint, void *stream)
+                                            int32_t runs_hint, int32_t intervals, void *stream)
 {
     return ampis_rle_measure_paint_flat_zero(d_cnt, d_cnt_off, d_cnt_len, d_h, d_w, n, d_cum, d_area, d_bbox, d_span,
                                              d_reg, d_bits_off, d_status, d_bits, bits_capacity, d_cursor, d_list,
-                                             runs_hint, nullptr, 0, stream);
+                                             runs_hint, nullptr, 0, intervals, stream);
 }

@@ -85,6 +85,9 @@ class MaskTable(object):
         self.zeroed = False     # the last measure_paint also cleared the buffer it was handed
         self.bits = None
         self.bits_capacity = 0
+        # the last measure_paint may have stored column-convex masks as interval windows (one word per column), which
+        # only the pairs join reads: see measure_paint(intervals=True) and require_bitmaps()
+        self.intervals = False
 
     # -- construction steps ---------------------------------------------------------------
     def measure(self):
@@ -104,6 +107,7 @@ class MaskTable(object):
             arena = torch.empty(4 * max(total, 1), dtype=torch.int32, device=self.device)
         self.bits = arena
         self.bits_capacity = arena.numel() // 4
+        self.intervals = False
         if self.layout == LAYOUT_CROP:
             N.call('ampis_rle_decode_crop', _p(self.cum), _p(self.cnt_off), _p(self.cnt_len), _p(self.bbox),
                    _p(self.h), _p(self.bits_off), self.n, _p(self.bits), self.bits_capacity, _stream())
@@ -112,13 +116,16 @@ class MaskTable(object):
                    _p(self.reg), _p(self.bits_off), self.n, _p(self.bits), self.bits_capacity, _stream())
         return self
 
-    def measure_paint(self, arena, zero=None):
+    def measure_paint(self, arena, zero=None, intervals=False):
         """Fused single-launch form of measure() + paint(arena): arena space is handed out by an
         atomic cursor, so the arena must be supplied (size it with a previous measure() or
         generously) and overflow is detected afterwards by check().  zero: a device tensor the launch also clears
         (the dense matrices of the rows that follow; flat crop decode only -- returns with self.zeroed set when the
-        kernel took the job, else the caller clears it)."""
+        kernel took the job, else the caller clears it).  intervals: store column-convex masks as one interval word
+        per column (flat crop decode only; smaller windows, a cheaper decode and join).  Such a table can only go to
+        the pairs join (intersect_rows with ROWS_KERNEL 'pairs'); every other reader of the windows raises."""
         self.zeroed = False
+        self.intervals = False
         self.bits = arena
         self.bits_capacity = arena.numel() // 4
         self.fused = True
@@ -126,21 +133,32 @@ class MaskTable(object):
         if self.layout == LAYOUT_CROP and CROP_DECODE == 'flat':
             if self.list is None:
                 self.list = torch.empty(self.n + 1, dtype=torch.int32, device=self.device)
+            iv = bool(intervals) and pairs_read_intervals()
             if zero is not None and zero.numel() and zero.data_ptr() % 16 == 0:
                 N.call('ampis_rle_measure_paint_flat_zero', _p(self.cnt), _p(self.cnt_off), _p(self.cnt_len),
                        _p(self.h), _p(self.w), self.n, _p(self.cum), _p(self.area), _p(self.bbox), _p(self.span),
                        _p(self.reg), _p(self.bits_off), _p(self.status), _p(self.bits), self.bits_capacity,
-                       _p(self.cursor), _p(self.list), hint, _p(zero), zero.numel() * zero.element_size(), _stream())
+                       _p(self.cursor), _p(self.list), hint, _p(zero), zero.numel() * zero.element_size(), int(iv),
+                       _stream())
                 self.zeroed = True
+                self.intervals = iv
                 return self
             N.call('ampis_rle_measure_paint_flat', _p(self.cnt), _p(self.cnt_off), _p(self.cnt_len), _p(self.h),
                    _p(self.w), self.n, _p(self.cum), _p(self.area), _p(self.bbox), _p(self.span), _p(self.reg),
                    _p(self.bits_off), _p(self.status), _p(self.bits), self.bits_capacity, _p(self.cursor),
-                   _p(self.list), hint, _stream())
+                   _p(self.list), hint, int(iv), _stream())
+            self.intervals = iv
             return self
         N.call('ampis_rle_measure_paint', _p(self.cnt), _p(self.cnt_off), _p(self.cnt_len), _p(self.h), _p(self.w),
                self.n, self.layout, _p(self.cum), _p(self.area), _p(self.bbox), _p(self.span), _p(self.reg),
                _p(self.bits_off), _p(self.status), _p(self.bits), self.bits_capacity, _p(self.cursor), hint, _stream())
+        return self
+
+    def require_bitmaps(self):
+        """Raise unless every window of the table is a bitmap (the form all readers but the pairs join expect)."""
+        if self.intervals:
+            raise ValueError('this mask table holds interval windows (measure_paint(intervals=True)), which only the '
+                             'pairs join reads; decode it with intervals=False for this use')
         return self
 
     def relayout(self, layout):
@@ -169,6 +187,12 @@ class MaskTable(object):
 
     def bbox_np(self):
         return self.bbox[:4 * self.n].cpu().numpy().reshape(-1, 4).copy()
+
+
+def pairs_read_intervals():
+    """True when the pairs join reads interval windows (its default intersection pass; not with the A/B variants
+    AMPIS_PI_FLAT=0 / 2)."""
+    return bool(N.lib().ampis_pairs_read_intervals())
 
 
 def table_from_counts(cnt, cnt_off, cnt_len, h, w, layout=None, arena=None, check=True):
@@ -746,14 +770,16 @@ def intersect_rows(table, groups, mode, out=None, grid=None, sparse=None, pairs=
     zero_stream: a torch stream on which the join zeroes the dense matrices itself while its first two passes run."""
     dev = table.device
     nr = max(groups.n_rows, 1)
+    use_grid = table.layout == LAYOUT_CROP and not isinstance(grid, str) and \
+        (grid is not None or sparse is not None or groups.max_cols >= ROWS_GRID_MIN_COLS)
+    if not (use_grid and ROWS_KERNEL == 'pairs'):
+        table.require_bitmaps()
     if out is None:
         imat = torch.empty(max(groups.imat_size, 1), dtype=torch.int32, device=dev) \
             if groups.imat_off is not None else None
         out = RowResult(torch.empty(nr, dtype=torch.int32, device=dev),
                         torch.empty(nr, dtype=torch.int32, device=dev),
                         torch.empty(nr, dtype=torch.float64, device=dev), imat)
-    use_grid = table.layout == LAYOUT_CROP and not isinstance(grid, str) and \
-        (grid is not None or sparse is not None or groups.max_cols >= ROWS_GRID_MIN_COLS)
     assert use_grid or sparse is None, 'sparse output comes from the grid kernel (crop layout)'
     if use_grid:
         if grid is None:
@@ -769,7 +795,8 @@ def intersect_rows(table, groups, mode, out=None, grid=None, sparse=None, pairs=
             if zeroed is not None and zeroed is not True:
                 torch.cuda.current_stream().wait_event(zeroed)
             while True:
-                N.call('ampis_intersect_rows_pairs', _p(table.bits), _p(table.bits_off), _p(table.bbox),
+                N.call('ampis_intersect_rows_pairs', _p(table.bits), _p(table.bits_off),
+                       _p(table.reg) if table.intervals else None, _p(table.bbox),
                        _p(table.area), _p(groups.row_mask), _p(groups.row_grp), groups.n_rows,
                        _p(groups.grp_row_begin), _p(groups.grp_col_begin), _p(groups.grp_col_count), _p(grid.shift),
                        _p(grid.cell_off), _p(grid.entries), _p(grid.entry_bbox), grid.capacity, _p(pairs.ab),
@@ -861,6 +888,7 @@ def intersect_mma(table, groups, mode, out=None, sort=True, pair=None):
     arg-max from the matrices.  Same RowResult as intersect_rows(), bit for bit; the choice
     between the two is a cost decision (DESIGN.md).  sort=True cuts the tiles from rows / columns
     ordered by position in the image, which shortens the pixel range each tile contracts."""
+    table.require_bitmaps()
     dev = table.device
     assert table.layout != LAYOUT_CROP, 'the contraction reads linear packed masks (span or full layout)'
     nr = max(groups.n_rows, 1)
@@ -890,6 +918,7 @@ def intersect_tma(table, groups, mode, out=None):
     the per-row arg-max from the matrices.  Same RowResult as intersect_rows() / intersect_mma(), bit for bit.  Needs
     a FULL-layout table painted by the unfused path (frames stored regularly, which is what a tensor map describes)
     whose masks all share one frame size.  A measurement kernel (profiles/crossover_r02.md), not a product path."""
+    table.require_bitmaps()
     dev = table.device
     assert table.layout == LAYOUT_FULL and not table.fused, 'regular full frames: MaskTable(..., LAYOUT_FULL).measure().paint()'
     nr = max(groups.n_rows, 1)
@@ -996,6 +1025,7 @@ def edge_distances(table, gt_ids, pred_ids, windows):
     """Boundary disagreement of matched pairs (analyze.mask_edge_distance): for pair i the masks
     gt_ids[i], pred_ids[i] of `table` inside windows[i] = (r1, r2, c1, c2).  Returns
     (counts int64[n, 4], fp_dist float64 device tensor, fn_dist float64 device tensor, off_fp, off_fn)."""
+    table.require_bitmaps()
     assert table.layout != LAYOUT_CROP
     dev = table.device
     n = len(gt_ids)
@@ -1032,6 +1062,7 @@ def hist_u32(values, lo, bin_width, n_bins, hist=None):
 
 def unpack_bool(table, ids, h, w):
     """Packed masks -> bool[n, h, w] device tensor (structures.masks_to_bitmask_array)."""
+    table.require_bitmaps()
     dev = table.device
     assert table.layout != LAYOUT_CROP, 'unpack reads linear packed masks (span or full layout)'
     
@@ -1194,6 +1225,7 @@ def encode_bool(masks):
 
 def project_pairs(table, gt_ids, pred_ids, h, w, mode):
     """Pixel-class frames of analyze.seg_perf_iset as RLE dicts: mode 'reduced' -> 4, 'all' -> 7."""
+    table.require_bitmaps()
     assert table.layout != LAYOUT_CROP
     dev = table.device
     chunks = (int(h) * int(w) + 127) // 128

@@ -129,12 +129,17 @@ int ampis_rle_measure_paint(const uint32_t *d_cnt, const int64_t *d_cnt_off, con
  * record-forming lane per mask, one arena reservation and one contiguous copy-out per warp (csrc/rle_flat.cu).
  * Same outputs as ampis_rle_measure_paint(layout = AMPIS_LAYOUT_CROP), bit for bit; arena order differs.
  * d_list: int32[n + 1] scratch; masks outside the per-warp budgets (more than 512 runs, window larger than 2 KB,
- * frame of 2^31 pixels or more or taller than 65,536 rows) are listed there and worked off by a second launch (a warp per mask, any size). */
+ * frame of 2^31 pixels or more or taller than 65,536 rows) are listed there and worked off by a second launch (a warp per mask, any size).
+ * intervals != 0: a column-convex mask (every 1-run inside one column, at most one per column) decoded by the flat
+ * kernel gets an INTERVAL window instead -- one u32 per box column, (first row ^ 0xffff) | last row << 16, zero for a
+ * column without pixels, reg = [AMPIS_WIN_INTERVALS = 1, ceil(width / 4)) -- which only ampis_intersect_rows_pairs
+ * reads (pass d_reg to it).  0 = bitmap windows for every mask. */
 int ampis_rle_measure_paint_flat(const uint32_t *d_cnt, const int64_t *d_cnt_off, const int32_t *d_cnt_len,
                                  const uint32_t *d_h, const uint32_t *d_w, int32_t n, uint32_t *d_cum,
                                  uint32_t *d_area, int32_t *d_bbox, uint32_t *d_span, uint32_t *d_reg,
                                  int64_t *d_bits_off, int32_t *d_status, void *d_bits, int64_t bits_capacity,
-                                 uint64_t *d_cursor, int32_t *d_list, int32_t runs_hint, void *stream);
+                                 uint64_t *d_cursor, int32_t *d_list, int32_t runs_hint, int32_t intervals,
+                                 void *stream);
 
 /* The same launch with a side job: the kernel also ZEROES d_zero[0 .. zero_bytes) (16-byte aligned; NULL = nothing), a
  * share per group of masks.  The decode is bound by instruction issue and leaves HBM idle, so the dense matrices the
@@ -145,7 +150,7 @@ int ampis_rle_measure_paint_flat_zero(const uint32_t *d_cnt, const int64_t *d_cn
                                       uint32_t *d_area, int32_t *d_bbox, uint32_t *d_span, uint32_t *d_reg,
                                       int64_t *d_bits_off, int32_t *d_status, void *d_bits, int64_t bits_capacity,
                                       uint64_t *d_cursor, int32_t *d_list, int32_t runs_hint, void *d_zero,
-                                      int64_t zero_bytes, void *stream);
+                                      int64_t zero_bytes, int32_t intervals, void *stream);
 
 /* bits -> bool[n][h][w] row-major bytes (RLE.decode(...).astype(bool).transpose(2,0,1),
  * structures.py:752,765).  All n masks must share (h,w). d_mask_ids selects masks. */
@@ -245,7 +250,12 @@ int ampis_intersect_rows_grid(const void *d_bits, const int64_t *d_bits_off, con
  * nothing useful was computed and the caller retries with a larger list.  zero_stream (may be NULL): a second
  * stream on which the dense matrices are zeroed while passes 1 and 2 run on `stream` (fork / join by events inside
  * the call); NULL = zeroed in line. */
-int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_bits_off, const int32_t *d_bbox,
+/* 1 when ampis_intersect_rows_pairs reads interval windows (its default intersection pass, AMPIS_PI_FLAT=1; 0 with
+ * the A/B variants AMPIS_PI_FLAT=0 / 2, where it refuses a non-NULL d_reg).  d_reg: the reg array of a table decoded with intervals on, or
+ * NULL when every window is a bitmap. */
+int ampis_pairs_read_intervals(void);
+int ampis_intersect_rows_pairs(const void *d_bits, const int64_t *d_bits_off, const uint32_t *d_reg,
+                               const int32_t *d_bbox,
                                const uint32_t *d_area, const int32_t *d_row_mask, const int32_t *d_row_grp,
                                int32_t n_rows, const int32_t *d_grp_row_begin, const int32_t *d_grp_col_begin,
                                const int32_t *d_grp_col_count, const int32_t *d_grp_shift,
