@@ -10,12 +10,15 @@
 // warp instructions per mask.  Most of them were per-MASK fixed costs executed by a whole group (five shuffle
 // reductions, the 60-instruction record store, arena reservation, tile zero-fill / copy-out loops with 1-2 trips)
 // and passes in which half of the lanes had no run left (75 runs on 2 x 64 slots).  Here
-//   * the unit of lane work is a PAIR (0-run, 1-run); the K masks a warp owns are laid end to end, so every pass of
-//     32 pairs is full except the last one of the warp;
-//   * run end positions, 1-pixel counts and row ranges come from segmented warp scans (segments = masks), three
-//     shuffles per step for all masks of a pass at once, in 32-bit saturating arithmetic; the last lane of every
-//     segment adds the segment's statistics to its mask with shared-memory atomics.  (Round 2 first reduced every
-//     mask of a pass in turn with REDUX: ~50 instructions per mask and pass, a quarter of the kernel.)
+//   * the unit of work is a PAIR (0-run, 1-run); the K masks a warp owns are laid end to end and taken in rounds of
+//     at most FL_PAIR_CAP = 256 pairs = 32 lanes x 8;
+//   * a round is measured in ONE pass: its pairs are staged in shared memory by coalesced lane-strided loads, then
+//     every lane walks its own slice of 8 consecutive pairs in registers.  Run end positions come from a sequential
+//     walk inside the slice and ONE segmented warp scan across the slices (segments = masks; 32-bit saturating
+//     arithmetic, the "a mask starts here" flag in bit 31); area, first / last 1-pixel and row range are kept per
+//     slice segment in registers and added to the mask with shared-memory atomics once per slice it touches.
+//     (Before: one pair per lane, passes of 32 pairs, three segmented scans, ballots and a carry per pass -- about
+//     half of the kernel's instructions.  Earlier still, a REDUX reduction per mask and pass.)
 //   * the measure pass leaves, per pair, what the painter needs -- column and first / last row of the 1-run in one
 //     64-bit word (runs that cross a column boundary keep start and length and take a slower path) -- and the
 //     per-mask constants of the painter are ONE 128-bit word: no division, no box clipping in the paint loop;
@@ -47,6 +50,7 @@
 #define FL_SAT 0x7fffffffu      // positions saturate here; frames must be smaller
 #define FL_HMAX 65536u          // rows of a column are kept in 16 bits; taller frames go to the fallback kernel
 #define FL_SPAN 0x80000000u     // pair.x flag: the 1-run crosses a column boundary, pair = (start | FL_SPAN, length)
+#define FL_HEAD 0x80000000u     // flag of a measure-scan value: a mask starts in the lane's slice
 
 // What the measure pass leaves for the painter, one per (0-run, 1-run) pair:
 //   1-run inside one column (every run of a blob):  x = column,           y = first row | last row << 16
@@ -63,10 +67,14 @@ struct __align__(16) FlatWarp {
     u32 pb[FL_KMAX + 1];            // first pair of every mask of the round
     u32 area[FL_KMAX], first[FL_KMAX], last[FL_KMAX], ymin[FL_KMAX], ymaxi[FL_KMAX], total[FL_KMAX];
     u32 convex[FL_KMAX];            // per mask of the round: column-convex so far (IV only)
-    uint8_t mid[FL_PAIR_CAP];       // mask (index inside the round) of every pair
+    __align__(8) uint8_t mid[FL_PAIR_CAP];  // mask (index inside the round) of every pair: 8 per lane in one load
 };
 
 __device__ __forceinline__ u32 sat_add(u32 a, u32 b) { return min(a + b, FL_SAT); }
+
+// where pair f of a round is kept in S.pair: bits 1-2 flipped by bits 4-5, so that the 16-byte chunks eight lanes
+// read of their own 8-pair slices fall on distinct banks; 16 consecutive pairs stay a permutation of themselves
+__device__ __forceinline__ u32 fl_swz(u32 f) { return f ^ ((f >> 3) & 6u); }
 
 __device__ __forceinline__ u32 warp_incl_scan(u32 v, u32 lane)
 {
@@ -118,8 +126,8 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
     // 32-bit group counter (gw < n < 2^31, one wave of warps added): a 64-bit one spills in the interval variant
     const u32 nwarps = gridDim.x * FL_WARPS;
     for (u32 gw = blockIdx.x * FL_WARPS + (threadIdx.x >> 5); (i64)gw * K < n; gw += nwarps) {
-        const i64 i0 = (i64)gw * K;
-        const int nm = (int)min((i64)K, (i64)n - i0);
+        const int i0 = (int)gw * K;                     // < n < 2^31 (loop condition); 64 bits would cost a register
+        const int nm = min(K, n - i0);
 
         // ---- side job: this group's share of a buffer the caller wants zeroed (the dense matrices of the rows that
         // follow).  The decode is bound by instruction issue and leaves HBM idle; these few fire-and-forget stores per
@@ -165,73 +173,110 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
             }
             __syncwarp();
 
-            // ---- pass over the pairs, 32 at a time.  Run end positions and 1-pixel counts by ONE pair of segmented
-            // scans (segments = masks), row ranges by a third (16-bit halves: min row | 0xffff - max row); the last
-            // lane of every segment adds the segment's statistics to its mask -- all masks of the pass at once.
-            u32 carry = 0;
-            int j = 0;                                   // my mask: the last one that starts at or before my pair
-            u32 cur = 0, nxt = S.pb[1];                  // its first pair and the next mask's: only grow
-            for (u32 f0 = 0; f0 < T; f0 += 32) {
-                const u32 f = f0 + lane;
-                const bool ok = f < T;
-                u32 p = 0, z = 0, o = 0, H = 1, rcp = 0, HW = 0;
-                if (ok) {
-                    while (f >= nxt) { j++; cur = nxt; nxt = S.pb[j + 1]; }
-                    S.mid[f] = (uint8_t)j;
-                    p = f - cur;
-                    const uint4 g = S.geo[a + j];
-                    H = g.x; rcp = g.y; HW = g.z;
-                    const u32 *c = S.src[a + j] + 2 * p;
-                    z = min(__ldcs(c), FL_SAT);                        // read once: evict first
-                    if ((int)(2 * p + 1) < (int)g.w) o = min(__ldcs(c + 1), FL_SAT);
+            // ---- staging: the round's raw pairs, lane-strided (coalesced reads of the run counts), and the mask of
+            // every pair.  The round is padded to whole slices of 8 with (0, 0) pairs of its last mask: they move no
+            // end, add no pixel and paint nothing.
+            const u32 Tr = (T + 7u) & ~7u;
+            {
+                int j = 0;
+                u32 cur = 0, nxt = S.pb[1];              // my mask's first pair and the next mask's: only grow
+                for (u32 f = lane; f < Tr; f += 32) {
+                    uint2 zo = make_uint2(0u, 0u);
+                    if (f < T) {
+                        while (f >= nxt) { j++; cur = nxt; nxt = S.pb[j + 1]; }
+                        const u32 p = f - cur;
+                        const u32 *c = S.src[a + j] + 2 * p;
+                        zo.x = min(__ldcs(c), FL_SAT);                      // read once: evict first
+                        if ((int)(2 * p + 1) < (int)S.geo[a + j].w) zo.y = min(__ldcs(c + 1), FL_SAT);
+                    }
+                    S.mid[f] = (uint8_t)(f < T ? j : nb - 1);
+                    S.pair[fl_swz(f)] = zo;
                 }
-                u32 end = sat_add(z, o), osum = o;
-                const u32 reach = ok ? min(lane, p) : 0u;            // lanes below me that belong to my mask
+            }
+            __syncwarp();
+
+            // ---- measure pass: lane l owns pairs 8l .. 8l+7 of the round.  Pass 1 sums (saturating) the run ends
+            // from the last mask start in the slice; ONE segmented warp scan of these sums (segments = masks) gives
+            // every lane the end position before its first pair; pass 2 walks the slice again, forms the painter's
+            // records and keeps each mask's statistics in registers, which it adds to the mask once per slice.
+            const u32 f8 = lane * 8u;
+            const uint2 mm = *reinterpret_cast<const uint2 *>(&S.mid[f8]);     // masks of my 8 pairs, a byte each
+            const u32 mprev = __shfl_up_sync(0xffffffffu, mm.y >> 24, 1);
+            // bit k: a mask starts at my pair k (pair 0 of the round always starts one, so lane 0 heads every scan)
+            u32 hb;
+            {
+                const u32 dl = __vcmpne4(mm.x, (mm.x << 8) | mprev), dh = __vcmpne4(mm.y, __funnelshift_l(mm.x, mm.y, 8));
+                hb = ((dl & 0x01010101u) * 0x01020408u) >> 24 | ((dh & 0x01010101u) * 0x01020408u) >> 20 | (lane == 0u);
+            }
+            // my slice in 16-byte chunks, chunk q at q ^ sw (fl_swz)
+            uint4 *slice = reinterpret_cast<uint4 *>(S.pair) + 4u * lane;
+            const u32 sw = (lane >> 1) & 3u;
+            u32 sum = 0;                                  // run ends summed (saturating) from the last start
 #pragma unroll
-                for (u32 d = 1; d < 32; d <<= 1) {
-                    const u32 t = __shfl_up_sync(0xffffffffu, end, d);
-                    const u32 u = __shfl_up_sync(0xffffffffu, osum, d);
-                    if (d <= reach) { end = sat_add(end, t); osum += u; }
-                }
-                if (ok && p > lane) end = sat_add(end, carry);        // my mask began in an earlier pass
-                carry = __shfl_sync(0xffffffffu, end, 31);
-                const bool inb = ok && end <= HW;                      // HW < FL_SAT: nothing saturated up to here
-                const bool good = inb && o > 0u;
-                const u32 start = end - o;
-                uint2 pr = FL_EMPTY;
-                u32 ypk = 0xffffffffu;
-                if (good) {
-                    const u32 x = div_by(start, H, rcp);
-                    const u32 ys = start - x * H, yl = ys + o - 1u;
-                    // column-convex test (IV): a 1-run over several columns, or one whose 0-run starts in its own
-                    // column behind an earlier pair of the mask -- the 1-run before it ends in this column, or (a
-                    // zero-length 1-run in between; conservative) the gap only looks so -- makes the mask a bitmap
-                    if (IV && (yl >= H || (p > 0u && z < ys))) S.convex[j] = 0u;
-                    if (yl >= H) { pr = make_uint2(start | FL_SPAN, o); ypk = (0xffffu - (H - 1u)) << 16; }
-                    else { pr = make_uint2(x, ys | (yl << 16)); ypk = ys | ((0xffffu - yl) << 16); }
-                }
-                if (ok) S.pair[f] = pr;
+            for (int q = 0; q < 4; q++) {
+                const uint4 c = slice[q ^ sw];
+                sum = sat_add((hb >> (2 * q)) & 1u ? 0u : sum, sat_add(c.x, c.y));
+                sum = sat_add((hb >> (2 * q + 1)) & 1u ? 0u : sum, sat_add(c.z, c.w));
+            }
+            u32 sc = sum | (hb ? FL_HEAD : 0u);
+            // sat_add is associative on operands <= FL_SAT, so the scan saturates as the sequential walk does.  No
+            // lane test: lane 0 is flagged, so a lane below d has a flag by step d and takes nothing from above
 #pragma unroll
-                for (u32 d = 1; d < 32; d <<= 1) {
-                    const u32 t = __shfl_up_sync(0xffffffffu, ypk, d);
-                    if (d <= reach) ypk = __vminu2(ypk, t);
-                }
-                // my segment = lanes (lane - reach)..lane; in-frame lanes are a prefix of it (ends only grow)
-                const u32 seg = ((2u << lane) - 1u) & (0xffffffffu << (lane - reach));
-                const u32 gs = __ballot_sync(0xffffffffu, good) & seg, is = __ballot_sync(0xffffffffu, inb) & seg;
-                const u32 r_f = __shfl_sync(0xffffffffu, start, gs ? __ffs(gs) - 1 : (int)lane);
-                const u32 r_l = __shfl_sync(0xffffffffu, end, gs ? 31 - __clz(gs) : (int)lane);
-                const u32 r_a = __shfl_sync(0xffffffffu, osum, is ? 31 - __clz(is) : (int)lane);
-                if (ok && (f + 1u == nxt || lane == 31u)) {
-                    if (gs) {
-                        atomicAdd(&S.area[j], r_a);
-                        atomicMin(&S.first[j], r_f);
-                        atomicMax(&S.last[j], r_l);
+            for (u32 d = 1; d < 32; d <<= 1) {
+                const u32 t = __shfl_up_sync(0xffffffffu, sc, d);
+                if (!(sc & FL_HEAD)) sc = sat_add(t & FL_SAT, sc) | (t & FL_HEAD);
+            }
+            u32 e = __shfl_up_sync(0xffffffffu, sc, 1) & FL_SAT;    // end of the pair before my slice
+            if (f8 < T) {
+                u32 j = mm.x & 0xffu;
+                uint4 g = S.geo[a + j];                   // H, 2^32 / H, H * W
+                u32 ar = 0, fi = 0xffffffffu, la = 0, ypk = 0xffffffffu;   // area, first / last pixel, row range
+                auto flush = [&](bool ended) {
+                    if (fi != 0xffffffffu) {
+                        atomicAdd(&S.area[j], ar);
+                        atomicMin(&S.first[j], fi);
+                        atomicMax(&S.last[j], la);
                         atomicMin(&S.ymin[j], ypk & 0xffffu);
                         atomicMin(&S.ymaxi[j], ypk >> 16);
                     }
-                    if (f + 1u == nxt) S.total[j] = end;
+                    if (ended) S.total[j] = e;
+                };
+                auto step = [&](u32 k, u32 z, u32 o) {
+                    const bool h = (hb >> k) & 1u;
+                    if (k > 0u && h) {                    // the previous mask ended at pair k - 1
+                        flush(true);
+                        j = S.mid[f8 + k];
+                        g = S.geo[a + j];
+                        ar = 0u; fi = 0xffffffffu; la = 0u; ypk = 0xffffffffu;
+                    }
+                    e = sat_add(h ? 0u : e, sat_add(z, o));
+                    uint2 pr = FL_EMPTY;
+                    if (e <= g.z) {                       // H * W < FL_SAT: nothing saturated up to here
+                        ar += o;
+                        if (o > 0u) {
+                            const u32 H = g.x, start = e - o;
+                            const u32 x = div_by(start, H, g.y);
+                            const u32 ys = start - x * H, yl = ys + o - 1u;
+                            // column-convex test (IV): a 1-run over several columns, or one whose 0-run starts in its
+                            // own column behind an earlier pair of the mask -- the 1-run before it ends in this column,
+                            // or (a zero-length 1-run in between; conservative) the gap only looks so -- makes the
+                            // mask a bitmap
+                            if (IV && (yl >= H || (!h && z < ys))) S.convex[j] = 0u;
+                            fi = min(fi, start); la = e;
+                            if (yl >= H) { pr = make_uint2(start | FL_SPAN, o); ypk = __vminu2(ypk, (0xffffu - (H - 1u)) << 16); }
+                            else { pr = make_uint2(x, ys | (yl << 16)); ypk = __vminu2(ypk, ys | ((0xffffu - yl) << 16)); }
+                        }
+                    }
+                    return pr;
+                };
+                // the painter's records replace the staged pairs
+#pragma unroll 1
+                for (u32 q = 0; q < 4u; q++) {
+                    const uint4 c = slice[q ^ sw];
+                    const uint2 r0 = step(2u * q, c.x, c.y), r1 = step(2u * q + 1u, c.z, c.w);
+                    slice[q ^ sw] = make_uint4(r0.x, r0.y, r1.x, r1.y);
                 }
+                flush(f8 + 8u >= T || S.mid[f8 + 8u] != j);
             }
             __syncwarp();
 
@@ -314,7 +359,7 @@ rle_flat_crop_kernel(const u32 *__restrict__ cnt, const i64 *__restrict__ cnt_of
                     // every 1-run lies inside its mask's box: the box was formed from the same runs
                     const u32 f_end = S.pb[last - a + 1];
                     for (u32 f = S.pb[lo - a] + lane; f < f_end; f += 32) {
-                        const uint2 pr = S.pair[f];
+                        const uint2 pr = S.pair[fl_swz(f)];
                         if (!(pr.x & FL_SPAN)) {
                             const u32 ys = pr.y & 0xffffu, yl = pr.y >> 16;
                             if (ys > yl) continue;
