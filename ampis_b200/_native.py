@@ -59,6 +59,8 @@ SIGNATURES = {
                                          _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p]),
     'ampis_eval_images_sweep_host': (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _i32, _p, _i32, _p, _i32, _p, _i64, _p,
                                                _i64, _p, _p, _p, _p, _p, _p, _p, _p]),
+    'ampis_eval_images_sat_sweep_host': (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _i32, _p, _i32, _p, _i32, _p, _i32,
+                                                   _i32, _p, _i64, _p, _i64, _p, _p, _p, _p, _p, _p, _p]),
     'ampis_mma_pair_tile_rows': (C.c_int, []),
     'ampis_mma_pair_tile_cols': (C.c_int, []),
     'ampis_intersect_tcgen05_pair': (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i32, _p, _p, _p, _p, _p, _p,

@@ -339,6 +339,26 @@ def _score_levels(scores, sorted_th):
     return lv.astype(np.uint16)
 
 
+def _image_levels(sc, sorted_th):
+    """Levels of the per-image score arrays sc (concatenated, uint16) and the kept counts int64 [n, K] (instances whose
+    level exceeds k), one numpy pass per score dtype."""
+    n, K = len(sc), len(sorted_th)
+    lens = np.fromiter(map(len, sc), np.int64, n)
+    dtypes = [s.dtype for s in sc]
+    kinds = sorted(set(dtypes), key=str)
+    if len(kinds) <= 1:
+        levels = _score_levels(np.concatenate(sc) if n else np.zeros(0), sorted_th)
+    else:
+        levels = np.zeros(int(lens.sum()), np.uint16)
+        code = np.asarray([kinds.index(d) for d in dtypes])
+        for c, dt in enumerate(kinds):
+            levels[np.repeat(code == c, lens)] = _score_levels(np.concatenate([s for s in sc if s.dtype == dt]), sorted_th)
+    img = np.repeat(np.arange(n), lens)
+    hist = np.bincount(img * (K + 1) + levels, minlength=n * (K + 1)).reshape(n, K + 1)
+    kept = np.cumsum(hist[:, ::-1], axis=1)[:, ::-1][:, 1:]                 # [n, K]: sum over levels > k
+    return levels, kept
+
+
 def _image_scores(p):
     inst = p if type(p) == Instances else p.instances if type(p) == InstanceSet else None
     if inst is None or getattr(inst, 'scores', None) is None:
@@ -390,22 +410,8 @@ def det_seg_scores_sweep(gt_list, pred_list, score_thresholds, iou_thresholds=No
         if len(s) != len(p):
             raise ValueError('image %d: %d scores for %d predictions' % (i, len(s), len(p)))
     n, K, T = len(gts), len(s_th), len(i_th)
-    # levels, one numpy pass per score dtype
-    lens = np.fromiter(map(len, sc), np.int64, n)
-    dtypes = [s.dtype for s in sc]
-    kinds = sorted(set(dtypes), key=str)
-    if len(kinds) <= 1:
-        levels = _score_levels(np.concatenate(sc) if n else np.zeros(0), s_sorted)
-    else:
-        levels = np.zeros(int(lens.sum()), np.uint16)
-        code = np.asarray([kinds.index(d) for d in dtypes])
-        for c, dt in enumerate(kinds):
-            levels[np.repeat(code == c, lens)] = _score_levels(np.concatenate([s for s in sc if s.dtype == dt]), s_sorted)
+    levels, kept = _image_levels(sc, s_sorted)
     r = engine.eval_images_sweep(gts, prs, levels, K, i_sorted)
-    # kept predictions per image and sorted level: predictions whose level exceeds k
-    img = np.repeat(np.arange(n), lens)
-    hist = np.bincount(img * (K + 1) + levels, minlength=n * (K + 1)).reshape(n, K + 1)
-    kept = np.cumsum(hist[:, ::-1], axis=1)[:, ::-1][:, 1:]                 # [n, K]: sum over levels > k
     # back to the caller's order of thresholds
     order = lambda a, ks: _reorder(_reorder(a, s_pos, ks), i_pos, ks + 1)
     totals, seg_totals = order(r.totals, 0), order(r.seg_totals, 0)

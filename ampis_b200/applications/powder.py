@@ -239,3 +239,132 @@ def satellite_measurements(psi, print_summary=True, output_dict=False):
         _print_summary(out)
     if output_dict:
         return out
+
+
+#: limits of the satellite sweep's grid (include/ampis_b200.h): K x L x T x B histogram cells, and (L + 1) x (T + 1),
+#: the per-cell tables the count kernel keeps in shared memory
+SAT_SWEEP_MAX_HIST = 1 << 26
+SAT_SWEEP_MAX_LT = 4096
+SAT_SWEEP_MAX_PARTICLES = 32768
+
+
+def _sweep_side(thresholds, scores, instances, counts, what):
+    """One score axis of the satellite sweep: (thresholds as given or None, position of each in sorted order, level of
+    every instance in image order, kept instances int64 [n, K]).  None keeps every instance: one level, no scores."""
+    n = len(counts)
+    if thresholds is None:
+        return None, np.zeros(1, np.int64), np.ones(int(sum(counts)), np.uint16), \
+            np.asarray(counts, np.int64).reshape(n, 1)
+    th = np.asarray(thresholds, np.float64).reshape(-1)
+    sorted_th, pos = analyze._sorted_thresholds(th, what + '_score_thresholds')
+    if len(th) > 65535:
+        raise ValueError('at most 65,535 %s score thresholds' % what)
+    if scores is None:
+        scores = [getattr(inst, 'scores', None) if hasattr(inst, 'has') and inst.has('scores') else None
+                  for inst in instances]
+        if any(s is None for s in scores):
+            raise ValueError('%s scores are needed: pass %s_scores or instances with scores' % (what, what))
+    if len(scores) != n:
+        raise ValueError('%d %s score arrays for %d images' % (len(scores), what, n))
+    sc = [analyze._score_array(s) for s in scores]
+    for i, (s, c) in enumerate(zip(sc, counts)):
+        if len(s) != c:
+            raise ValueError('image %d: %d %s scores for %d %ss' % (i, len(s), what, c, what))
+    levels, kept = analyze._image_levels(sc, sorted_th)
+    return th, pos, levels, kept
+
+
+def _sweep_summary(n_images, n_particles, n_satellite_instances, totals, spp_hist):
+    """The dataset keys of satellite_measurements_sweep from its sum-reducible parts: kept particles [K], kept
+    satellites [L], totals [K, L, T, 3] and the satellites-per-particle histogram [K, L, T, B].  sat_frac is NaN where
+    no particle is kept, mspp (the median of the histogram, as np.median forms it) where none is satellited."""
+    satp = totals[..., 2]
+    with np.errstate(invalid='ignore', divide='ignore'):
+        sat_frac = satp / n_particles.astype(np.float64)[:, None, None]
+    cum = np.cumsum(spp_hist, axis=-1)
+    lo = ((cum <= ((satp - 1) // 2)[..., None]).sum(axis=-1)).astype(np.float64)
+    hi = ((cum <= (satp // 2)[..., None]).sum(axis=-1)).astype(np.float64)
+    mspp = np.where(satp > 0, (lo + hi) / 2, np.nan)
+    return {'n_images': n_images, 'n_particles': n_particles, 'n_satellite_instances': n_satellite_instances,
+            'n_satellites': totals[..., 0], 'n_satellites_unmatched': totals[..., 1], 'n_satellited_particels': satp,
+            'sat_frac': sat_frac, 'mspp': mspp, 'spp_hist': spp_hist}
+
+
+def _sweep_bins(images):
+    """Histogram bins of a sweep over these images: 1 + the most satellites of any image (no particle owns more)."""
+    return 1 + max([len(im.satellites.instances) for im in images], default=0)
+
+
+def satellite_measurements_sweep(psi, particle_score_thresholds=None, satellite_score_thresholds=None,
+                                 match_thresholds=(0.5,), particle_scores=None, satellite_scores=None, _n_bins=None):
+    """Satellite statistics of a set of images over a grid of particle-score x satellite-score x match thresholds,
+    from one evaluation.  Cell (k, l, t) of image i is ``_rle_satellite_match(particles_i[ps_i > P_k],
+    satellites_i[ss_i > S_l], match_thresh=T_t)`` reduced to counts (numpy's comparison on the caller's scores: NaN is
+    never kept); the dataset cell is ``satellite_measurements(filtered psi, output_dict=True)`` after
+    ``compute_matches(T_t)``.  Where the reference raises (nothing matched in an image, satellites without particles,
+    no particle at all) the counts are returned instead: sat_frac is NaN when no particle is kept, mspp when none is
+    satellited, and the unique / cumulative arrays of satellite_measurements_at are empty.
+
+    psi: a PowderSatelliteImage or a list of them.  A threshold vector of None keeps every instance of that side (the
+    axis has length 1 and needs no scores: ground-truth sets).  Scores default to ``instances.scores``;
+    particle_scores / satellite_scores (one float16/32/64 numpy or torch array per image) override them.  Thresholds
+    may come in any order and repeat; results come back in the caller's order.  match_thresholds must be >= 0.
+
+    Returns a dict: the three threshold vectors as given (float64, None stays None), ``n_images``, ``n_particles``
+    int64 [K] and ``n_satellite_instances`` int64 [L] (kept), ``n_satellites`` / ``n_satellites_unmatched`` /
+    ``n_satellited_particels`` int64 [K, L, T], ``sat_frac`` / ``mspp`` float64 [K, L, T], ``spp_hist`` int64
+    [K, L, T, B] (bin b >= 1: particles owning exactly b satellites; B = 1 + the most satellites of any image),
+    ``image_counts`` int64 [n, K, L, T, 3] (matched, unmatched, satellited particles per image), ``image_particles``
+    int64 [n, K] and ``image_satellites`` int64 [n, L].  Read one cell with satellite_measurements_at.  One library
+    call (engine.eval_images_sat_sweep).  _n_bins (internal): B of the whole dataset when psi is one shard of it."""
+    images = [psi] if type(psi) == PowderSatelliteImage else list(psi)
+    assert all(type(im) == PowderSatelliteImage for im in images), 'psi must be list of PowderSatelliteImage objects!'
+    n = len(images)
+    m_th = np.asarray(match_thresholds, np.float64).reshape(-1)
+    m_sorted, m_pos = analyze._sorted_thresholds(m_th, 'match_thresholds')
+    if m_sorted[0] < 0:
+        raise ValueError('match_thresholds must not be negative')
+    if len(m_th) > 256:
+        raise ValueError('at most 256 match thresholds')
+    parts = [masks_to_rle(im.particles.instances) for im in images]
+    sats = [masks_to_rle(im.satellites.instances) for im in images]
+    n_part, n_sat = [len(p) for p in parts], [len(s) for s in sats]
+    if n and max(n_part) > SAT_SWEEP_MAX_PARTICLES:
+        raise ValueError('more than %d particles in one image' % SAT_SWEEP_MAX_PARTICLES)
+    p_th, p_pos, plevels, p_kept = _sweep_side(particle_score_thresholds, particle_scores,
+                                               [im.particles.instances for im in images], n_part, 'particle')
+    s_th, s_pos, slevels, s_kept = _sweep_side(satellite_score_thresholds, satellite_scores,
+                                               [im.satellites.instances for im in images], n_sat, 'satellite')
+    K, L, T = len(p_pos), len(s_pos), len(m_th)
+    B = 1 + max(n_sat, default=0) if _n_bins is None else int(_n_bins)
+    if K * L * T * B > SAT_SWEEP_MAX_HIST or (L + 1) * (T + 1) > SAT_SWEEP_MAX_LT:
+        raise ValueError('satellite sweep grid too large: K x L x T x B = %d x %d x %d x %d (at most 2^26 cells) and '
+                         '(L + 1) x (T + 1) = %d (at most %d)' % (K, L, T, B, (L + 1) * (T + 1), SAT_SWEEP_MAX_LT))
+    r = engine.eval_images_sat_sweep(sats, parts, plevels, K, slevels, L, m_sorted, B)
+    # back to the caller's order of thresholds
+    order = lambda a, ax: analyze._reorder(analyze._reorder(analyze._reorder(a, p_pos, ax), s_pos, ax + 1), m_pos, ax + 2)
+    n_particles = analyze._reorder(p_kept.sum(axis=0), p_pos, 0)
+    n_satellite_instances = analyze._reorder(s_kept.sum(axis=0), s_pos, 0)
+    out = {'particle_score_thresholds': p_th, 'satellite_score_thresholds': s_th, 'match_thresholds': m_th}
+    out.update(_sweep_summary(n, n_particles, n_satellite_instances, order(r.totals, 0), order(r.spp_hist, 0)))
+    out['image_counts'] = order(r.counts, 1).astype(np.int64)
+    out['image_particles'] = analyze._reorder(p_kept, p_pos, 1)
+    out['image_satellites'] = analyze._reorder(s_kept, s_pos, 1)
+    return out
+
+
+def satellite_measurements_at(result, k, l, t):
+    """Cell (k, l, t) of a satellite_measurements_sweep result as the dict of satellite_measurements(output_dict=True):
+    the counts, sat_frac and mspp of the cell, and the unique / cumulative satellites-per-particle arrays formed from
+    its spp_hist row."""
+    h = np.asarray(result['spp_hist'][k, l, t])
+    values = np.flatnonzero(h).astype(np.int64)
+    freq = h[values]
+    with np.errstate(invalid='ignore', divide='ignore'):
+        cum = freq.cumsum() / freq.sum()
+    return {'n_images': result['n_images'], 'n_particles': int(result['n_particles'][k]),
+            'n_satellites': int(result['n_satellites'][k, l, t]),
+            'n_satellites_unmatched': int(result['n_satellites_unmatched'][k, l, t]),
+            'n_satellited_particels': int(result['n_satellited_particels'][k, l, t]),
+            'sat_frac': float(result['sat_frac'][k, l, t]), 'mspp': np.float64(result['mspp'][k, l, t]),
+            'unique_satellites_per_particle': values, 'counts_satellites_per_particle': cum}

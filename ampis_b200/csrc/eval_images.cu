@@ -147,13 +147,13 @@ struct ImagesIn {
     void *stream;
 };
 
-// The caller's own parts of the workspaces: up to two host arrays uploaded with the strings, a block downloaded with
+// The caller's own parts of the workspaces: up to three host arrays uploaded with the strings, a block downloaded with
 // the counters, and device-only space.  images_front places them and returns their offsets.
 struct ImagesExtra {
-    const void *up[2] = {nullptr, nullptr};
-    int64_t up_bytes[2] = {0, 0};
+    const void *up[3] = {nullptr, nullptr, nullptr};
+    int64_t up_bytes[3] = {0, 0, 0};
     int64_t dl_bytes = 0, dev_bytes = 0;
-    int64_t up_off[2] = {0, 0}, dl_off = 0, dev_off = 0;
+    int64_t up_off[3] = {0, 0, 0}, dl_off = 0, dev_off = 0;
 };
 
 // Where everything lies after images_front (offsets into both workspaces), and the sizes of the call
@@ -224,7 +224,7 @@ static int images_front(const ImagesIn &in, ImagesExtra &x, double crowd_frac, I
     const int64_t u_rowmask = on_device ? 0 : c.take(4 * R), u_rowgrp = on_device ? 0 : c.take(4 * R);
     const int64_t u_grb = on_device ? 0 : c.take(4 * NI), u_grc = on_device ? 0 : c.take(4 * NI),
                   u_gcb = on_device ? 0 : c.take(4 * NI), u_gcc = on_device ? 0 : c.take(4 * NI);
-    for (int k = 0; k < 2; k++) x.up_off[k] = c.take(x.up_bytes[k]);
+    for (int k = 0; k < 3; k++) x.up_off[k] = c.take(x.up_bytes[k]);
     const int64_t i_nr = on_device ? c.take(4 * NI) : 0, i_nc = on_device ? c.take(4 * NI) : 0,
                   i_h = on_device ? c.take(4 * NI) : 0, i_w = on_device ? c.take(4 * NI) : 0,
                   i_moff = on_device ? c.take(8 * NI) : 0, i_roff = on_device ? c.take(8 * NI) : 0;
@@ -293,7 +293,7 @@ static int images_front(const ImagesIn &in, ImagesExtra &x, double crowd_frac, I
     r.grid_base = grid_base; r.grid_cap = grid_cap; r.arena_chunks = arena_chunks;
 
     // ---- fill the upload block ------------------------------------------------------------------------------------
-    for (int k = 0; k < 2; k++)
+    for (int k = 0; k < 3; k++)
         if (x.up_bytes[k]) memcpy(H + x.up_off[k], x.up[k], (size_t)x.up_bytes[k]);
     if (on_device) {
         if (!len_direct) memcpy(H + u_len, str_len, (size_t)(4 * n));
@@ -602,5 +602,106 @@ extern "C" int ampis_eval_images_sweep_host(const uint8_t *const *str_ptr, const
     if (e != cudaSuccess) { ampis_set_error("download: %s", cudaGetErrorString(e)); return AMPIS_ECUDA; }
     memcpy(totals, H + o_totals, (size_t)(8 * KT3));
     memcpy(seg_totals, H + o_segtot, (size_t)(8 * KT3));
+    return AMPIS_OK;
+}
+
+int ampis_sweep_chunks(int32_t n_levels, int32_t n_groups);
+int ampis_sat_sweep_counts(const uint32_t *d_area, const int32_t *d_row_mask, const int32_t *d_row_grp,
+                           int32_t n_rows, const int32_t *d_grp_row_begin, const int32_t *d_grp_row_count,
+                           const int32_t *d_grp_col_begin, const int32_t *d_grp_col_count, int32_t n_groups,
+                           int32_t max_cols, const int32_t *d_pair_ab, const uint32_t *d_pair_inter,
+                           const int64_t *d_row_pair_off, const int32_t *d_row_pair_cnt, const uint16_t *d_plevels,
+                           int32_t n_plevels, const uint16_t *d_slevels, int32_t n_slevels,
+                           const double *d_match_thresh, int32_t n_match, int32_t n_bins, int32_t chunks,
+                           void *d_stair, void *d_node, int32_t *d_claimed, int32_t *d_counts, int64_t *d_totals,
+                           int64_t *d_spp_hist, void *stream);
+
+extern "C" int ampis_eval_images_sat_sweep_host(const uint8_t *const *str_ptr, const int32_t *str_len,
+                                                int32_t n_images, const int32_t *n_rows, const int32_t *n_cols,
+                                                const uint32_t *h, const uint32_t *w, int32_t flags,
+                                                const uint16_t *plevels, int32_t n_plevels, const uint16_t *slevels,
+                                                int32_t n_slevels, const double *match_thresh, int32_t n_match,
+                                                int32_t n_bins, void *d_ws, int64_t d_ws_bytes, void *h_ws,
+                                                int64_t h_ws_bytes, int32_t *status, int64_t *totals,
+                                                int64_t *spp_hist, int32_t *counts, int64_t *pairs_found,
+                                                int64_t *need_bytes, void *stream)
+{
+    AMPIS_REQUIRE(n_images >= 0, "negative size");
+    AMPIS_REQUIRE(n_plevels >= 1 && n_plevels <= 65535, "the number of particle score levels must be in [1, 65535]");
+    AMPIS_REQUIRE(n_slevels >= 1 && n_slevels <= 65535, "the number of satellite score levels must be in [1, 65535]");
+    AMPIS_REQUIRE(n_match >= 1 && n_match <= AMPIS_SWEEP_MAX_IOU, "the number of match thresholds must be in [1, 256]");
+    AMPIS_REQUIRE(n_bins >= 1, "n_bins must be at least 1");
+    const int64_t KLT = (int64_t)n_plevels * n_slevels * n_match, NI = n_images;
+    AMPIS_REQUIRE(KLT * n_bins <= AMPIS_SAT_SWEEP_MAX_HIST, "more than 2^26 histogram cells (K x L x T x n_bins)");
+    AMPIS_REQUIRE(((int64_t)n_slevels + 1) * (n_match + 1) <= AMPIS_SAT_SWEEP_MAX_LT,
+                  "(satellite levels + 1) x (match thresholds + 1) above 4096");
+    AMPIS_REQUIRE(d_ws && h_ws && need_bytes && pairs_found && totals && spp_hist && match_thresh, "null pointer");
+    AMPIS_REQUIRE(((uintptr_t)d_ws & 255u) == 0, "device workspace must be 256-byte aligned");
+    for (int32_t j = 0; j < n_match; j++)
+        AMPIS_REQUIRE(match_thresh[j] >= 0.0 && (j == 0 || match_thresh[j] >= match_thresh[j - 1]),
+                      "match thresholds must be sorted ascending and not negative or NaN");
+    *pairs_found = 0;
+    for (int64_t t = 0; t < 3 * KLT; t++) totals[t] = 0;
+    for (int64_t t = 0; t < KLT * n_bins; t++) spp_hist[t] = 0;
+    if (n_images == 0) return AMPIS_OK;
+    AMPIS_REQUIRE(n_rows && n_cols, "null pointer");
+    int64_t n_part = 0, n_sat = 0;
+    for (int32_t g = 0; g < n_images; g++) {
+        AMPIS_REQUIRE(n_cols[g] <= AMPIS_SWEEP_MAX_PREDS, "more than 32768 particles in one image");
+        AMPIS_REQUIRE(n_rows[g] < n_bins, "n_bins must exceed the number of satellites of every image");
+        n_part += n_cols[g] > 0 ? n_cols[g] : 0;
+        n_sat += n_rows[g] > 0 ? n_rows[g] : 0;
+    }
+    AMPIS_REQUIRE((plevels || n_part == 0) && (slevels || n_sat == 0), "null pointer");
+    for (int64_t p = 0; p < n_part; p++) AMPIS_REQUIRE(plevels[p] <= n_plevels, "particle level above n_plevels");
+    for (int64_t p = 0; p < n_sat; p++) AMPIS_REQUIRE(slevels[p] <= n_slevels, "satellite level above n_slevels");
+    if (counts) for (int64_t t = 0; t < 3 * KLT * NI; t++) counts[t] = 0;
+    const int32_t chunks = ampis_sweep_chunks(n_plevels, n_images);
+    if (chunks <= 0) { ampis_set_error("no CUDA device"); return AMPIS_ECUDA; }
+    const ImagesIn in{str_ptr, str_len, n_images, n_rows, n_cols, h, w, AMPIS_MODE_SAT, flags, d_ws, d_ws_bytes, h_ws,
+                      h_ws_bytes, false, nullptr, nullptr, nullptr, nullptr, nullptr, status, nullptr, need_bytes, stream};
+    ImagesExtra x;
+    x.up[0] = match_thresh;
+    x.up_bytes[0] = 8 * (int64_t)n_match;
+    x.up[1] = plevels;
+    x.up_bytes[1] = 2 * n_part;
+    x.up[2] = slevels;
+    x.up_bytes[2] = 2 * n_sat;
+    // device only: totals, the histogram, the per-image counts and the per-(image, chunk) particle lists
+    const int64_t tot_bytes = al256(24 * KLT), hist_bytes = al256(8 * KLT * n_bins),
+                  counts_bytes = counts ? al256(12 * KLT * NI) : 0, node_bytes = al256(8 * n_sat * chunks);
+    x.dev_bytes = tot_bytes + hist_bytes + counts_bytes + node_bytes + 4 * n_sat * chunks;
+    ImagesRun r;
+    int rc = images_front(in, x, -1.0, r);
+    if (rc != AMPIS_OK || r.n == 0) return rc;
+    uint8_t *D = r.D;
+    const int64_t d_tot = x.dev_off, d_hist = d_tot + tot_bytes, d_counts = d_hist + hist_bytes,
+                  d_node = d_counts + counts_bytes, d_claimed = d_node + node_bytes;
+    cudaError_t e = cudaMemsetAsync(D + d_tot, 0, (size_t)(tot_bytes + hist_bytes), r.st);
+    // rows without candidate pairs: when the join did not run, no row has any
+    if (e == cudaSuccess && !r.have_rows && r.R > 0) e = cudaMemsetAsync(D + r.p_cnt, 0, (size_t)(4 * r.R), r.st);
+    if (e != cudaSuccess) { ampis_set_error("memset: %s", cudaGetErrorString(e)); return AMPIS_ECUDA; }
+    rc = ampis_sat_sweep_counts((const uint32_t *)(D + r.o_area), (const int32_t *)(D + r.x_rowmask),
+                                (const int32_t *)(D + r.x_rowgrp), r.have_rows ? (int32_t)r.R : 0,
+                                (const int32_t *)(D + r.x_grb), (const int32_t *)(D + r.x_grc),
+                                (const int32_t *)(D + r.x_gcb), (const int32_t *)(D + r.x_gcc), n_images, r.max_cols,
+                                (const int32_t *)(D + r.p_ab), (const uint32_t *)(D + r.p_inter),
+                                (const int64_t *)(D + r.p_off), (const int32_t *)(D + r.p_cnt),
+                                (const uint16_t *)(D + x.up_off[1]), n_plevels, (const uint16_t *)(D + x.up_off[2]),
+                                n_slevels, (const double *)(D + x.up_off[0]), n_match, n_bins, chunks, D + r.p_desc,
+                                D + d_node, (int32_t *)(D + d_claimed), counts ? (int32_t *)(D + d_counts) : nullptr,
+                                (int64_t *)(D + d_tot), (int64_t *)(D + d_hist), stream);
+    if (rc != AMPIS_OK) return rc;
+    int32_t crowded = 0;
+    rc = images_back(in, r, pairs_found, &crowded);
+    if (rc != AMPIS_OK) return rc;
+    // the outputs go straight into the caller's arrays once everything is known to have fit (pageable destinations
+    // make these copies blocking)
+    e = cudaMemcpyAsync(totals, D + d_tot, (size_t)(24 * KLT), cudaMemcpyDeviceToHost, r.st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(spp_hist, D + d_hist, (size_t)(8 * KLT * n_bins), cudaMemcpyDeviceToHost, r.st);
+    if (e == cudaSuccess && counts)
+        e = cudaMemcpyAsync(counts, D + d_counts, (size_t)(12 * KLT * NI), cudaMemcpyDeviceToHost, r.st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(r.st);
+    if (e != cudaSuccess) { ampis_set_error("download: %s", cudaGetErrorString(e)); return AMPIS_ECUDA; }
     return AMPIS_OK;
 }

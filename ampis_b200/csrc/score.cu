@@ -89,6 +89,12 @@ extern "C" int ampis_match_counts(const int32_t *d_best_col, const double *d_bes
 // Each entry costs one walk over the row's pairs, so a row costs cnt x S pair visits with S <= min(cnt, K) entries.
 // Rows have a few pairs; S stays small when scores rise with IoU, and only reaches cnt when every higher-scored
 // prediction of the row overlaps it less -- on a crowded frame with many score levels that is quadratic in cnt.
+// MODE = AMPIS_MODE_SAT (rows = satellites, columns = particles, the satellite sweep): pairs rank by intersection,
+// the first index winning ties -- the reference's arg-max of I / area(s), which for a fixed satellite is monotone in I
+// (distinct integers give distinct quotients) -- and the entry's second level counts the match thresholds strictly
+// below (double)I / (double)area(s); its last word is 0.  Zero-area satellites intersect nothing: no entry, never
+// matched (the reference's NaN row).
+template <int MODE>
 __global__ void __launch_bounds__(128)
 sweep_rows_kernel(const u32 *__restrict__ area, const int *__restrict__ row_mask, const int *__restrict__ row_grp,
                   int n_rows, const int *__restrict__ grp_row_begin, const int *__restrict__ grp_row_count,
@@ -118,11 +124,12 @@ sweep_rows_kernel(const u32 *__restrict__ area, const int *__restrict__ row_mask
             const int k = cm - cb;
             const u32 lv = __ldg(levels + pred0 + k);
             if (lv <= lo) continue;
-            const u32 ca = __ldg(area + cm);
-            const double s = pair_iou(inter, ra, ca);
+            const u32 ca = MODE == AMPIS_MODE_IOU ? __ldg(area + cm) : 0u;
+            const double s = MODE == AMPIS_MODE_IOU ? pair_iou(inter, ra, ca) : (double)inter;
             if (score_beats(s, k, best_s, best_c)) { best_s = s; best_c = k; best_i = inter; best_a = ca; best_lv = lv; }
         }
         if (best_c < 0) break;
+        if (MODE == AMPIS_MODE_SAT) best_s = (double)best_i / (double)ra;
         u32 il = 0;
         for (int j = 0; j < n_iou; j++) il += __ldg(iou_thresh + j) < best_s;
         stair[first + out++] = make_uint4(best_lv | (il << 16), (u32)best_c, best_i, best_a);
@@ -251,6 +258,17 @@ sweep_counts_kernel(const uint4 *__restrict__ stair, const i64 *__restrict__ row
     }
 }
 
+// Score-level chunks of the sweep count kernels: enough CTAs (images x chunks) for a few per SM, so small batches split
+// the levels into chunks (each re-reads its staircases).  0 when the device cannot be queried.
+int ampis_sweep_chunks(int32_t n_levels, int32_t n_groups)
+{
+    const int sms = ampis_sm_count();
+    if (sms <= 0 || n_groups <= 0) return 0;
+    const int chunks = (int)std::min<int64_t>(n_levels, std::max<int64_t>(1, (8 * (int64_t)sms + n_groups - 1) / n_groups));
+    const int per = (n_levels + chunks - 1) / chunks;
+    return (n_levels + per - 1) / per;
+}
+
 // (not part of the C ABI: the step of ampis_eval_images_sweep_host after the join)
 int ampis_sweep_counts(const uint32_t *d_area, const int32_t *d_row_mask, const int32_t *d_row_grp,
                                   int32_t n_rows, const int32_t *d_grp_row_begin, const int32_t *d_grp_row_count,
@@ -267,7 +285,7 @@ int ampis_sweep_counts(const uint32_t *d_area, const int32_t *d_row_mask, const 
     if (n_groups == 0) return AMPIS_OK;
     cudaStream_t st = as_stream(stream);
     if (n_rows > 0) {
-        sweep_rows_kernel<<<(unsigned)((n_rows + 127) / 128), 128, 0, st>>>(
+        sweep_rows_kernel<AMPIS_MODE_IOU><<<(unsigned)((n_rows + 127) / 128), 128, 0, st>>>(
             d_area, d_row_mask, d_row_grp, n_rows, d_grp_row_begin, d_grp_row_count, d_grp_col_begin,
             (const int2 *)d_pair_ab, d_pair_inter, d_row_pair_off, d_row_pair_cnt, (const unsigned short *)d_levels,
             d_iou_thresh, n_iou, (uint4 *)d_stair);
@@ -282,17 +300,212 @@ int ampis_sweep_counts(const uint32_t *d_area, const int32_t *d_row_mask, const 
             return AMPIS_ECUDA;
         }
     }
-    // enough CTAs for a few per SM: small batches split the score levels into chunks (each re-reads its staircases)
-    const int sms = ampis_sm_count();
-    if (sms <= 0) return AMPIS_ECUDA;
-    int chunks = (int)std::min<int64_t>(n_levels, std::max<int64_t>(1, (8 * (int64_t)sms + n_groups - 1) / n_groups));
+    const int chunks = ampis_sweep_chunks(n_levels, n_groups);
+    if (chunks <= 0) return AMPIS_ECUDA;
     const int per = (n_levels + chunks - 1) / chunks;
-    chunks = (n_levels + per - 1) / per;
     sweep_counts_kernel<<<dim3((unsigned)n_groups, (unsigned)chunks), 256, smem, st>>>(
         (const uint4 *)d_stair, d_row_pair_off, d_row_pair_cnt, d_area, d_row_mask, d_grp_row_begin, d_grp_row_count,
         d_grp_col_begin, d_grp_col_count, (const unsigned short *)d_levels, n_levels, n_iou, per, d_counts,
         (long long *)d_seg, (unsigned long long *)d_totals, (unsigned long long *)d_seg_totals);
     AMPIS_CHECK_LAUNCH("sweep_counts_kernel");
+    return AMPIS_OK;
+}
+
+// ---- satellite sweep ------------------------------------------------------------------------------------------------
+// Rows are satellites, columns particles.  A particle's level (plevels, K of them) drives the staircase as above; a
+// satellite's own level sigma (slevels, L) only removes its row: it is kept at sorted satellite threshold l iff
+// sigma > l.  A row's active entry at particle level k is (particle p, match level m): it is matched at (l, t) iff
+// sigma > l and m > t.
+//
+// sat_sweep_counts_kernel, one CTA per (image, chunk of particle levels).  Per level k:
+//  - every row takes its active entry; a matched row (sigma, m >= 1) is added to a shared (sigma, m) histogram and
+//    pushed onto its particle's list (a shared head per particle, the links in `node`); the first row of a particle
+//    appends it to the claimed list;
+//  - 2-D suffix sums of the histogram give the matched rows of every (l, t); unmatched = kept satellites - matched;
+//  - one warp per claimed particle, lanes over the cells (l < its largest sigma, t < its largest m), walks the
+//    particle's list for its count c at the cell; c >= 1 counts a satellited particle and goes into bin c of the
+//    cell's histogram: shared for c <= cs (cs = min(n_bins - 1, 32) as far as shared memory allows), a global atomic
+//    above that (a particle owning more than cs satellites);
+//  - per cell: the per-image counts, atomics into the totals and the non-zero shared bins into spp_hist.
+// Cost per level and image: the rows' staircase walks, O(L * T) for the suffix sums and the output, and
+// O(sum over claimed particles of satellites x cells below its largest (sigma, m)) <= O(matched rows x L x T) for the
+// per-particle counts.  node / claimed: one slice per (image, chunk), rows of the image long.
+__global__ void __launch_bounds__(256)
+sat_sweep_counts_kernel(const uint4 *__restrict__ stair, const i64 *__restrict__ row_pair_off,
+                        const int *__restrict__ row_pair_cnt, const int *__restrict__ grp_row_begin,
+                        const int *__restrict__ grp_row_count, const int *__restrict__ grp_col_count,
+                        const unsigned short *__restrict__ slevels, int n_plevels, int n_slevels, int n_match,
+                        int levels_per_cta, int n_bins, int cs, uint2 *__restrict__ node, int *__restrict__ claimed,
+                        int *__restrict__ counts, unsigned long long *__restrict__ totals,
+                        unsigned long long *__restrict__ spp_hist)
+{
+    extern __shared__ u32 ss_smem[];
+    const int L = n_slevels, T = n_match, LT = L * T, W = T + 1;
+    const int g = blockIdx.x;
+    const int r0 = grp_row_begin[g], S = grp_row_count[g], P = grp_col_count[g];
+    int *head = (int *)ss_smem;                                       // [P] last row pushed per particle, -1: none
+    u32 *kept = (u32 *)(head + P);                                    // [L + 1] satellites by level, then suffix sums
+    u32 *h2 = kept + L + 1;                                           // [1 + (L + 1) * W] bin 1 + sigma * W + m
+    u32 *sp = h2 + 1 + (L + 1) * W;                                   // [L * T] satellited particles per cell
+    u32 *hist = sp + LT;                                              // [L * T * cs] particles owning c = 1 .. cs
+    int *s_nq = (int *)(hist + (i64)LT * cs);
+    const int chunk = blockIdx.y, k0 = chunk * levels_per_cta, k1 = min(n_plevels, k0 + levels_per_cta);
+    const i64 slice = (i64)gridDim.y * r0 + (i64)chunk * S;
+    uint2 *nd = node + slice;
+    int *cl = claimed + slice;
+    for (int i = threadIdx.x; i < P; i += blockDim.x) head[i] = -1;
+    for (int i = threadIdx.x; i < L + 1; i += blockDim.x) kept[i] = 0u;
+    for (int i = threadIdx.x; i < 1 + (L + 1) * W; i += blockDim.x) h2[i] = 0u;
+    for (int i = threadIdx.x; i < LT; i += blockDim.x) sp[i] = 0u;
+    for (i64 i = threadIdx.x; i < (i64)LT * cs; i += blockDim.x) hist[i] = 0u;
+    if (threadIdx.x == 0) *s_nq = 0;
+    __syncthreads();
+    const int S32 = (S + 31) & ~31;
+    for (int i = threadIdx.x; i < S32; i += blockDim.x)
+        sweep_bin_add(i < S ? (u32)slevels[r0 + i] : 0u, 0u, 0u, 0u, kept, nullptr, nullptr, nullptr);
+    __syncthreads();
+    if (threadIdx.x == 0)
+        for (int l = L - 1; l >= 1; l--) kept[l] += kept[l + 1];      // kept[l + 1]: satellites kept at l
+    __syncthreads();
+    const int lane = (int)lane_id(), warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
+    for (int k = k0; k < k1; k++) {
+        for (int i = threadIdx.x; i < S32; i += blockDim.x) {
+            u32 bin = 0;
+            const u32 sg = i < S ? slevels[r0 + i] : 0u;
+            const int cnt = sg ? row_pair_cnt[r0 + i] : 0;
+            if (cnt) {
+                const uint4 *e = stair + row_pair_off[r0 + i];
+                for (int j = 0; j < cnt; j++) {
+                    const uint4 v = e[j];
+                    const u32 lv = v.x & 0xffffu;
+                    if (lv == 0u) break;                              // end of a short staircase
+                    if (lv > (u32)k) {
+                        const u32 m = v.x >> 16;
+                        if (m) {
+                            bin = 1u + sg * (u32)W + m;
+                            const int prev = atomicExch(head + v.y, i);
+                            nd[i] = make_uint2((u32)prev, sg | (m << 16));
+                            if (prev < 0) cl[atomicAdd(s_nq, 1)] = (int)v.y;
+                        }
+                        break;
+                    }
+                }
+            }
+            sweep_bin_add(bin, 0u, 0u, 0u, h2, nullptr, nullptr, nullptr);
+        }
+        __syncthreads();
+        // suffix sums: h2[1 + sigma * W + m] = matched rows with level >= sigma and match level >= m
+        for (int a = threadIdx.x; a <= L; a += blockDim.x)
+            for (int m = T - 1; m >= 0; m--) h2[1 + a * W + m] += h2[1 + a * W + m + 1];
+        __syncthreads();
+        for (int m = threadIdx.x; m <= T; m += blockDim.x)
+            for (int a = L - 1; a >= 0; a--) h2[1 + a * W + m] += h2[1 + (a + 1) * W + m];
+        const int nq = *s_nq;
+        for (int q = warp; q < nq; q += n_warps) {
+            const int p = cl[q];
+            const int first = head[p];
+            u32 ms = 0, mm = 0;
+            for (int i = first; i >= 0;) {
+                const uint2 v = nd[i];
+                ms = max(ms, v.y & 0xffffu);
+                mm = max(mm, v.y >> 16);
+                i = (int)v.x;
+            }
+            const int cells = (int)(ms * mm);
+            for (int c = lane; c < cells; c += 32) {
+                const u32 l = (u32)c / mm, t = (u32)c - l * mm;
+                u32 n = 0;
+                for (int i = first; i >= 0;) {
+                    const uint2 v = nd[i];
+                    n += (v.y & 0xffffu) > l && (v.y >> 16) > t;
+                    i = (int)v.x;
+                }
+                if (n) {
+                    const int cell = (int)l * T + (int)t;
+                    atomicAdd(sp + cell, 1u);
+                    if ((int)n <= cs) atomicAdd(hist + (i64)cell * cs + n - 1, 1u);
+                    else atomicAdd(spp_hist + ((i64)k * LT + cell) * n_bins + n, 1ull);
+                }
+            }
+        }
+        __syncthreads();
+        const int top = min(cs, S);                                   // no particle owns more satellites than S
+        for (int cell = threadIdx.x; cell < LT; cell += blockDim.x) {
+            const int l = cell / T, t = cell - l * T;
+            const u32 matched = h2[1 + (l + 1) * W + t + 1], unmatched = kept[l + 1] - matched, satp = sp[cell];
+            const i64 tcell = (i64)k * LT + cell;
+            if (counts) {
+                int *o = counts + 3 * ((i64)g * n_plevels * LT + tcell);
+                o[0] = (int)matched; o[1] = (int)unmatched; o[2] = (int)satp;
+            }
+            if (matched) atomicAdd(totals + 3 * tcell, (unsigned long long)matched);
+            if (unmatched) atomicAdd(totals + 3 * tcell + 1, (unsigned long long)unmatched);
+            if (satp) atomicAdd(totals + 3 * tcell + 2, (unsigned long long)satp);
+            if (satp)
+                for (int b = 0; b < top; b++) {
+                    const u32 v = hist[(i64)cell * cs + b];
+                    if (v) { atomicAdd(spp_hist + tcell * n_bins + b + 1, (unsigned long long)v); hist[(i64)cell * cs + b] = 0u; }
+                }
+            sp[cell] = 0u;
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < 1 + (L + 1) * W; i += blockDim.x) h2[i] = 0u;
+        for (int q = threadIdx.x; q < nq; q += blockDim.x) head[cl[q]] = -1;
+        if (threadIdx.x == 0) *s_nq = 0;
+        __syncthreads();
+    }
+}
+
+// Shared bytes of sat_sweep_counts_kernel for P particles per image and cs shared bins per cell
+static inline size_t sat_sweep_smem(int64_t P, int64_t L, int64_t T, int64_t cs)
+{
+    return (size_t)(4 * (P + (L + 1) + 1 + (L + 1) * (T + 1) + L * T * (1 + cs) + 1));
+}
+
+// (not part of the C ABI: the step of ampis_eval_images_sat_sweep_host after the join)
+int ampis_sat_sweep_counts(const uint32_t *d_area, const int32_t *d_row_mask, const int32_t *d_row_grp,
+                           int32_t n_rows, const int32_t *d_grp_row_begin, const int32_t *d_grp_row_count,
+                           const int32_t *d_grp_col_begin, const int32_t *d_grp_col_count, int32_t n_groups,
+                           int32_t max_cols, const int32_t *d_pair_ab, const uint32_t *d_pair_inter,
+                           const int64_t *d_row_pair_off, const int32_t *d_row_pair_cnt, const uint16_t *d_plevels,
+                           int32_t n_plevels, const uint16_t *d_slevels, int32_t n_slevels,
+                           const double *d_match_thresh, int32_t n_match, int32_t n_bins, int32_t chunks,
+                           void *d_stair, void *d_node, int32_t *d_claimed, int32_t *d_counts, int64_t *d_totals,
+                           int64_t *d_spp_hist, void *stream)
+{
+    AMPIS_REQUIRE(n_rows >= 0 && n_groups >= 0 && max_cols >= 0 && n_bins >= 1 && chunks >= 1, "bad size");
+    AMPIS_REQUIRE(max_cols <= AMPIS_SWEEP_MAX_PREDS, "too many particles in one image for the shared lists");
+    if (n_groups == 0) return AMPIS_OK;
+    cudaStream_t st = as_stream(stream);
+    if (n_rows > 0) {
+        sweep_rows_kernel<AMPIS_MODE_SAT><<<(unsigned)((n_rows + 127) / 128), 128, 0, st>>>(
+            d_area, d_row_mask, d_row_grp, n_rows, d_grp_row_begin, d_grp_row_count, d_grp_col_begin,
+            (const int2 *)d_pair_ab, d_pair_inter, d_row_pair_off, d_row_pair_cnt, (const unsigned short *)d_plevels,
+            d_match_thresh, n_match, (uint4 *)d_stair);
+        AMPIS_CHECK_LAUNCH("sweep_rows_kernel");
+    }
+    int dev = 0, optin = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (e != cudaSuccess) { ampis_set_error("sat_sweep_counts: %s", cudaGetErrorString(e)); return AMPIS_ECUDA; }
+    const int64_t L = n_slevels, T = n_match;
+    const size_t fixed = sat_sweep_smem(max_cols, L, T, 0);
+    AMPIS_REQUIRE(fixed <= (size_t)optin, "too many particles per image x (satellite levels + 1) x (match thresholds + 1) for shared memory");
+    const int64_t cs = std::min<int64_t>(std::min<int64_t>(n_bins - 1, 32), ((int64_t)optin - (int64_t)fixed) / (4 * L * T));
+    const size_t smem = sat_sweep_smem(max_cols, L, T, cs);
+    if (smem > 48 * 1024) {
+        e = cudaFuncSetAttribute(sat_sweep_counts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) {
+            ampis_set_error("sat_sweep_counts_kernel: %zu bytes of shared memory: %s", smem, cudaGetErrorString(e));
+            return AMPIS_ECUDA;
+        }
+    }
+    const int per = (n_plevels + chunks - 1) / chunks;
+    sat_sweep_counts_kernel<<<dim3((unsigned)n_groups, (unsigned)chunks), 256, smem, st>>>(
+        (const uint4 *)d_stair, d_row_pair_off, d_row_pair_cnt, d_grp_row_begin, d_grp_row_count, d_grp_col_count,
+        (const unsigned short *)d_slevels, n_plevels, n_slevels, n_match, per, n_bins, (int)cs, (uint2 *)d_node,
+        d_claimed, d_counts, (unsigned long long *)d_totals, (unsigned long long *)d_spp_hist);
+    AMPIS_CHECK_LAUNCH("sat_sweep_counts_kernel");
     return AMPIS_OK;
 }
 

@@ -350,3 +350,41 @@ def satellite_measurements_sharded(psi, thresh=0.5, print_summary=False, group=N
     if print_summary and rank == 0:
         powder._print_summary(out)
     return out
+
+
+def satellite_measurements_sweep_sharded(psi, particle_score_thresholds=None, satellite_score_thresholds=None,
+                                         match_thresholds=(0.5,), particle_scores=None, satellite_scores=None,
+                                         group=None, compute_fn=None):
+    """``powder.satellite_measurements_sweep`` of a dataset whose images are sharded over the ranks: rank r sweeps
+    images r, r+W, ... in one library call on its GPU and the totals, the satellites-per-particle histograms and the
+    kept counts are summed with ONE int64 all-reduce.  Every quantity, mspp included, is exact after the sum (the
+    median is read off the summed histogram), so the dataset keys equal the single-process ones on every rank.  Every
+    rank passes the full dataset (and the full per-image score lists); the histogram's length comes from all of it.
+    The per-image keys are those of the local shard, ``index`` the images this rank swept.  compute_fn: replaces
+    powder.satellite_measurements_sweep (same arguments, CPU tests)."""
+    from .applications import powder
+    rank, world = world_info(group)
+    images = [psi] if type(psi) == powder.PowderSatelliteImage else list(psi)
+    assert all(type(im) == powder.PowderSatelliteImage for im in images), 'psi must be list of PowderSatelliteImage objects!'
+    n = len(images)
+    idx = shard_indices(n, rank, world)
+    pick = lambda xs: None if xs is None else [xs[int(i)] for i in idx]
+    local = (compute_fn or powder.satellite_measurements_sweep)(
+        [images[int(i)] for i in idx], particle_score_thresholds, satellite_score_thresholds, match_thresholds,
+        pick(particle_scores), pick(satellite_scores), _n_bins=powder._sweep_bins(images))
+    parts = [np.asarray(local[k], np.int64) for k in ('n_particles', 'n_satellite_instances')]
+    tot, hist = np.asarray(local['n_satellites'], np.int64), np.asarray(local['spp_hist'], np.int64)
+    totals = np.stack([tot, local['n_satellites_unmatched'], local['n_satellited_particels']], axis=-1).astype(np.int64)
+    sums = torch.from_numpy(np.concatenate([totals.ravel(), hist.ravel()] + parts))
+    if world > 1 and dist.get_backend(group) == 'nccl':
+        sums = sums.cuda()
+    all_reduce_sum_(sums, group)
+    sums = sums.cpu().numpy()
+    a, b = totals.size, totals.size + hist.size
+    K, L = len(parts[0]), len(parts[1])
+    out = {k: local[k] for k in ('particle_score_thresholds', 'satellite_score_thresholds', 'match_thresholds')}
+    out.update(powder._sweep_summary(n, sums[b:b + K], sums[b + K:b + K + L], sums[:a].reshape(totals.shape),
+                                     sums[a:b].reshape(hist.shape)))
+    out.update({k: local[k] for k in ('image_counts', 'image_particles', 'image_satellites')})
+    out['index'] = idx
+    return out

@@ -567,6 +567,48 @@ def eval_images_sweep(rows_lists, cols_lists, levels, n_levels, iou_sorted, per_
     return out
 
 
+class ImagesSatSweep(object):
+    """Result of eval_images_sat_sweep() (numpy), thresholds in sorted order: totals int64 [K, L, T, 3] (matched,
+    unmatched, satellited particles), spp_hist int64 [K, L, T, n_bins], counts int32 [n_images, K, L, T, 3] (None
+    unless per_image), n_rows (satellites) / n_cols (particles) per image, pairs_found."""
+    __slots__ = ('totals', 'spp_hist', 'counts', 'n_rows', 'n_cols', 'pairs_found')
+
+
+def eval_images_sat_sweep(sat_lists, part_lists, plevels, n_plevels, slevels, n_slevels, match_sorted, n_bins,
+                          per_image=True):
+    """Satellite statistics of many images over a grid of particle-score x satellite-score x match thresholds in ONE
+    library call (ampis_eval_images_sat_sweep_host): the decode, join and intersections of eval_images in MODE_SAT
+    once, then the staircase and satellite count passes of csrc/score.cu.  sat_lists / part_lists: satellites (rows)
+    and particles (columns) of every image (RLE dicts).  plevels / slevels: uint16 per particle / satellite in image
+    order, the number of the n_plevels / n_slevels sorted score thresholds strictly below its score.  match_sorted:
+    match thresholds, ascending, each >= 0.  n_bins: 1 + at least the most satellites of any image."""
+    device = require_cuda()
+    n_img = len(sat_lists)
+    r, ptr, ln, hw, n, R = _marshal_images(sat_lists, part_lists, None)
+    mt = np.ascontiguousarray(match_sorted, np.float64)
+    K, L, T, B = int(n_plevels), int(n_slevels), len(mt), int(n_bins)
+    plv, slv = np.ascontiguousarray(plevels, np.uint16), np.ascontiguousarray(slevels, np.uint16)
+    assert len(plv) == int(r.n_cols.astype(np.int64).sum()) and len(slv) == R
+    out = ImagesSatSweep()
+    out.n_rows, out.n_cols, out.pairs_found = r.n_rows, r.n_cols, 0
+    out.totals = np.zeros((K, L, T, 3), np.int64)
+    out.spp_hist = np.zeros((K, L, T, B), np.int64)
+    out.counts = np.zeros((n_img, K, L, T, 3), np.int32) if per_image else None
+    status = np.empty(max(n, 1), np.int32)
+    found = C.c_int64(0)
+    pa = _addr
+    h32, w32 = np.ascontiguousarray(r.hw[:, 0].astype(np.uint32)), np.ascontiguousarray(r.hw[:, 1].astype(np.uint32))
+    lib = N.lib()
+    _call_growing(device, 'ampis_eval_images_sat_sweep_host', lambda d_ws, h_ws, need: lib.ampis_eval_images_sat_sweep_host(
+        pa(ptr), pa(ln), n_img, pa(r.n_rows), pa(r.n_cols), pa(h32), pa(w32), 0, pa(plv) if len(plv) else None, K,
+        pa(slv) if len(slv) else None, L, pa(mt), T, B, _p(d_ws), d_ws.numel(), _p(h_ws), h_ws.numel(), pa(status),
+        pa(out.totals), pa(out.spp_hist), pa(out.counts) if per_image and out.counts.size else None, C.byref(found),
+        C.byref(need), _stream()))
+    out.pairs_found = int(found.value)
+    _check_status(status[:n])
+    return out
+
+
 def measure_rle(masks):
     """(area uint32[n], tight bbox int32[n, 4]) of a list of RLE dicts: rleArea (structures.py:568,571;
     powder.py:264) and the box extract_boxes (data_utils.py:229-239) reads off the decoded mask.  Masks of one image size go through the one-call entry point (no intersection is run); mixed

@@ -346,6 +346,32 @@ int ampis_eval_images_sweep_host(const uint8_t *const *str_ptr, const int32_t *s
                                  int32_t *status, int64_t *totals, int64_t *seg_totals, int32_t *counts,
                                  int64_t *seg_sums, int64_t *pairs_found, int64_t *need_bytes, void *stream);
 
+/* ---- many images, satellite statistics over particle-score x satellite-score x match thresholds, one call --------
+ * What ampis_eval_images_host in AMPIS_MODE_SAT followed by powder.py:85-103 gives for every cut-off of the particles'
+ * and the satellites' scores and every match threshold, from one decode, one join and one intersection per candidate
+ * pair.  Strings, sizes, flags, workspaces and the AMPIS_ENOSPC protocol as ampis_eval_images_sweep_host, with rows =
+ * satellites and columns = particles.  plevels[p], one per particle in image order, and slevels[s], one per satellite
+ * in image order: the number of sorted score thresholds strictly below the score (0 for NaN); a particle is kept at
+ * particle level k iff plevels[p] > k, a satellite at satellite level l iff slevels[s] > l.  match_thresh[0 .. n_match):
+ * sorted ascending, each >= 0.  A kept satellite goes to the kept particle it overlaps most (first index on ties)
+ * when intersection / satellite area > match_thresh[t].  Outputs for cell (k, l, t): totals int64[K][L][T][3] =
+ * matched satellites, unmatched kept satellites, satellited particles; spp_hist int64[K][L][T][n_bins], bin c >= 1 =
+ * particles owning exactly c satellites, bin 0 = 0 (required; n_bins >= 1 + the most satellites in one image);
+ * counts int32[n_images][K][L][T][3] the same per image (NULL: not formed, its device space is not needed); status
+ * as ampis_eval_images_host.  Limits (AMPIS_EINVAL, checked before any upload): at most AMPIS_SWEEP_MAX_PREDS
+ * particles per image, 1 <= K, L <= 65535, 1 <= n_match <= AMPIS_SWEEP_MAX_IOU, K * L * T * n_bins <=
+ * AMPIS_SAT_SWEEP_MAX_HIST and (L + 1) * (T + 1) <= AMPIS_SAT_SWEEP_MAX_LT (the count kernel keeps per-cell tables in
+ * shared memory). */
+#define AMPIS_SAT_SWEEP_MAX_HIST (1LL << 26)
+#define AMPIS_SAT_SWEEP_MAX_LT   4096
+int ampis_eval_images_sat_sweep_host(const uint8_t *const *str_ptr, const int32_t *str_len, int32_t n_images,
+                                     const int32_t *n_rows, const int32_t *n_cols, const uint32_t *h,
+                                     const uint32_t *w, int32_t flags, const uint16_t *plevels, int32_t n_plevels,
+                                     const uint16_t *slevels, int32_t n_slevels, const double *match_thresh,
+                                     int32_t n_match, int32_t n_bins, void *d_ws, int64_t d_ws_bytes, void *h_ws,
+                                     int64_t h_ws_bytes, int32_t *status, int64_t *totals, int64_t *spp_hist,
+                                     int32_t *counts, int64_t *pairs_found, int64_t *need_bytes, void *stream);
+
 /* ---- dense intersection matrices on the tensor cores (tcgen05, int8 contraction) -----------
  * Same quantity as the dense output of ampis_intersect_rows -- I[r][c] = popcount(row AND col),
  * what rleIou's run walk accumulates per pair (analyze.py:108,158; powder.py:82) -- computed for
